@@ -8,6 +8,7 @@ BASELINE.json's metric is quoted on; 41 GB, fits one B200).
     python bench.py [--gpus N] [--steps K] [--warmup W] [--rows R] [--batch B] [--dtype fp32|bf16]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   (N > 1)
     python bench.py --impl reference ...      # the CPU arm (NumPy replica of the SQL ordering)
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's answer to DIR/*.npy (rank 0)
 
 Output: ONE JSON line on rank 0.
   value      whole-job QPS over EXACTLY K steps, queries already in HBM, results left in HBM (CUDA events on the
@@ -74,7 +75,15 @@ def parse_args():
     ap.add_argument("--no-group-e2e", action="store_true",
                     help="N > 1: keep e2e on the rank-per-GPU path instead of the one-process multi-GPU index")
     ap.add_argument("--lib", default=None, help="A/B: load this build of liborx.so instead of the in-tree default")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline's last timed step returned (ids, distances, counts) to DIR/<name>.npy; "
+                         "the inputs depend on the arguments only, so two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.mixed:
+        ap.error("--dump-outputs is not available with --mixed")
+    return a
 
 
 def workload_name(rows, dtype, batch):
@@ -151,6 +160,28 @@ def measured_peaks():
     return 6650.0, 1590.0, 1400.0, "fallback (B200_PROFILING.md)"
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, ids, dist, counts) -> None:
+    """`--dump-outputs`: one search answer as float64 .npy files -- `ids` [B, k, 2] (the hi and lo words of each 128-bit
+    id; every id the bench generates is below 2**53, so the float64 values are exact), `distances` [B, k] and `counts`
+    [B].  A batch whose answer exceeds 64 MB is cut to a fixed, seeded sample of its queries, whose positions in the
+    batch go to `query_index.npy`."""
+    ids = np.asarray(ids, np.uint64).reshape(len(dist), -1, 2)
+    assert not (ids >> np.uint64(53)).any(), "ids of 2**53 and above have no exact float64 form"
+    out = {"ids": ids.astype(np.float64), "distances": np.asarray(dist, np.float64),
+           "counts": np.asarray(counts, np.float64)}
+    per_query = sum(v[0].nbytes for v in out.values()) + 8
+    if per_query * len(dist) > DUMP_LIMIT_BYTES:
+        sel = np.sort(np.random.default_rng(0).choice(len(dist), DUMP_LIMIT_BYTES // per_query, replace=False))
+        out = {name: v[sel] for name, v in out.items()}
+        out["query_index"] = sel.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), v)
+
+
 def traffic_from_profile(tag: str, rows: int):
     """DRAM bytes per launch from the committed ncu --set full capture (profiles/traffic.json holds
     bytes for the captured row count; the scan is linear in rows, so it is scaled to this launch)."""
@@ -174,18 +205,18 @@ def _blas_threads(n):
 
 
 def _time_queries(X, inv, ids, Q, n_warm, n_timed, budget_s):
-    """Closed loop of single-query NumPy-replica searches; returns the per-query latencies (s)."""
+    """Closed loop of single-query NumPy-replica searches; returns the per-query latencies (s) and the last answer."""
     from oracle import cosine_topk as O
     for i in range(n_warm):
         O.numpy_replica_topk(X, ids, Q[i % Q.shape[0]], K, row_inv_norm=inv)
     lat, t_end = [], time.perf_counter() + budget_s
     for i in range(n_timed):
         t0 = time.perf_counter()
-        O.numpy_replica_topk(X, ids, Q[i % Q.shape[0]], K, row_inv_norm=inv)
+        last = O.numpy_replica_topk(X, ids, Q[i % Q.shape[0]], K, row_inv_norm=inv)
         lat.append(time.perf_counter() - t0)
         if time.perf_counter() > t_end and len(lat) >= 3:
             break
-    return np.asarray(lat)
+    return np.asarray(lat), last
 
 
 def time_cpu_arm(rows_full: int, batch: int, steps: int, warmup: int, budget_s: float = 25.0, exact_steps=False):
@@ -205,7 +236,7 @@ def time_cpu_arm(rows_full: int, batch: int, steps: int, warmup: int, budget_s: 
     X = syn.table(100_000)
     Q, _ = syn.queries(64, 100_000)
     inv = 1.0 / np.sqrt(np.einsum("ij,ij->i", X, X).astype(np.float64))
-    lat = _time_queries(X, inv, O.ids_arange(0, 100_000), Q, 5, max(200, steps), budget_s * 0.2)
+    lat, _ = _time_queries(X, inv, O.ids_arange(0, 100_000), Q, 5, max(200, steps), budget_s * 0.2)
     out["measured"].append({"rows": 100_000, "config": "BASELINE.json configs[0]", "queries": int(lat.size),
                             "p50_ms": float(np.median(lat) * 1e3), "p99_ms": float(np.percentile(lat, 99) * 1e3),
                             "qps": float(1.0 / np.median(lat)), "extrapolated": False})
@@ -216,8 +247,8 @@ def time_cpu_arm(rows_full: int, batch: int, steps: int, warmup: int, budget_s: 
     Q, _ = syn.queries(64, rows_full)
     inv = 1.0 / np.sqrt(np.einsum("ij,ij->i", X, X).astype(np.float64))
     ids = O.ids_arange(0, n_meas)
-    lat = _time_queries(X, inv, ids, Q, max(warmup, 3), steps if exact_steps else max(60, steps),
-                        1e9 if exact_steps else budget_s * 0.5)
+    lat, last = _time_queries(X, inv, ids, Q, max(warmup, 3), steps if exact_steps else max(60, steps),
+                              1e9 if exact_steps else budget_s * 0.5)
     p50 = float(np.median(lat))
     out["measured"].append({"rows": n_meas, "config": "first rows of the benchmarked table", "queries": int(lat.size),
                             "p50_ms": p50 * 1e3, "p99_ms": float(np.percentile(lat, 99) * 1e3), "qps": 1.0 / p50,
@@ -246,6 +277,7 @@ def time_cpu_arm(rows_full: int, batch: int, steps: int, warmup: int, budget_s: 
         thr = os.cpu_count() or 1
     out["cores"] = int(min(thr, n_cores))
     out["_lat_measured"] = lat
+    out["_last_answer"] = last
     return out
 
 
@@ -285,6 +317,9 @@ def run_reference(a):
         return
     cb = time_cpu_arm(a.rows, a.batch, a.steps, a.warmup, exact_steps=True)
     lat = cb.pop("_lat_measured")
+    ids, dist = cb.pop("_last_answer")
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, ids[None], dist[None], [len(dist)])
     qps = cb["value"]
     line = {"impl": "reference", "metric": METRIC, "value": qps, "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps,
             "warmup": max(a.warmup, 3), "ms_per_step": a.batch / qps * 1e3,
@@ -385,10 +420,11 @@ class Bench:
         e0.record()
         for i in range(steps):
             t = time.perf_counter()
-            step_fn(warmup + i)
+            out = step_fn(warmup + i)
             lat[i] = time.perf_counter() - t
         e1.record()
         self.barrier()
+        self.last_out = out
         ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device="cuda")
         if self.world > 1:
             self.dist.all_reduce(ms, op=self.dist.ReduceOp.MAX)
@@ -407,13 +443,14 @@ class Bench:
         e0.record()
         prev = None
         for i in range(steps):
-            t, _ = sh.search_submit(batches[(warmup + i) % n], K)
+            t, out = sh.search_submit(batches[(warmup + i) % n], K)
             if prev is not None:
                 sh.search_wait(prev)
             prev = t
         sh.search_wait(prev)
         e1.record()
         self.barrier()
+        self.last_out = out           # valid until the submit after next
         ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device="cuda")
         if self.world > 1:
             self.dist.all_reduce(ms, op=self.dist.ReduceOp.MAX)
@@ -554,12 +591,14 @@ class Bench:
             l0 = ix.stats()
             if pipelined:
                 total_ms = self.timed_pipelined(sh, dev_batches, steps, warmup)
-                l1 = ix.stats()
-                closed_ms, lat = self.timed(step_device, steps, warmup)
             else:
                 total_ms, lat = self.timed(step_device, steps, warmup)
-                l1 = ix.stats()
                 closed_ms = total_ms
+            l1 = ix.stats()
+            if a.dump_outputs:          # before a later search can reuse the result buffers
+                self.head_out = step_out_to_host(self.last_out)
+            if pipelined:
+                closed_ms, lat = self.timed(step_device, steps, warmup)
             # (2) the same loop again with a CUDA event pair recorded around every scan launch (on the stream the kernel
             #     runs on): the kernel's own duration for the roofline.  The two event records cost ~10 us per step, which
             #     is why they are not in region (1); this region's step time is reported beside the kernel time.
@@ -667,6 +706,8 @@ def run_ours(a):
 
     sh, owned, build_s = bn.build(a.rows, a.dtype)
     head = bn.measure(sh, owned, a.rows, a.dtype, a.batch, a.steps, a.warmup, a.verify)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, *bn.head_out)
     head_check = getattr(bn, "last_check", None) if a.verify > 0 else None       # (queries, ids, distances) the oracle confirmed
     extras = []
 
@@ -790,6 +831,7 @@ def run_ours(a):
     if not a.no_cpu_baseline and world == 1:
         cb = time_cpu_arm(a.rows, a.batch, 20, 3)
         cb.pop("_lat_measured", None)
+        cb.pop("_last_answer", None)
         line["cpu_baseline"] = cb
     emit(line)
 

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -43,3 +45,45 @@ def test_non_zero_ranks_of_the_reference_arm_exit_quietly():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"],
                          capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_dump_outputs_writes_the_last_timed_answer_the_same_on_every_run(tmp_path):
+    """`--dump-outputs DIR`: the answer of the last of exactly `--steps` timed queries, as float64 arrays; the same
+    arguments give the same inputs, so two runs write the same files."""
+    dumps = []
+    for run in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--rows", "20000",
+                              "--steps", "5", "--warmup", "1", "--dump-outputs", str(tmp_path / run)],
+                             capture_output=True, text=True, timeout=300, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads(out.stdout.strip().splitlines()[-1])
+        assert line["steps"] == 5 and line["cpu_baseline"]["measured"][1]["queries"] == 5
+        assert sorted(os.listdir(tmp_path / run)) == ["counts.npy", "distances.npy", "ids.npy"]
+        dumps.append({n: np.load(tmp_path / run / f"{n}.npy") for n in ("ids", "distances", "counts")})
+    a, b = dumps
+    assert a["ids"].shape == (1, 12, 2) and a["distances"].shape == (1, 12) and a["counts"].tolist() == [12.0]
+    assert all(v.dtype == np.float64 for v in a.values())
+    assert (a["ids"][..., 0] == 0).all() and ((a["ids"][..., 1] >= 0) & (a["ids"][..., 1] < 20000)).all()
+    assert (np.diff(a["distances"][0]) >= 0).all()
+    for n in a:
+        assert np.array_equal(a[n], b[n]), n
+
+
+def test_dump_outputs_samples_an_answer_above_the_size_limit(tmp_path, monkeypatch):
+    import bench
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 10_000)
+    B, k = 100, 12
+    ids = np.zeros((B, k, 2), np.uint64)
+    ids[:, :, 1] = np.arange(B * k, dtype=np.uint64).reshape(B, k) + np.uint64(2**53 - 1 - B * k)
+    dist = np.random.default_rng(1).random((B, k))
+    counts = np.full(B, k, np.int32)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), ids, dist, counts)
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("ids", "distances", "counts", "query_index")}
+    assert sum(v.nbytes for v in got.values()) <= 10_000
+    sel = got["query_index"].astype(np.int64)
+    assert len(sel) > 0 and (np.diff(sel) > 0).all() and sel[-1] < B
+    assert np.array_equal(got["ids"], ids[sel].astype(np.float64))
+    assert np.array_equal(got["ids"].astype(np.uint64), ids[sel])                  # exact below 2**53
+    assert np.array_equal(got["distances"], dist[sel]) and (got["counts"] == k).all()
+    assert np.array_equal(np.load(tmp_path / "b" / "query_index.npy"), got["query_index"])   # a fixed sample

@@ -16,6 +16,15 @@ from tests.test_batcher import FakeIndex
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
+@pytest.fixture
+def sock_path(tmp_path, monkeypatch):
+    """The owner's socket inside `tmp_path`, named relative to it: a unix socket path may hold at most 107 bytes,
+    and `tmp_path` alone can be longer than that.  Server, clients and child processes resolve it from the working
+    directory, which is `tmp_path` for the duration of the test."""
+    monkeypatch.chdir(tmp_path)
+    return "orx.sock"
+
+
 class FakeOwner(FakeIndex):
     def __init__(self, X, ids):
         super().__init__(X.copy(), ids.copy())
@@ -43,12 +52,12 @@ class FakeOwner(FakeIndex):
         return int((~keep).sum())
 
 
-def test_two_workers_share_one_owner(small_table, tmp_path):
+def test_two_workers_share_one_owner(small_table, sock_path):
     import outline_rag_b200 as orx
     from outline_rag_b200.daemon import RemoteIndex, serve_in_thread
     X, Q, _ = small_table
     owner = FakeOwner(X[:500], O.ids_arange(0, 500))
-    path = str(tmp_path / "orx.sock")
+    path = sock_path
     srv = serve_in_thread(owner, path, batch_window_ms=30.0, max_batch=64)
     try:
         a, b = RemoteIndex(path), RemoteIndex(path)
@@ -89,7 +98,7 @@ def test_two_workers_share_one_owner(small_table, tmp_path):
     assert not os.path.exists(path)
 
 
-def test_a_failed_call_never_desynchronises_the_next_one(small_table, tmp_path):
+def test_a_failed_call_never_desynchronises_the_next_one(small_table, sock_path):
     """ADVICE r1: after a timeout (or any exception between send and receive) the old client kept its socket, and the
     next caller read the tail of the previous response -- another query's ids.  Now the connection is dropped, a
     fresh one serves the next call, responses carry the request id, and concurrent calls of ONE client use several
@@ -108,7 +117,7 @@ def test_a_failed_call_never_desynchronises_the_next_one(small_table, tmp_path):
             return super().search(Qb, k)
 
     owner = SlowOwner(X[:400], ids)
-    path = str(tmp_path / "orx.sock")
+    path = sock_path
     srv = serve_in_thread(owner, path, batch_window_ms=None)
     try:
         c = RemoteIndex(path, timeout=0.3)
@@ -157,12 +166,12 @@ print(json.dumps([len(ix), ids[:, :, 1].tolist(), [float(d).hex() for d in dist[
 
 
 @pytest.mark.gpu
-def test_real_index_served_to_another_process(small_table, tmp_path):
+def test_real_index_served_to_another_process(small_table, sock_path):
     import outline_rag_b200 as orx
     from outline_rag_b200.daemon import serve_in_thread
     X, Q, _ = small_table
     ids = O.ids_arange(0, X.shape[0])
-    path = str(tmp_path / "orx.sock")
+    path = sock_path
     with orx.Index("fp32") as ix:
         ix.upsert(ids, X)
         srv = serve_in_thread(ix, path, batch_window_ms=2.0)
@@ -179,7 +188,7 @@ def test_real_index_served_to_another_process(small_table, tmp_path):
     assert dist0 == [float(d).hex() for d in O.topk_exact(X, ids, Q[0], 12)[1]]
 
 
-def test_prepared_filters_live_in_the_owner_and_their_searches_are_coalesced(small_table, tmp_path):
+def test_prepared_filters_live_in_the_owner_and_their_searches_are_coalesced(small_table, sock_path):
     """`RemoteIndex.make_filter`: the allow-list crosses the socket once, the handle stays in the owner process, and
     searches of different workers under the same handle share one filtered pass of the owner's batcher.  A
     `GpuVectorStore` over a `RemoteIndex` prepares and uses such a filter like a local one."""
@@ -212,7 +221,7 @@ def test_prepared_filters_live_in_the_owner_and_their_searches_are_coalesced(sma
             return super().search_filtered(Q, k, allow)
 
     owner = Owner(X[:500], ids)
-    path = str(tmp_path / "orx.sock")
+    path = sock_path
     srv = serve_in_thread(owner, path, batch_window_ms=40.0, max_batch=64)
     try:
         a, b = RemoteIndex(path), RemoteIndex(path)
@@ -263,7 +272,7 @@ def uuid_of(i):
 
 
 @pytest.mark.gpu
-def test_remote_prepared_filter_on_a_real_index(small_table, tmp_path):
+def test_remote_prepared_filter_on_a_real_index(small_table, sock_path):
     """The same over a real device table: a worker prepares a filter that admits 5000 of 8192 rows (bitmap regime); 12
     concurrent searches under it are coalesced by the owner into filtered tensor-core passes; answers equal the oracle's."""
     import outline_rag_b200 as orx
@@ -272,7 +281,7 @@ def test_remote_prepared_filter_on_a_real_index(small_table, tmp_path):
     n = X.shape[0]
     ids = O.ids_arange(0, n)
     sel = np.sort(np.random.default_rng(8).choice(n, size=5000, replace=False))
-    path = str(tmp_path / "orx.sock")
+    path = sock_path
     with orx.Index("fp32") as ix:
         ix.upsert(ids, X)
         srv = serve_in_thread(ix, path, batch_window_ms=30.0, max_batch=64)
