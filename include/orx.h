@@ -208,6 +208,13 @@ int orx_search_sharded(orx_index *idx, const float *queries, int nq, int dim, in
  * the completeness proof assumes.  1 <= nq <= 2048. */
 int orx_debug_coarse_scores(orx_index *idx, const float *queries, int nq, int use_pairs, float *out_device);
 
+/* Diagnostic for the same argument, GEMV side: the FAST scores of the GEMV scans (orx_search of one query, batches the
+ * tensor pass does not take, filtered bitmap scans) -- the fp32 FMA-chain dot of every live row with every normalised
+ * query, times the row's 1/|x|, exactly the value the scans key their candidates on (same load / FMA / shuffle
+ * sequence).  Irregular rows (norm outside [2^-40, 2^40]) come out +-inf or NaN, zero-norm rows NaN.  out_device
+ * [live rows, nq] fp32 in table row order.  1 <= nq <= 65535. */
+int orx_debug_fast_scores(orx_index *idx, const float *queries, int nq, float *out_device);
+
 /* Read back stored rows (as fp32) by id -- snapshot / debugging / tests.
  * out_vecs [n, dim] host; out_found [n] host (1/0). */
 int orx_fetch(orx_index *idx, const orx_id *ids, uint64_t n, float *out_vecs, int *out_found);

@@ -104,6 +104,7 @@ SIGNATURES = {
     "orx_search_sharded": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp]),
     "orx_fetch": (C.c_int, [_vp, _vp, C.c_uint64, _vp, _vp]),
     "orx_debug_coarse_scores": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp]),
+    "orx_debug_fast_scores": (C.c_int, [_vp, _vp, C.c_int, _vp]),
     "orx_pgcopy_open": (C.c_int, [_vp, C.POINTER(_vp)]),
     "orx_pgcopy_open_sharded": (C.c_int, [_vp, C.c_int, C.c_int, C.POINTER(_vp)]),
     "orx_pgcopy_feed": (C.c_int, [_vp, _vp, C.c_uint64]),

@@ -533,18 +533,28 @@ void launch_merge_topk(int n_lists, int nq, int k, const orx_id *ids, const doub
 
 // -------------------------------------------------- exhaustive fallback (rare path)
 // collect: every row whose fast score could still reach `fast_floor` (or every row).
-template <typename T>
+// DUMP (diagnostic instantiation behind orx_debug_fast_scores): query blockIdx.y of a batch, and instead of collecting,
+// every row's fast score -- the `dot * scale` that score_ord keys on -- is written to dump[row * nq + query], so that a
+// test can MEASURE max |fast - cosine| against the eps of the GEMV scans (same load / FMA / butterfly sequence).
+template <typename T, bool DUMP = false>
 __global__ void __launch_bounds__(256)
 collect_kernel(const T *__restrict__ table, const float *__restrict__ scale, uint32_t n_rows,
                const float *__restrict__ qhat, float fast_floor, int collect_all,
-               uint32_t *__restrict__ list, uint32_t *__restrict__ count) {
+               uint32_t *__restrict__ list, uint32_t *__restrict__ count, float *__restrict__ dump = nullptr) {
     const int lane = threadIdx.x & 31;
     const uint32_t gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const uint32_t n_gw = gridDim.x * (blockDim.x >> 5);
     float4 qv[8];
-    load_q_slice<T>(qhat, lane, qv);
+    load_q_slice<T>(qhat + (DUMP ? (size_t)blockIdx.y * ORX_DIM : 0), lane, qv);
     const uint4 *tab = reinterpret_cast<const uint4 *>(table);
     for (uint32_t row = gw; row < n_rows; row += n_gw) {
+        if constexpr (DUMP) {
+            uint4 v[RowVec<T>::NV];
+            load_row_vecs<T>(tab, row, lane, v);
+            const float acc = warp_row_dot<T>(v, qv);
+            if (lane == 0) dump[(size_t)row * gridDim.y + blockIdx.y] = acc * __ldg(scale + row);
+            continue;
+        }
         bool take = collect_all != 0;
         if (!take) {
             uint4 v[RowVec<T>::NV];
@@ -571,6 +581,18 @@ void launch_collect(int dtype, const void *table, const float *scale, uint32_t n
         collect_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(
             static_cast<const __nv_bfloat16 *>(table), scale, n_rows, qhat, fast_floor, collect_all,
             list, count);
+}
+
+void launch_dump_fast_scores(int dtype, const void *table, const float *scale, uint32_t n_rows, const float *qhat,
+                             int nq, float *out, cudaStream_t st) {
+    if (n_rows == 0 || nq <= 0) return;
+    const dim3 grid(device_sms() * 4, nq);
+    if (dtype == ORX_DTYPE_F32)
+        collect_kernel<float, true><<<grid, 256, 0, st>>>(static_cast<const float *>(table), scale, n_rows, qhat, 0.f, 0,
+                                                          nullptr, nullptr, out);
+    else
+        collect_kernel<__nv_bfloat16, true><<<grid, 256, 0, st>>>(static_cast<const __nv_bfloat16 *>(table), scale,
+                                                                  n_rows, qhat, 0.f, 0, nullptr, nullptr, out);
 }
 
 template <typename T>

@@ -9,8 +9,11 @@ namespace orx {
 // Rigorous bounds on |fast score - canonical cosine| per scan path (DESIGN.md, "Exactness").
 constexpr double EPS_GEMV_F32 = 3.0e-6;   // fp32 FMA chain of depth 32 + 5 shuffle adds
 constexpr double EPS_GEMV_BF16 = 3.0e-6;  // same arithmetic on exactly-converted bf16 rows
-constexpr double EPS_UMMA_TF32 = 2.5e-3;  // both operands cut to 10 mantissa bits: (1+2^-10)^2-1 = 1.96e-3, + accumulation
-constexpr double EPS_UMMA_BF16 = 2.5e-3;  // RNE bf16 query: 2^-9 = 1.96e-3 (rows are exact bf16), + accumulation
+// kind::tf32 truncates both operands to 10 mantissa bits (measured on sm_100a, tests/test_epsilon_adversarial_gpu.py):
+// worst case (1+2^-10)^2-1 = 1.96e-3; a worst-case query against its own row measures 1.927e-3 (DESIGN.md section 2)
+constexpr double EPS_UMMA_TF32 = 2.5e-3;
+// RNE bf16 query: 2^-9 = 1.96e-3 (rows are exact bf16); the worst-case construction measures 1.929e-3
+constexpr double EPS_UMMA_BF16 = 2.5e-3;
 
 // candidate list = 32 * slots keys per query: k <= 16 -> 32 candidates, k <= 32 -> 64
 // candidate list = 32 * slots keys per query: k <= 16 -> 32, k <= 32 -> 64, k <= 128 -> 32 more than k at least
@@ -70,6 +73,9 @@ void launch_merge_topk(int n_lists, int nq, int k, const orx_id *ids, const doub
 void launch_collect(int dtype, const void *table, const float *scale, uint32_t n_rows,
                     const float *qhat, float fast_floor, int collect_all,
                     uint32_t *list, uint32_t *count, cudaStream_t st);
+// diagnostic: fast scores of every row for nq staged queries, out [n_rows, nq] (orx_debug_fast_scores)
+void launch_dump_fast_scores(int dtype, const void *table, const float *scale, uint32_t n_rows, const float *qhat,
+                             int nq, float *out, cudaStream_t st);
 void launch_rescore_list(int dtype, const void *table, const double *n2, const orx_id *row_ids,
                          const float *q, const QueryPrep *prep, const uint32_t *list,
                          const uint32_t *count, double *dist_out, cudaStream_t st);

@@ -1967,6 +1967,26 @@ int orx_debug_coarse_scores(orx_index *ix, const float *queries, int nq, int use
     return ORX_OK;
 }
 
+int orx_debug_fast_scores(orx_index *ix, const float *queries, int nq, float *out_device) {
+    if (!ix || !queries || !out_device) return fail(ORX_ERR_INVALID, "null argument");
+    if (ix->group) return fail(ORX_ERR_INVALID, "per-GPU diagnostic: call it on a single-GPU index");
+    if (!is_device_ptr(out_device)) return fail(ORX_ERR_INVALID, "out must be device memory");
+    if (nq < 1 || nq > 65535) return fail(ORX_ERR_INVALID, "1 <= nq <= 65535, got %d", nq);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    DeviceGuard g(ix->device);
+    if (any_in_flight(ix)) return fail(ORX_ERR_INVALID, "wait for the searches in flight (orx_search_wait) first");
+    if (ix->n_live == 0) return fail(ORX_ERR_INVALID, "empty table");
+    const float *q_src = nullptr;
+    int rc = stage_queries(ix, queries, nq, &q_src);
+    if (rc != ORX_OK) return rc;
+    orx::launch_dump_fast_scores(ix->dtype, ix->table, ix->scale, (uint32_t)ix->n_live, ix->cur->qhat.p, nq, out_device,
+                                 ix->stream);
+    ix->stats.kernel_launches += 1;
+    CK(cudaStreamSynchronize(ix->stream));
+    CK(cudaGetLastError());
+    return ORX_OK;
+}
+
 int orx_fetch(orx_index *ix, const orx_id *ids, uint64_t n, float *out_vecs, int *out_found) {
     if (!ix) return fail(ORX_ERR_INVALID, "index is null");
     if (n == 0) return ORX_OK;

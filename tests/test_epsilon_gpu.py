@@ -4,8 +4,8 @@ all 1M rows x 256 queries come out of the very TMA / tcgen05.mma / TMEM pipeline
 (`orx_debug_coarse_scores`: only the epilogue differs -- it writes instead of selecting), for both operand kinds (tf32
 on fp32 tables, bf16 on bf16 tables) and both kernels (one CTA per tile, CTA pairs); the reference cosine is a plain
 PyTorch float64 matmul on the rows as stored.  Asserted: max error < eps / 2.  The measured maxima are printed and
-recorded in DESIGN.md section 2.  (GEMV scan: eps 3e-6, checked the same way on a sample through the candidate keys'
-scores would need another hook; its bound is a textbook FMA-chain bound, see DESIGN.md.)"""
+recorded in DESIGN.md section 2.  This is the benign corpus: the worst-case inputs of both scans, and the GEMV scan's
+eps, are measured in tests/test_epsilon_adversarial_gpu.py."""
 import numpy as np
 import pytest
 
