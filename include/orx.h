@@ -169,6 +169,34 @@ void orx_filter_destroy(orx_filter *flt);
 int orx_search_with_filter(orx_index *idx, orx_filter *flt, const float *queries, int nq, int dim, int k,
                            orx_id *out_ids, double *out_dist, int *out_counts);
 
+/* Maximal marginal relevance over the exact candidates -- what langchain's `VectorStoreRetriever(search_type="mmr")`
+ * gets from `max_marginal_relevance_search(query, k, fetch_k, lambda_mult)`, which langchain-postgres answers by
+ * fetching fetch_k rows with their embeddings and running `maximal_marginal_relevance` on the host.  Here both halves
+ * stay on the GPU and the result is defined bit for bit (DESIGN.md section 2, "MMR"):
+ *   candidates  C = the exact top-fetch_k of orx_search / orx_search_filtered / orx_search_with_filter, in contract
+ *               order; position p in C is the tie-break below;
+ *   s_q[p]      = 1 - distance[p] (binary64);
+ *   s_dd(p, r)  = clamp(canonical dot / sqrt(n2_p * n2_r), -1, 1) of the rows AS STORED (the halving tree of the
+ *               canonical distance, IEEE div / sqrt / mul);
+ *   greedy      first pick = position 0; then argmax of lambda*s_q[p] - (1-lambda)*max over picked r of s_dd(p, r),
+ *               evaluated without contraction; ties -> lowest position; NaN scores (zero-norm rows, zero query) only
+ *               once no finite score is left, in position order.
+ * Outputs as orx_search (host buffers only): out_ids [nq, k] and out_dist [nq, k] in SELECTION order, each with the
+ * canonical query distance orx_search reports for that row; out_counts [nq] = min(k, candidates); unused slots (0,0) /
+ * NaN.  1 <= k <= fetch_k <= ORX_MAX_K and 0 <= lambda_mult <= 1 (lambda 0 = pure diversity), else ORX_ERR_INVALID.
+ * The candidate search and the gather of their rows run under the index lock: no write lands in between.  Queries are
+ * processed in chunks of 256 (candidate matrix <= 256 x 128 x 4 KB = 128 MB of device scratch).  Rejected while
+ * orx_search_submit tickets are in flight (ORX_ERR_INVALID).  A multi-GPU handle gathers each shard's candidates on its own GPU and runs
+ * the selection on devices[0]; orx_search_mmr_with_filter is per GPU.  Not available: the row-sharded
+ * one-process-per-GPU search (orx_search_sharded), asynchronous submit / wait, device-resident buffers. */
+int orx_search_mmr(orx_index *idx, const float *queries, int nq, int dim, int k, int fetch_k, double lambda_mult,
+                   orx_id *out_ids, double *out_dist, int *out_counts);
+int orx_search_mmr_filtered(orx_index *idx, const float *queries, int nq, int dim, int k, int fetch_k,
+                            double lambda_mult, const orx_id *allow_ids, uint64_t n_allow,
+                            orx_id *out_ids, double *out_dist, int *out_counts);
+int orx_search_mmr_with_filter(orx_index *idx, orx_filter *flt, const float *queries, int nq, int dim, int k,
+                               int fetch_k, double lambda_mult, orx_id *out_ids, double *out_dist, int *out_counts);
+
 /* Merge `n_lists` per-shard results (each [nq, k] as written by orx_search, all on
  * this index's device or all on the host) into the global top-k with the same
  * ordering.  The on-device step after the NCCL allgather of the row-sharded path. */

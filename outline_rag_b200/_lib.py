@@ -95,6 +95,11 @@ SIGNATURES = {
     "orx_filter_create": (C.c_int, [_vp, _vp, C.c_uint64, C.POINTER(_vp)]),
     "orx_filter_destroy": (None, [_vp]),
     "orx_search_with_filter": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp]),
+    "orx_search_mmr": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _vp, _vp, _vp]),
+    "orx_search_mmr_filtered": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _vp, C.c_uint64,
+                                          _vp, _vp, _vp]),
+    "orx_search_mmr_with_filter": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double,
+                                             _vp, _vp, _vp]),
     "orx_merge_topk": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp]),
     "orx_merge_topk_strided": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp, C.c_uint64, _vp, _vp, _vp]),
     "orx_export_rows": (C.c_int, [_vp, C.c_uint64, C.c_uint64, _vp, _vp]),

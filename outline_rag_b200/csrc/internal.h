@@ -129,6 +129,12 @@ void launch_mask_scale(const float *scale, const uint32_t *allow_bits, uint32_t 
 void launch_decode_pgvector(const uint8_t *raw, const uint64_t *payload_off, uint32_t n, float *out,
                             cudaStream_t st);
 
+// ---- mmr.cu (orx_search_mmr*): rows [nq, fetch_k, ORX_DIM] = each query's candidates in contract order, gathered
+//      as fp32; dist [nq, fetch_k] their canonical distances; counts [nq].  sel [nq, k] <- picked positions in selection
+//      order, -1 past min(k, count)
+void launch_mmr_select(const float *rows, const double *dist, const int *counts, int nq, int fetch_k, int k,
+                       double lam, int *sel, cudaStream_t st);
+
 // launch `kernel` on `st` with the programmatic-stream-serialization attribute (common.cuh: PDL)
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {

@@ -315,6 +315,12 @@ struct orx_index {
     // exhaustive fallback scratch
     DevBuf<uint32_t> fb_list, fb_count;
     DevBuf<double> fb_dist;
+    // maximal-marginal-relevance scratch (orx_search_mmr*)
+    DevBuf<float> mmr_rows;              // [queries of a chunk, fetch_k, ORX_DIM] candidate matrix the kernel reads
+    DevBuf<float> mmr_stage;             // multi-GPU: this shard's candidates, gathered before the copy to the root
+    DevBuf<uint32_t> mmr_idx;
+    DevBuf<double> mmr_dist;
+    DevBuf<int> mmr_cnt, mmr_sel;
     // upsert / delete scratch
     DevBuf<float> stage;
     DevBuf<uint32_t> d_src_idx, d_dst_row;
@@ -1067,6 +1073,122 @@ int filtered_search_locked(orx_index *ix, const FilterOnDevice &f, const float *
     return ORX_OK;
 }
 
+// the live rows of a filter handle, re-resolved when the id -> row map has changed since (upsert of new ids, delete,
+// import)
+int filter_on_device(orx_index *ix, orx_filter *f, FilterOnDevice *out) {
+    if (!f->resolved || f->generation != ix->generation) {
+        std::vector<uint32_t> rows;
+        resolve_allow_ids(ix, f->ids.data(), f->ids.size(), rows);
+        int rc = upload_filter(ix, rows, f->d_list, f->d_count, f->d_bits);
+        if (rc != ORX_OK) return rc;
+        f->m = (uint32_t)rows.size();
+        f->generation = ix->generation;
+        f->resolved = true;
+    }
+    *out = FilterOnDevice{f->m, f->d_list.p, f->d_count.p, f->m >= FILTER_SCAN_MIN_ROWS ? f->d_bits.p : nullptr};
+    return ORX_OK;
+}
+
+// =========================================================================== maximal marginal relevance
+// Two phases per chunk of queries, under the caller's lock: `fetch` = the exact top-fetch_k (any search path) into host
+// arrays; `gather` = the candidates' stored rows as the fp32 matrix [m, fetch_k, ORX_DIM] on `kx`'s device (zero rows
+// past a query's count); then mmr_select_kernel on `kx`'s stream picks positions, and the host maps them back to the
+// candidates' ids and distances.
+constexpr int MMR_QCHUNK = 256;          // queries per chunk: candidate matrix <= 256 x 128 x 4 KB = 128 MB
+
+using MmrFetch = std::function<int(const float *q, int m, orx_id *ids, double *dist, int *cnt)>;
+using MmrGather = std::function<int(const orx_id *ids, const int *cnt, int m, const float **rows)>;
+
+int check_mmr_args(orx_index *ix, const float *queries, int nq, int dim, int k, int fetch_k, double lam,
+                   orx_id *out_ids, double *out_dist, int *out_counts) {
+    if (!ix) return fail(ORX_ERR_INVALID, "index is null");
+    if (dim != ORX_DIM) return fail(ORX_ERR_DIM, "different vector dimensions %d and %d", ORX_DIM, dim);
+    if (k < 1 || fetch_k < k || fetch_k > ORX_MAX_K)
+        return fail(ORX_ERR_INVALID, "need 1 <= k <= fetch_k <= %d, got k = %d, fetch_k = %d", ORX_MAX_K, k, fetch_k);
+    if (!(lam >= 0.0 && lam <= 1.0)) return fail(ORX_ERR_INVALID, "lambda_mult must be a number in [0, 1], got %g", lam);
+    if (nq < 0) return fail(ORX_ERR_INVALID, "nq must be >= 0");
+    if (nq == 0) return ORX_OK;
+    if (!queries || !out_ids || !out_dist || !out_counts) return fail(ORX_ERR_INVALID, "null argument");
+    if (is_device_ptr(queries) || is_device_ptr(out_ids) || is_device_ptr(out_dist) || is_device_ptr(out_counts))
+        return fail(ORX_ERR_INVALID, "MMR search takes host queries and host outputs");
+    return ORX_OK;
+}
+
+int mmr_run(orx_index *kx, const float *queries, int nq, int k, int fetch_k, double lam, orx_id *out_ids,
+            double *out_dist, int *out_counts, const MmrFetch &fetch, const MmrGather &gather) {
+    std::vector<orx_id> ids;
+    std::vector<double> dist;
+    std::vector<int> cnt, sel;
+    for (int q0 = 0; q0 < nq; q0 += MMR_QCHUNK) {
+        const int m = std::min(MMR_QCHUNK, nq - q0);
+        const size_t nc = (size_t)m * fetch_k;
+        ids.assign(nc, orx_id{0, 0});
+        dist.assign(nc, NAN);
+        cnt.assign(m, 0);
+        sel.assign((size_t)m * k, -1);
+        int rc = fetch(queries + (size_t)q0 * ORX_DIM, m, ids.data(), dist.data(), cnt.data());
+        if (rc != ORX_OK) return rc;
+        const float *rows = nullptr;
+        rc = gather(ids.data(), cnt.data(), m, &rows);
+        if (rc != ORX_OK) return rc;
+        {
+            DeviceGuard g(kx->device);
+            cudaStream_t st = kx->stream;
+            CK(kx->mmr_dist.ensure(nc));
+            CK(kx->mmr_cnt.ensure(m));
+            CK(kx->mmr_sel.ensure((size_t)m * k));
+            CK(cudaMemcpyAsync(kx->mmr_dist.p, dist.data(), nc * sizeof(double), cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(kx->mmr_cnt.p, cnt.data(), m * sizeof(int), cudaMemcpyHostToDevice, st));
+            orx::launch_mmr_select(rows, kx->mmr_dist.p, kx->mmr_cnt.p, m, fetch_k, k, lam, kx->mmr_sel.p, st);
+            kx->stats.kernel_launches += 1;
+            CK(cudaGetLastError());
+            CK(cudaMemcpyAsync(sel.data(), kx->mmr_sel.p, (size_t)m * k * sizeof(int), cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+        }
+        for (int j = 0; j < m; ++j) {
+            const int n = std::min(k, cnt[j]);
+            const size_t o = (size_t)(q0 + j) * k;
+            out_counts[q0 + j] = n;
+            for (int t = 0; t < k; ++t) {
+                const int p = t < n ? sel[(size_t)j * k + t] : -1;
+                if (t < n && (p < 0 || p >= cnt[j]))
+                    return fail(ORX_ERR_CUDA, "MMR selection returned position %d of %d (query %d)", p, cnt[j], q0 + j);
+                out_ids[o + t] = p >= 0 ? ids[(size_t)j * fetch_k + p] : orx_id{0, 0};
+                out_dist[o + t] = p >= 0 ? dist[(size_t)j * fetch_k + p] : NAN;
+            }
+        }
+    }
+    return ORX_OK;
+}
+
+// candidates of a one-GPU index -> their table rows (the map is stable: the caller holds ix->mu since the fetch)
+int mmr_gather_local(orx_index *ix, const orx_id *ids, const int *cnt, int m, int fetch_k, const float **rows) {
+    const size_t nc = (size_t)m * fetch_k;
+    std::vector<uint32_t> idx(nc, 0xFFFFFFFFu);
+    for (int j = 0; j < m; ++j)
+        for (int p = 0; p < cnt[j]; ++p) {
+            const uint32_t *r = ix->map.find(ids[(size_t)j * fetch_k + p]);
+            if (!r) return fail(ORX_ERR_CUDA, "MMR candidate of query %d is not in the table", j);
+            idx[(size_t)j * fetch_k + p] = *r;
+        }
+    CK(ix->mmr_idx.ensure(nc));
+    CK(ix->mmr_rows.ensure(nc * ORX_DIM));
+    CK(cudaMemcpyAsync(ix->mmr_idx.p, idx.data(), nc * sizeof(uint32_t), cudaMemcpyHostToDevice, ix->stream));
+    orx::launch_gather_rows(ix->dtype, ix->table, ix->mmr_idx.p, (uint32_t)nc, ix->mmr_rows.p, ix->stream);
+    ix->stats.kernel_launches += 1;
+    CK(cudaStreamSynchronize(ix->stream));      // `idx` is host memory of this frame
+    *rows = ix->mmr_rows.p;
+    return ORX_OK;
+}
+
+int mmr_local(orx_index *ix, const float *queries, int nq, int k, int fetch_k, double lam, orx_id *out_ids,
+              double *out_dist, int *out_counts, const MmrFetch &fetch) {
+    return mmr_run(ix, queries, nq, k, fetch_k, lam, out_ids, out_dist, out_counts, fetch,
+                   [&](const orx_id *ids, const int *cnt, int m, const float **rows) {
+                       return mmr_gather_local(ix, ids, cnt, m, fetch_k, rows);
+                   });
+}
+
 // =========================================================================== sharded search
 // Layout of one rank's result block for (nq, k): ids | dist | counts | flags (16-byte padded).
 struct SlotLayout {
@@ -1414,6 +1536,8 @@ void orx_destroy(orx_index *ix) {
     cudaFree(ix->n2);
     cudaFree(ix->row_ids);
     ix->fb_list.release(); ix->fb_count.release(); ix->fb_dist.release();
+    ix->mmr_rows.release(); ix->mmr_stage.release(); ix->mmr_idx.release(); ix->mmr_dist.release();
+    ix->mmr_cnt.release(); ix->mmr_sel.release();
     ix->allow_bits.release(); ix->h_allow_bits.release(); ix->scale_masked.release();
     ix->stage.release(); ix->d_src_idx.release(); ix->d_dst_row.release(); ix->d_ids.release();
     ix->d_flag.release(); ix->h_u32a.release(); ix->h_u32b.release(); ix->h_flag.release();
@@ -1703,18 +1827,69 @@ int orx_search_with_filter(orx_index *ix, orx_filter *f, const float *queries, i
     std::lock_guard<std::mutex> lk(ix->mu);
     DeviceGuard g(ix->device);
     if (any_in_flight(ix)) return fail(ORX_ERR_INVALID, "wait for the searches in flight (orx_search_wait) first");
-    if (!f->resolved || f->generation != ix->generation) {
-        // the id -> row map changed since the bitmap was built (upsert of new ids, delete, import)
-        std::vector<uint32_t> rows;
-        resolve_allow_ids(ix, f->ids.data(), f->ids.size(), rows);
-        rc = upload_filter(ix, rows, f->d_list, f->d_count, f->d_bits);
-        if (rc != ORX_OK) return rc;
-        f->m = (uint32_t)rows.size();
-        f->generation = ix->generation;
-        f->resolved = true;
-    }
-    const FilterOnDevice fd{f->m, f->d_list.p, f->d_count.p, f->m >= FILTER_SCAN_MIN_ROWS ? f->d_bits.p : nullptr};
+    FilterOnDevice fd;
+    rc = filter_on_device(ix, f, &fd);
+    if (rc != ORX_OK) return rc;
     return filtered_search_locked(ix, fd, queries, nq, k, out_ids, out_dist, out_counts);
+}
+
+int orx_search_mmr(orx_index *ix, const float *queries, int nq, int dim, int k, int fetch_k, double lambda_mult,
+                   orx_id *out_ids, double *out_dist, int *out_counts) {
+    int rc = check_mmr_args(ix, queries, nq, dim, k, fetch_k, lambda_mult, out_ids, out_dist, out_counts);
+    if (rc != ORX_OK || nq == 0) return rc;
+    if (ix->group)
+        return group_search_mmr(ix->group, queries, nq, k, fetch_k, lambda_mult, nullptr, 0, false, out_ids, out_dist,
+                                out_counts);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    DeviceGuard g(ix->device);
+    if (any_in_flight(ix)) return fail(ORX_ERR_INVALID, "wait for the searches in flight (orx_search_wait) first");
+    return mmr_local(ix, queries, nq, k, fetch_k, lambda_mult, out_ids, out_dist, out_counts,
+                     [&](const float *q, int m, orx_id *ids, double *dist, int *cnt) {
+                         return search_locked(ix, q, m, fetch_k, ids, dist, cnt);
+                     });
+}
+
+int orx_search_mmr_filtered(orx_index *ix, const float *queries, int nq, int dim, int k, int fetch_k,
+                            double lambda_mult, const orx_id *allow_ids, uint64_t n_allow, orx_id *out_ids,
+                            double *out_dist, int *out_counts) {
+    int rc = check_mmr_args(ix, queries, nq, dim, k, fetch_k, lambda_mult, out_ids, out_dist, out_counts);
+    if (rc != ORX_OK || nq == 0) return rc;
+    if (n_allow && !allow_ids) return fail(ORX_ERR_INVALID, "null argument");
+    if (is_device_ptr(allow_ids)) return fail(ORX_ERR_INVALID, "allow_ids must be a host pointer");
+    if (ix->group)
+        return group_search_mmr(ix->group, queries, nq, k, fetch_k, lambda_mult, allow_ids, n_allow, true, out_ids,
+                                out_dist, out_counts);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    DeviceGuard g(ix->device);
+    if (any_in_flight(ix)) return fail(ORX_ERR_INVALID, "wait for the searches in flight (orx_search_wait) first");
+    std::vector<uint32_t> rows;
+    resolve_allow_ids(ix, allow_ids, n_allow, rows);
+    rc = upload_filter(ix, rows, ix->fb_list, ix->fb_count, ix->allow_bits);
+    if (rc != ORX_OK) return rc;
+    const uint32_t m_allow = (uint32_t)rows.size();
+    const FilterOnDevice f{m_allow, ix->fb_list.p, ix->fb_count.p, m_allow >= FILTER_SCAN_MIN_ROWS ? ix->allow_bits.p : nullptr};
+    return mmr_local(ix, queries, nq, k, fetch_k, lambda_mult, out_ids, out_dist, out_counts,
+                     [&](const float *q, int m, orx_id *ids, double *dist, int *cnt) {
+                         return filtered_search_locked(ix, f, q, m, fetch_k, ids, dist, cnt);
+                     });
+}
+
+int orx_search_mmr_with_filter(orx_index *ix, orx_filter *f, const float *queries, int nq, int dim, int k,
+                               int fetch_k, double lambda_mult, orx_id *out_ids, double *out_dist, int *out_counts) {
+    int rc = check_mmr_args(ix, queries, nq, dim, k, fetch_k, lambda_mult, out_ids, out_dist, out_counts);
+    if (rc != ORX_OK || nq == 0) return rc;
+    if (ix->group) return fail(ORX_ERR_INVALID, "filter handles are per GPU: use orx_search_mmr_filtered on a multi-GPU index");
+    if (!f || f->ix != ix) return fail(ORX_ERR_INVALID, "filter does not belong to this index");
+    std::lock_guard<std::mutex> lk(ix->mu);
+    DeviceGuard g(ix->device);
+    if (any_in_flight(ix)) return fail(ORX_ERR_INVALID, "wait for the searches in flight (orx_search_wait) first");
+    FilterOnDevice fd;
+    rc = filter_on_device(ix, f, &fd);
+    if (rc != ORX_OK) return rc;
+    return mmr_local(ix, queries, nq, k, fetch_k, lambda_mult, out_ids, out_dist, out_counts,
+                     [&](const float *q, int m, orx_id *ids, double *dist, int *cnt) {
+                         return filtered_search_locked(ix, fd, q, m, fetch_k, ids, dist, cnt);
+                     });
 }
 
 int orx_merge_topk(orx_index *ix, int n_lists, int nq, int k, const orx_id *ids, const double *dist,

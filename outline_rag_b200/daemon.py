@@ -143,6 +143,19 @@ class IndexServer:
                 else:
                     ids, dist, cnt = await asyncio.to_thread(self.index.search_filtered, Q, k, _unpack_arr(req["allow"]))
                 return {"ids": _pack_arr(ids), "dist": _pack_arr(dist), "cnt": _pack_arr(cnt)}
+            if op == "search_mmr":
+                # never through the batcher: one MMR call per request, on the owner's index
+                Q, k = _unpack_arr(req["q"]), int(req["k"])
+                allow = None
+                if "fid" in req:
+                    allow = self._filters.get(int(req["fid"]))
+                    if allow is None:
+                        return {"err": ORX_ERR_INVALID, "msg": f"unknown filter {req['fid']}", "value_error": True}
+                elif "allow" in req:
+                    allow = _unpack_arr(req["allow"])
+                ids, dist, cnt = await asyncio.to_thread(self.index.search_mmr, Q, k, int(req["fetch_k"]),
+                                                         float(req["lambda_mult"]), allow)
+                return {"ids": _pack_arr(ids), "dist": _pack_arr(dist), "cnt": _pack_arr(cnt)}
             if op == "filter_create":
                 flt = await asyncio.to_thread(self.index.make_filter, _unpack_arr(req["allow"]))
                 self._next_fid += 1
@@ -326,6 +339,23 @@ class RemoteIndex:
                 raise OrxValueError(ORX_ERR_INVALID, "filter is closed or belongs to another index")
             req["fid"] = allow_ids._fid
         else:
+            req["allow"] = _pack_arr(ids_to_array(allow_ids))
+        r = self._call(req)
+        return _unpack_arr(r["ids"]), _unpack_arr(r["dist"]), _unpack_arr(r["cnt"])
+
+    def search_mmr(self, queries, k: int = 4, fetch_k: int = 20, lambda_mult: float = 0.5, allow_ids=None):
+        """`Index.search_mmr` on the owner; `allow_ids`: None, ids or a `RemoteFilter`."""
+        from .engine import ids_to_array
+        q = np.asarray(queries, dtype=np.float32)
+        if q.ndim == 1:
+            q = q.reshape(1, -1)
+        req = {"op": "search_mmr", "q": _pack_arr(q), "k": int(k), "fetch_k": int(fetch_k),
+               "lambda_mult": float(lambda_mult)}
+        if isinstance(allow_ids, RemoteFilter):
+            if allow_ids._index is not self or allow_ids._fid is None:
+                raise OrxValueError(ORX_ERR_INVALID, "filter is closed or belongs to another index")
+            req["fid"] = allow_ids._fid
+        elif allow_ids is not None:
             req["allow"] = _pack_arr(ids_to_array(allow_ids))
         r = self._call(req)
         return _unpack_arr(r["ids"]), _unpack_arr(r["dist"]), _unpack_arr(r["cnt"])

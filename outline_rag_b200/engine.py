@@ -406,6 +406,30 @@ class Index:
                                       C.c_void_p(dist.ctypes.data), C.c_void_p(cnt.ctypes.data)))
         return ids, dist, cnt
 
+    def search_mmr(self, queries, k: int = 4, fetch_k: int = 20, lambda_mult: float = 0.5, allow_ids=None):
+        """Maximal marginal relevance over the exact top-`fetch_k` (`orx_search_mmr*`): `min(k, candidates)` rows per
+        query, picked greedily by `lambda_mult * (1 - distance) - (1 - lambda_mult) * max cosine to the rows picked so
+        far` (include/orx.h states the exact rule).  `allow_ids`: None, ids or a `Filter`, as in `search_filtered`.
+        NumPy in / out: ``(ids uint64 [nq,k,2], dist float64 [nq,k], counts int32 [nq])`` in SELECTION order, each
+        row with its query distance.  Not served by the micro-batcher or the row-sharded `ShardedIndex`."""
+        q = _host_f32(queries, "queries")
+        nq, dim = q.shape
+        ids = np.zeros((nq, max(k, 0), 2), np.uint64)
+        dist = np.full((nq, max(k, 0)), np.nan, np.float64)
+        cnt = np.zeros(nq, np.int32)
+        outs = (C.c_void_p(ids.ctypes.data), C.c_void_p(dist.ctypes.data), C.c_void_p(cnt.ctypes.data))
+        head = (C.c_void_p(q.ctypes.data), nq, dim, int(k), int(fetch_k), float(lambda_mult))
+        if allow_ids is None:
+            check(lib.orx_search_mmr(self._h, *head, *outs))
+        elif isinstance(allow_ids, Filter):
+            if allow_ids._index is not self or not allow_ids._f:
+                raise _lib.OrxValueError(_lib.ORX_ERR_INVALID, "filter is closed or belongs to another index")
+            check(lib.orx_search_mmr_with_filter(self._h, allow_ids._f, *head, *outs))
+        else:
+            allow = ids_to_array(allow_ids)
+            check(lib.orx_search_mmr_filtered(self._h, *head, C.c_void_p(allow.ctypes.data), allow.shape[0], *outs))
+        return ids, dist, cnt
+
     def search_into(self, queries, k: int, ids_out, dist_out, counts_out) -> None:
         """`search` of a float32 CUDA tensor writing into caller-owned CUDA tensors (views of one
         result block in the row-sharded path: no allocation, no packing kernels)."""

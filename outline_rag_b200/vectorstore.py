@@ -151,18 +151,36 @@ def _canon_uuid(v) -> str:
     return str(uuid.UUID(str(v)))
 
 
-class GpuRetriever:
-    """``VectorStoreRetriever`` stand-in (search_type="similarity") for hosts WITHOUT langchain-core; with it,
-    `GpuVectorStore.as_retriever` returns langchain's own ``VectorStoreRetriever``."""
+SEARCH_TYPES = ("similarity", "similarity_score_threshold", "mmr")     # langchain-core's VectorStoreRetriever
 
-    def __init__(self, store: "GpuVectorStore", search_kwargs: Optional[dict] = None):
+
+class GpuRetriever:
+    """``VectorStoreRetriever`` stand-in for hosts WITHOUT langchain-core (with it, `GpuVectorStore.as_retriever`
+    returns langchain's own ``VectorStoreRetriever``).  Same three search types and the same dispatch:
+    ``similarity`` -> ``similarity_search``, ``mmr`` -> ``max_marginal_relevance_search`` (never micro-batched),
+    ``similarity_score_threshold`` -> ``similarity_search_with_relevance_scores`` (``score_threshold`` required)."""
+
+    def __init__(self, store: "GpuVectorStore", search_kwargs: Optional[dict] = None, search_type: str = "similarity"):
+        if search_type not in SEARCH_TYPES:
+            raise ValueError(f"search_type of {search_type} not allowed. Valid values are: {SEARCH_TYPES}")
         self.vectorstore = store
+        self.search_type = search_type
         self.search_kwargs = dict(search_kwargs or {})
+        if search_type == "similarity_score_threshold" and not isinstance(self.search_kwargs.get("score_threshold"), float):
+            raise ValueError("`score_threshold` is not specified with a float value(0~1) in `search_kwargs`.")
 
     async def ainvoke(self, query: str, **_: Any) -> list:
+        if self.search_type == "mmr":
+            return await self.vectorstore.amax_marginal_relevance_search(query, **self.search_kwargs)
+        if self.search_type == "similarity_score_threshold":
+            return [d for d, _ in await self.vectorstore.asimilarity_search_with_relevance_scores(query, **self.search_kwargs)]
         return await self.vectorstore.asimilarity_search(query, **self.search_kwargs)
 
     def invoke(self, query: str, **_: Any) -> list:
+        if self.search_type == "mmr":
+            return self.vectorstore.max_marginal_relevance_search(query, **self.search_kwargs)
+        if self.search_type == "similarity_score_threshold":
+            return [d for d, _ in self.vectorstore.similarity_search_with_relevance_scores(query, **self.search_kwargs)]
         return self.vectorstore.similarity_search(query, **self.search_kwargs)
 
 
@@ -209,7 +227,7 @@ class GpuVectorStore(_VectorStoreBase):
         ``asimilarity_search(query, **search_kwargs)``.  Without it: the duck-typed `GpuRetriever`."""
         if HAVE_LANGCHAIN:
             return super().as_retriever(**kwargs)
-        return GpuRetriever(self, kwargs.get("search_kwargs"))
+        return GpuRetriever(self, kwargs.get("search_kwargs"), kwargs.get("search_type", "similarity"))
 
     # -- the rest of langchain's abstract VectorStore surface
     @property
@@ -395,5 +413,77 @@ class GpuVectorStore(_VectorStoreBase):
         emb = self.embedding_service.embed_query(query)
         return [d for d, _ in self.similarity_search_with_score_by_vector(emb, k, **kw)]
 
+    # ---------------------------------------------------------------- relevance scores
+    @staticmethod
+    def _cosine_relevance(distance: float) -> float:
+        return 1.0 - distance
 
-__all__ = ["GpuVectorStore", "GpuRetriever", "MemoryDocStore", "Document", "DEFAULT_METADATA_COLUMNS", "HAVE_LANGCHAIN"]
+    def _select_relevance_score_fn(self):
+        """Cosine distance -> relevance, as langchain-postgres does for its default (cosine) strategy: 1 - distance."""
+        return self._cosine_relevance
+
+    @staticmethod
+    def _apply_threshold(pairs, score_threshold: Optional[float]):
+        return pairs if score_threshold is None else [(d, s) for d, s in pairs if s >= score_threshold]
+
+    def similarity_search_with_relevance_scores(self, query: str, k: int = 4, score_threshold: Optional[float] = None,
+                                                **kw: Any):
+        """-> ``[(Document, 1 - distance)]`` in distance order, keeping those with relevance >= `score_threshold`."""
+        fn = self._select_relevance_score_fn()
+        emb = self.embedding_service.embed_query(query)
+        pairs = [(d, fn(s)) for d, s in self.similarity_search_with_score_by_vector(emb, k, **kw)]
+        return self._apply_threshold(pairs, score_threshold)
+
+    async def asimilarity_search_with_relevance_scores(self, query: str, k: int = 4,
+                                                       score_threshold: Optional[float] = None, **kw: Any):
+        fn = self._select_relevance_score_fn()
+        pairs = [(d, fn(s)) for d, s in await self.asimilarity_search_with_score(query, k, **kw)]
+        return self._apply_threshold(pairs, score_threshold)
+
+    # ---------------------------------------------------------------- maximal marginal relevance
+    def max_marginal_relevance_search_with_score_by_vector(self, embedding, k: int = 4, fetch_k: int = 20,
+                                                           lambda_mult: float = 0.5, filter=None, **_: Any):
+        """``[(Document, cosine distance)]``: the `k` rows MMR picks among the exact top-`fetch_k` (`Index.search_mmr`,
+        on the GPU), returned in distance order as langchain-postgres returns them.  `k` is clamped to `fetch_k`;
+        ``lambda_mult=0`` means pure diversity (not replaced by the default)."""
+        q = np.asarray(embedding, dtype=np.float32).reshape(1, -1)
+        k = min(int(k), int(fetch_k))
+        allow = None
+        if filter is not None:
+            allow = filter if _is_handle(filter) else self.doc_store.ids_for_filter(filter)
+        ids, dist, cnt = self.index.search_mmr(q, k, fetch_k, lambda_mult, allow)
+        n = int(cnt[0])
+        d = dist[0, :n]
+        nan = np.isnan(d)
+        # fetch order = the ordering contract (distance ASC, NaN last, id ASC)
+        order = np.lexsort((ids[0, :n, 1], ids[0, :n, 0], np.where(nan, 0.0, d), nan))
+        return self._hydrate(ids[0, :n][order], d[order], n)
+
+    def max_marginal_relevance_search_by_vector(self, embedding, k: int = 4, fetch_k: int = 20,
+                                                lambda_mult: float = 0.5, **kw: Any):
+        return [d for d, _ in self.max_marginal_relevance_search_with_score_by_vector(embedding, k, fetch_k,
+                                                                                     lambda_mult, **kw)]
+
+    def max_marginal_relevance_search(self, query: str, k: int = 4, fetch_k: int = 20, lambda_mult: float = 0.5,
+                                      **kw: Any):
+        """What ``as_retriever(search_type="mmr", search_kwargs={"k": 12, "fetch_k": 48})`` calls."""
+        emb = self.embedding_service.embed_query(query)
+        return self.max_marginal_relevance_search_by_vector(emb, k, fetch_k, lambda_mult, **kw)
+
+    async def amax_marginal_relevance_search_with_score_by_vector(self, embedding, k: int = 4, fetch_k: int = 20,
+                                                                  lambda_mult: float = 0.5, **kw: Any):
+        return await asyncio.to_thread(self.max_marginal_relevance_search_with_score_by_vector, embedding, k, fetch_k,
+                                       lambda_mult, **kw)
+
+    async def amax_marginal_relevance_search_by_vector(self, embedding, k: int = 4, fetch_k: int = 20,
+                                                       lambda_mult: float = 0.5, **kw: Any):
+        return [d for d, _ in await self.amax_marginal_relevance_search_with_score_by_vector(embedding, k, fetch_k,
+                                                                                            lambda_mult, **kw)]
+
+    async def amax_marginal_relevance_search(self, query: str, k: int = 4, fetch_k: int = 20,
+                                             lambda_mult: float = 0.5, **kw: Any):
+        emb = await self.embedding_service.aembed_query(query)
+        return await self.amax_marginal_relevance_search_by_vector(emb, k, fetch_k, lambda_mult, **kw)
+
+
+__all__ = ["GpuVectorStore", "GpuRetriever", "SEARCH_TYPES", "MemoryDocStore", "Document", "DEFAULT_METADATA_COLUMNS", "HAVE_LANGCHAIN"]
