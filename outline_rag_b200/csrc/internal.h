@@ -158,6 +158,16 @@ template <typename T> inline T cap_grid(T blocks, int ctas_per_sm) {     // pers
     return blocks > cap ? cap : blocks;
 }
 
+// mix64(hi * GOLD ^ lo): the hash of the host's id -> row map and, mod the shard count, the row-shard function
+// (== outline_rag_b200/sharded.py shard_of, SURVEY.md 8e)
+inline uint64_t id_hash(const orx_id &id) {
+    uint64_t z = id.hi * 0x9E3779B97F4A7C15ull ^ id.lo;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+inline uint32_t shard_of_id(const orx_id &id, uint32_t world) { return (uint32_t)(id_hash(id) % world); }
+
 // ---- orx_api.cu: what the other translation units need from an index
 int set_error(int code, const char *fmt, ...);     // records the thread-local message, returns code
 int index_device(const orx_index *ix);

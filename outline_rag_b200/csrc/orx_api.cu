@@ -46,12 +46,7 @@ int fail(int code, const char *fmt, ...) {
     } while (0)
 
 struct IdHash {
-    size_t operator()(const orx_id &a) const {
-        uint64_t z = a.hi * 0x9E3779B97F4A7C15ull ^ a.lo;
-        z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-        z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-        return (size_t)(z ^ (z >> 31));
-    }
+    size_t operator()(const orx_id &a) const { return (size_t)orx::id_hash(a); }
 };
 struct IdEq {
     bool operator()(const orx_id &a, const orx_id &b) const { return a.hi == b.hi && a.lo == b.lo; }
@@ -82,7 +77,6 @@ class IdMap {
     }
 
 public:
-    size_t size() const { return used_; }
     void reserve(size_t n) {
         if (tab_.size() < n * 2) rehash(n);
     }
@@ -215,6 +209,19 @@ struct PinBuf {
     }
 };
 
+// Layout of one rank's result block for (nq, k): ids | dist | counts | flags (16-byte padded).
+struct SlotLayout {
+    size_t dist_off = 0, counts_off = 0, flags_off = 0, bytes = 0;
+};
+SlotLayout slot_layout(int nq, int k) {
+    SlotLayout L;
+    L.dist_off = (size_t)nq * k * sizeof(orx_id);
+    L.counts_off = L.dist_off + (size_t)nq * k * sizeof(double);
+    L.flags_off = L.counts_off + (size_t)nq * sizeof(int);
+    L.bytes = (L.flags_off + (size_t)nq * sizeof(int) + 15) & ~(size_t)15;
+    return L;
+}
+
 }  // namespace
 
 constexpr int XQ_MAX = 1024;                         // queries per exchange round (larger batches are chunked)
@@ -226,7 +233,6 @@ struct Exchange {   // peer-memory exchange state of one rank (orx_shard_*) or o
     size_t slot_bytes = 0;                           // capacity of one slot
     size_t set_bytes = 0;                            // world slots
     size_t flags_off = 0;                            // offset of the arrival words (2 sets x world x 128 B)
-    size_t total_bytes = 0;
     char *base = nullptr;                            // my buffer
     std::vector<char *> peer_base;                   // every rank's buffer as mapped in this process
     void **d_peer_slot[2] = {nullptr, nullptr};      // device arrays [world]: MY slot inside peer g's set s
@@ -235,10 +241,6 @@ struct Exchange {   // peer-memory exchange state of one rank (orx_shard_*) or o
     bool connected = false;
 };
 
-
-struct SlotLayoutPod {      // layout of one rank's result block for (nq, k) -- see slot_layout()
-    size_t dist_off = 0, counts_off = 0, flags_off = 0, bytes = 0;
-};
 struct SearchSlot {         // everything ONE search in flight owns
     DevBuf<float> q_dev, qhat;
     DevBuf<__nv_bfloat16> qhat16;
@@ -262,12 +264,13 @@ struct SearchSlot {         // everything ONE search in flight owns
         int settled_rc = ORX_OK;
         std::string settled_err;
         int nq = 0, k = 0, path = 1;
-        orx_id *out_ids = nullptr;
+        orx_id *out_ids = nullptr;          // the caller's arrays
         double *out_dist = nullptr;
         int *out_counts = nullptr;
+        orx::ResultOut out{};               // where the kernels write (prepare_results)
         const float *q_src = nullptr;
         uint32_t token = 0, seq = 0, ticket = 0;
-        SlotLayoutPod L;
+        SlotLayout L;
         std::chrono::steady_clock::time_point t_begin;
     } pend;
     void release() {
@@ -287,7 +290,6 @@ struct orx_index {
     uint64_t n_live = 0;
     uint64_t generation = 0;            // bumped whenever the id -> row map changes (orx_filter re-resolves then)
     std::atomic<uint64_t> mutations{0}; // bumped by EVERY successful write (upsert incl. in-place, delete, import): snapshots check it
-    int scan_grid_sms = 0;              // multiProcessorCount of `device` (orx_create)
 
     // the table (device)
     void *table = nullptr;
@@ -333,12 +335,19 @@ struct orx_index {
     orx_stats stats{};
 };
 
+struct FilterOnDevice {          // a resolved predicate: the eligible rows, as a sorted list and (when large) a bitmap
+    uint32_t m;
+    const uint32_t *list;        // [m] device
+    const uint32_t *count;       // device word holding m
+    const uint32_t *bits;        // [(n_live+31)/32] device, or null: rescore the list, no scan
+};
+
 struct orx_filter {     // a reusable resolved predicate (orx_filter_create / orx_search_with_filter)
     orx_index *ix = nullptr;
     int device = 0;
     std::vector<orx_id> ids;              // the id set as given
     DevBuf<uint32_t> d_list, d_count, d_bits;
-    uint32_t m = 0;                       // eligible live rows at `generation`
+    FilterOnDevice dev{};                 // the eligible live rows at `generation`, in d_list / d_count / d_bits
     uint64_t generation = 0;
     bool resolved = false;
 };
@@ -416,14 +425,37 @@ int grow_table(orx_index *ix, uint64_t need) {
     ix->n2 = n;
     ix->row_ids = r;
     ix->capacity = cap;
-    for (SearchSlot &sl : ix->slot)
-        if (sl.umma) orx::umma_plan_invalidate(sl.umma);
     return ORX_OK;
 }
 
 int group_upsert(Group *g, const orx_id *ids, const float *vecs, uint64_t n);
 
 // ---------------------------------------------------------------- upsert
+int validate_locked(orx_index *ix, const float *vecs, uint64_t n) {      // pgvector's element check, whole batch
+    cudaStream_t st = ix->stream;
+    const bool on_dev = is_device_ptr(vecs);
+    const uint64_t chunk = std::min<uint64_t>(n, STAGE_ROWS);
+    CK(ix->d_flag.ensure(1));
+    CK(ix->h_flag.ensure(1));
+    if (!on_dev) CK(ix->stage.ensure(chunk * ORX_DIM));
+    CK(cudaMemsetAsync(ix->d_flag.p, 0, sizeof(int), st));
+    for (uint64_t s = 0; s < n; s += chunk) {
+        const uint64_t m = std::min(chunk, n - s);
+        const float *src = vecs + s * ORX_DIM;
+        if (!on_dev) {
+            CK(cudaMemcpyAsync(ix->stage.p, src, m * ORX_DIM * sizeof(float), cudaMemcpyHostToDevice, st));
+            src = ix->stage.p;
+        }
+        orx::launch_validate_rows(src, m, ix->d_flag.p, st);
+        ix->stats.kernel_launches += 1;
+    }
+    CK(cudaMemcpyAsync(ix->h_flag.p, ix->d_flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+    if (*ix->h_flag.p) return fail(ORX_ERR_NONFINITE, "NaN or infinite value not allowed in vector");
+    return ORX_OK;
+}
+
 // validate (pgvector's element check over the WHOLE batch) -> commit, stream-ordered: the commit kernels read the
 // validation flag on the device and write nothing when it is set, so a batch of up to STAGE_ROWS rows needs ONE host
 // synchronisation.  Host state (id -> row map, live row count) is published only after the device work of a chunk
@@ -432,29 +464,16 @@ int upsert_locked(orx_index *ix, const orx_id *ids, const float *vecs, uint64_t 
     cudaStream_t st = ix->stream;
     const bool on_dev = is_device_ptr(vecs);
     const uint64_t chunk = std::min<uint64_t>(n, STAGE_ROWS);
+    const bool single = n <= chunk;           // one chunk: staged once, validated and committed back to back
+    if (validate && !single) {
+        // several chunks: the whole batch is checked before anything is written
+        int rc = validate_locked(ix, vecs, n);
+        if (rc != ORX_OK) return rc;
+    }
     CK(ix->d_flag.ensure(1));
     CK(ix->h_flag.ensure(1));
     if (!on_dev) CK(ix->stage.ensure(chunk * ORX_DIM));
-    const bool single = n <= chunk;           // one chunk: staged once, validated and committed back to back
-
     CK(cudaMemsetAsync(ix->d_flag.p, 0, sizeof(int), st));
-    if (validate && !single) {
-        // several chunks: the whole batch is checked before anything is written
-        for (uint64_t s = 0; s < n; s += chunk) {
-            const uint64_t m = std::min(chunk, n - s);
-            const float *src = vecs + s * ORX_DIM;
-            if (!on_dev) {
-                CK(cudaMemcpyAsync(ix->stage.p, src, m * ORX_DIM * sizeof(float), cudaMemcpyHostToDevice, st));
-                src = ix->stage.p;
-            }
-            orx::launch_validate_rows(src, m, ix->d_flag.p, st);
-            ix->stats.kernel_launches += 1;
-        }
-        CK(cudaMemcpyAsync(ix->h_flag.p, ix->d_flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        CK(cudaGetLastError());
-        if (*ix->h_flag.p) return fail(ORX_ERR_NONFINITE, "NaN or infinite value not allowed in vector");
-    }
 
     CK(ix->d_src_idx.ensure(chunk));
     CK(ix->d_dst_row.ensure(chunk));
@@ -570,9 +589,9 @@ struct SearchCtx {          // where a search's results go and how its completio
     orx::PublishArgs pub;
     orx::DoneArgs done;
 };
-SearchCtx plain_ctx(orx_id *ids, double *dist, int *counts, int *flags) {      // no publish, no completion word
+SearchCtx plain_ctx(const orx::ResultOut &out) {      // no publish, no completion word
     SearchCtx c{};
-    c.out = orx::ResultOut{ids, dist, counts, flags};
+    c.out = out;
     return c;
 }
 
@@ -604,7 +623,9 @@ int exhaustive_query(orx_index *ix, const float *q_src, int qi, int k, double dk
     return ORX_OK;
 }
 
-int gemv_pass(orx_index *ix, const float *q_src, int q0, int nq, int k, const SearchCtx &ctx) {
+// f: a filter with a bitmap -- the sequential scan skips the rows whose bit is clear (HBM traffic = eligible rows only)
+int gemv_pass(orx_index *ix, const float *q_src, int q0, int nq, int k, const SearchCtx &ctx,
+              const FilterOnDevice *f = nullptr) {
     const uint32_t n_rows = (uint32_t)ix->n_live;
     const int grid = orx::scan_gemv_grid(ix->device, n_rows);
     const double eps = ix->dtype == ORX_DTYPE_F32 ? orx::EPS_GEMV_F32 : orx::EPS_GEMV_BF16;
@@ -613,20 +634,25 @@ int gemv_pass(orx_index *ix, const float *q_src, int q0, int nq, int k, const Se
         const int m = std::min(GEMV_QCHUNK, nq - s);
         const int qa = q0 + s;
         // several queries: the batched kernel (8 queries share every row through shared memory); one: the streaming kernel
-        const int parts = m >= 2 ? orx::scan_gemv_batch_parts(ix->device, n_rows, m) : grid;
+        const int parts = !f && m >= 2 ? orx::scan_gemv_batch_parts(ix->device, n_rows, m) : grid;
         CK(ix->cur->partial.ensure((size_t)m * parts * 32 * slots));
         cudaEvent_t e0 = scan_event(ix), e1 = scan_event(ix);
         if (e0 && e1) CK(cudaEventRecord(e0, ix->stream));
-        if (m >= 2)
+        if (f)
+            orx::launch_scan_gemv_filtered(ix->dtype, ix->table, ix->scale, n_rows, f->bits,
+                                           ix->cur->qhat.p + (size_t)qa * ORX_DIM, m, slots, ix->cur->partial.p, grid,
+                                           ix->stream);
+        else if (m >= 2)
             orx::launch_scan_gemv_batch(ix->dtype, ix->table, ix->scale, n_rows, ix->cur->qhat.p + (size_t)qa * ORX_DIM, m,
                                         slots, ix->cur->partial.p, parts, ix->stream);
         else
             orx::launch_scan_gemv(ix->dtype, ix->table, ix->scale, n_rows, ix->cur->qhat.p + (size_t)qa * ORX_DIM, m,
                                   slots, ix->cur->partial.p, grid, ix->stream);
         if (e0 && e1) CK(cudaEventRecord(e1, ix->stream));
+        // a filter's row bound is the eligible count: "every eligible row is a candidate" when it fits the list
         orx::launch_finalize(ix->dtype, ix->table, ix->n2, ix->row_ids, q_src + (size_t)qa * ORX_DIM,
-                             ix->cur->prep.p + qa, ix->cur->partial.p, parts, slots, m, k, n_rows, eps, ctx.out, qa, ctx.pub,
-                             ctx.done, ix->stream);
+                             ix->cur->prep.p + qa, ix->cur->partial.p, parts, slots, m, k, f ? f->m : n_rows, eps, ctx.out,
+                             qa, ctx.pub, ctx.done, ix->stream);
         ix->stats.kernel_launches += 2;
     }
     CK(cudaGetLastError());
@@ -681,19 +707,30 @@ int stage_queries(orx_index *ix, const float *queries, int nq, const float **q_s
 }
 
 // ---- the scan + finalize of all nq queries (tcgen05 for batches, GEMV otherwise); *path = 1 / 2
-int scan_pass(orx_index *ix, const float *q_src, int nq, int k, const SearchCtx &ctx, int *path) {
+//      f: a filter with a bitmap.  A BATCH of filtered queries whose bitmap scans together would read more than the
+//      whole table takes ONE tcgen05 pass over all rows instead: the predicate enters through the per-row scale (a
+//      cleared bit -> the "never a candidate" marker), so the kernel and its candidate proof are those of orx_search.
+int scan_pass(orx_index *ix, const float *q_src, int nq, int k, const SearchCtx &ctx, int *path,
+              const FilterOnDevice *f = nullptr) {
     const uint32_t n_rows = (uint32_t)ix->n_live;
-    if (ix->cur->umma && orx::umma_should_use(ix->cur->umma, nq, k, n_rows)) {
+    if (ix->cur->umma && orx::umma_should_use(ix->cur->umma, nq, k, n_rows) && (!f || (uint64_t)nq * f->m >= n_rows)) {
+        const float *scale = ix->scale;
+        if (f) {
+            CK(ix->scale_masked.ensure(n_rows));
+            orx::launch_mask_scale(ix->scale, f->bits, n_rows, ix->scale_masked.p, ix->stream);
+            ix->stats.kernel_launches += 1;
+            scale = ix->scale_masked.p;
+        }
         *path = 2;
         cudaEvent_t e0 = scan_event(ix), e1 = scan_event(ix);
-        int rc = orx::umma_search(ix->cur->umma, ix->dtype, ix->table, ix->scale, ix->n2, ix->row_ids, n_rows,
+        int rc = orx::umma_search(ix->cur->umma, ix->dtype, ix->table, scale, ix->n2, ix->row_ids, n_rows,
                                   q_src, ix->cur->qhat.p, ix->cur->qhat16.p, ix->cur->prep.p, nq, k, ctx.out, ctx.pub, ctx.done,
                                   ix->stream, &ix->stats.kernel_launches, e0, e1);
         if (rc != ORX_OK) return fail(rc, "tcgen05 scan failed: %s", orx::umma_last_error());
         return ORX_OK;
     }
     *path = 1;
-    return gemv_pass(ix, q_src, 0, nq, k, ctx);
+    return gemv_pass(ix, q_src, 0, nq, k, ctx, f);
 }
 
 // ---- completion of the search whose last kernel writes `token` into the mapped completion word: the host polls the
@@ -733,12 +770,57 @@ int ensure_signalling(orx_index *ix) {
     return ORX_OK;
 }
 
+// ---- where a search's results land: the caller's device arrays, or the slot's mapped pinned staging (the kernels write
+//      it over PCIe) that deliver_results copies into the caller's host arrays after the wait.  Flags always go to the
+//      staging.
+int prepare_results(SearchSlot *sl, int nq, int k, bool on_dev, orx_id *ids, double *dist, int *counts,
+                    orx::ResultOut *out) {
+    const size_t nk = (size_t)nq * k;
+    CK(sl->h_flags.ensure(nq));
+    if (!on_dev) {
+        CK(sl->h_ids.ensure(nk));
+        CK(sl->h_dist.ensure(nk));
+        CK(sl->h_counts.ensure(nq));
+    }
+    *out = on_dev ? orx::ResultOut{ids, dist, counts, sl->h_flags.p}
+                  : orx::ResultOut{sl->h_ids.p, sl->h_dist.p, sl->h_counts.p, sl->h_flags.p};
+    return ORX_OK;
+}
+void deliver_results(const SearchSlot *sl, int nq, int k, bool on_dev, orx_id *ids, double *dist, int *counts) {
+    if (on_dev) return;
+    const size_t nk = (size_t)nq * k;
+    memcpy(ids, sl->h_ids.p, nk * sizeof(orx_id));
+    memcpy(dist, sl->h_dist.p, nk * sizeof(double));
+    memcpy(counts, sl->h_counts.p, nq * sizeof(int));
+}
+int outputs_on_device(const orx_id *ids, const double *dist, const int *counts, bool *on_dev) {
+    *on_dev = is_device_ptr(ids);
+    if (*on_dev != is_device_ptr(dist) || *on_dev != is_device_ptr(counts))
+        return fail(ORX_ERR_INVALID, "out_ids, out_dist and out_counts must all be host or all be device");
+    return ORX_OK;
+}
+
+// ---- the verdict of a finished search from the flags on the host (bit 1: non-finite query; bit 3: a peer failed) and,
+//      when `peer` names the other parties of a sharded search, the merge's timeout word.  *unproven: a query has bit 0.
+int search_verdict(const SearchSlot *sl, int nq, const char *peer, bool *unproven) {
+    if (peer && sl->h_done.p[1]) return fail(ORX_ERR_CUDA, "%s did not publish its candidates within 10 s", peer);
+    bool any = false;
+    for (int j = 0; j < nq; ++j) {
+        const int f = sl->h_flags.p[j];
+        if (peer && (f & 8)) return fail(ORX_ERR_CUDA, "%s failed (query %d)", peer, j);
+        if (f & 2) return fail(ORX_ERR_NONFINITE, "NaN or infinite value not allowed in vector (query %d)", j);
+        any |= (f & 1) != 0;
+    }
+    *unproven = any;
+    return ORX_OK;
+}
+
 // ---- re-answer the queries whose flag bit 0 (unproven) is set.  `flags` is where the kernels
 //      write (device or mapped host); hflags is a host-readable copy, refreshed here as needed.
 int resolve_unproven(orx_index *ix, const float *q_src, int nq, int k, const orx::ResultOut &out,
                      int *hflags, int path, bool host_readable) {
     int *flags = out.flags;
-    const SearchCtx ctx = plain_ctx(out.ids, out.dist, out.counts, out.flags);
+    const SearchCtx ctx = plain_ctx(out);
     cudaStream_t st = ix->stream;
     // level 1: coarse tensor-core pass unproven -> exact fp32 scan for those queries
     if (path == 2) {
@@ -799,17 +881,9 @@ int search_submit_locked(orx_index *ix, const float *queries, int nq, int k, orx
     const size_t nk = (size_t)nq * k;
     ix->cur->scan_ev_used = 0;
 
-    CK(ix->cur->h_flags.ensure(nq));
-    if (!out_on_dev) {
-        CK(ix->cur->h_ids.ensure(nk));
-        CK(ix->cur->h_dist.ensure(nk));
-        CK(ix->cur->h_counts.ensure(nq));
-    }
-    // host-side results are written by the kernels straight into mapped pinned memory
-    int *flags = ix->cur->h_flags.p;
-    const orx::ResultOut out{out_on_dev ? out_ids : ix->cur->h_ids.p, out_on_dev ? out_dist : ix->cur->h_dist.p,
-                             out_on_dev ? out_counts : ix->cur->h_counts.p, flags};
-    int rc = ensure_signalling(ix);
+    int rc = prepare_results(ix->cur, nq, k, out_on_dev, out_ids, out_dist, out_counts, &pd.out);
+    if (rc != ORX_OK) return rc;
+    rc = ensure_signalling(ix);
     if (rc != ORX_OK) return rc;
 
     rc = stage_queries(ix, queries, nq, &pd.q_src);
@@ -838,8 +912,7 @@ int search_submit_locked(orx_index *ix, const float *queries, int nq, int k, orx
         pd.complete = true;
         return ORX_OK;
     }
-    SearchCtx ctx{};
-    ctx.out = out;
+    SearchCtx ctx = plain_ctx(pd.out);
     pd.token = next_token(ix);
     ctx.done = orx::DoneArgs{ix->cur->d_counters.p, (unsigned int)nq, ix->cur->h_done.p, pd.token};
     rc = scan_pass(ix, pd.q_src, nq, k, ctx, &pd.path);
@@ -850,46 +923,6 @@ int search_submit_locked(orx_index *ix, const float *queries, int nq, int k, orx
         return rc;
     }
     pd.active = true;
-    return ORX_OK;
-}
-
-int search_wait_locked(orx_index *ix) {
-    SearchSlot::Pending &pd = ix->cur->pend;
-    if (!pd.active) return fail(ORX_ERR_INVALID, "no search in flight under this ticket");
-    pd.active = false;
-    if (pd.settled) {
-        if (pd.settled_rc != ORX_OK) g_err = pd.settled_err;
-        return pd.settled_rc;
-    }
-    const int nq = pd.nq, k = pd.k;
-    if (!pd.complete) {
-        const size_t nk = (size_t)nq * k;
-        int *flags = ix->cur->h_flags.p;
-        const orx::ResultOut out{pd.out_on_dev ? pd.out_ids : ix->cur->h_ids.p, pd.out_on_dev ? pd.out_dist : ix->cur->h_dist.p,
-                                 pd.out_on_dev ? pd.out_counts : ix->cur->h_counts.p, flags};
-        int rc = wait_done(ix, pd.token);       // the last finalize CTA wrote the completion word; flags are on the host
-        if (rc != ORX_OK) return rc;
-        bool any_unproven = false;
-        for (int j = 0; j < nq; ++j) {
-            if (flags[j] & 2) return fail(ORX_ERR_NONFINITE, "NaN or infinite value not allowed in vector (query %d)", j);
-            any_unproven |= (flags[j] & 1) != 0;
-        }
-        if (any_unproven) {
-            rc = resolve_unproven(ix, pd.q_src, nq, k, out, flags, pd.path, /*host_readable=*/!pd.out_on_dev);
-            if (rc != ORX_OK) return rc;
-        }
-        if (!pd.out_on_dev) {
-            memcpy(pd.out_ids, ix->cur->h_ids.p, nk * sizeof(orx_id));
-            memcpy(pd.out_dist, ix->cur->h_dist.p, nk * sizeof(double));
-            memcpy(pd.out_counts, ix->cur->h_counts.p, nq * sizeof(int));
-        }
-        harvest_scan_events(ix);
-        ix->stats.last_path = pd.path;
-    }
-    ix->stats.last_search_ms =
-        std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - pd.t_begin).count();
-    ix->stats.searches += 1;
-    ix->stats.queries += nq;
     return ORX_OK;
 }
 
@@ -904,27 +937,10 @@ int claim_slot(orx_index *ix, int *ticket) {
 }
 bool any_in_flight(const orx_index *ix) { return ix->slot[0].pend.active || ix->slot[1].pend.active; }
 
-int search_locked(orx_index *ix, const float *queries, int nq, int k, orx_id *out_ids, double *out_dist,
-                  int *out_counts) {
-    int rc = claim_slot(ix, nullptr);
-    if (rc != ORX_OK) return rc;
-    rc = search_submit_locked(ix, queries, nq, k, out_ids, out_dist, out_counts);
-    if (rc != ORX_OK) return rc;
-    ix->tickets += 1;
-    return search_wait_locked(ix);
-}
-
-
 // =========================================================================== filtered search
-struct FilterOnDevice {          // a resolved predicate: the eligible rows, as a sorted list and (when large) a bitmap
-    uint32_t m;
-    const uint32_t *list;        // [m] device
-    const uint32_t *count;       // device word holding m
-    const uint32_t *bits;        // [(n_live+31)/32] device, or null: rescore the list, no scan
-};
-
-int check_filtered_args(orx_index *ix, const float *queries, int nq, int dim, int k, orx_id *out_ids, double *out_dist,
-                        int *out_counts) {
+// the arguments every search form checks (an empty batch is valid: nothing to do)
+int check_query_args(orx_index *ix, const float *queries, int nq, int dim, int k, orx_id *out_ids, double *out_dist,
+                     int *out_counts) {
     if (!ix) return fail(ORX_ERR_INVALID, "index is null");
     if (dim != ORX_DIM) return fail(ORX_ERR_DIM, "different vector dimensions %d and %d", ORX_DIM, dim);
     if (k < 1 || k > ORX_MAX_K) return fail(ORX_ERR_INVALID, "k must be in [1, %d], got %d", ORX_MAX_K, k);
@@ -932,17 +948,6 @@ int check_filtered_args(orx_index *ix, const float *queries, int nq, int dim, in
     if (nq == 0) return ORX_OK;
     if (!queries || !out_ids || !out_dist || !out_counts) return fail(ORX_ERR_INVALID, "null argument");
     return ORX_OK;
-}
-
-// the eligible rows: ids that are live, each row once (the WHERE clause of the SQL), ascending
-void resolve_allow_ids(const orx_index *ix, const orx_id *ids, uint64_t n, std::vector<uint32_t> &rows) {
-    rows.clear();
-    rows.reserve(n);
-    for (uint64_t i = 0; i < n; ++i) {
-        if (const uint32_t *r = ix->map.find(ids[i])) rows.push_back(*r);
-    }
-    std::sort(rows.begin(), rows.end());
-    rows.erase(std::unique(rows.begin(), rows.end()), rows.end());
 }
 
 int upload_filter(orx_index *ix, const std::vector<uint32_t> &rows, DevBuf<uint32_t> &list, DevBuf<uint32_t> &count,
@@ -967,28 +972,40 @@ int upload_filter(orx_index *ix, const std::vector<uint32_t> &rows, DevBuf<uint3
     return ORX_OK;
 }
 
+// the eligible rows of `ids` -- ids that are live, each row once (the WHERE clause of the SQL), ascending -- uploaded
+// into list / count / bits
+int resolve_filter(orx_index *ix, const orx_id *ids, uint64_t n, DevBuf<uint32_t> &list, DevBuf<uint32_t> &count,
+                   DevBuf<uint32_t> &bits, FilterOnDevice *out) {
+    std::vector<uint32_t> rows;
+    rows.reserve(n);
+    for (uint64_t i = 0; i < n; ++i) {
+        if (const uint32_t *r = ix->map.find(ids[i])) rows.push_back(*r);
+    }
+    std::sort(rows.begin(), rows.end());
+    rows.erase(std::unique(rows.begin(), rows.end()), rows.end());
+    int rc = upload_filter(ix, rows, list, count, bits);
+    if (rc != ORX_OK) return rc;
+    const uint32_t m = (uint32_t)rows.size();
+    *out = FilterOnDevice{m, list.p, count.p, m >= FILTER_SCAN_MIN_ROWS ? bits.p : nullptr};
+    return ORX_OK;
+}
+
 int filtered_search_locked(orx_index *ix, const FilterOnDevice &f, const float *queries, int nq, int k, orx_id *out_ids,
                            double *out_dist, int *out_counts) {
     cudaStream_t st = ix->stream;
-    const bool out_on_dev = is_device_ptr(out_ids);
-    if (out_on_dev != is_device_ptr(out_dist) || out_on_dev != is_device_ptr(out_counts))
-        return fail(ORX_ERR_INVALID, "out_ids, out_dist and out_counts must all be host or all be device");
-    const size_t nk = (size_t)nq * k;
+    bool out_on_dev = false;
+    int rc = outputs_on_device(out_ids, out_dist, out_counts, &out_on_dev);
+    if (rc != ORX_OK) return rc;
     const uint32_t m = f.m;
 
     const float *q_src = nullptr;
-    int rc = stage_queries(ix, queries, nq, &q_src);
+    rc = stage_queries(ix, queries, nq, &q_src);
     if (rc != ORX_OK) return rc;
     CK(ix->cur->h_prep.ensure(nq));
     CK(cudaMemcpyAsync(ix->cur->h_prep.p, ix->cur->prep.p, nq * sizeof(orx::QueryPrep), cudaMemcpyDeviceToHost, st));
-    if (!out_on_dev) {
-        CK(ix->cur->h_ids.ensure(nk));
-        CK(ix->cur->h_dist.ensure(nk));
-        CK(ix->cur->h_counts.ensure(nq));
-    }
-    CK(ix->cur->h_flags.ensure(nq));
-    const orx::ResultOut out{out_on_dev ? out_ids : ix->cur->h_ids.p, out_on_dev ? out_dist : ix->cur->h_dist.p,
-                             out_on_dev ? out_counts : ix->cur->h_counts.p, ix->cur->h_flags.p};
+    orx::ResultOut out;
+    rc = prepare_results(ix->cur, nq, k, out_on_dev, out_ids, out_dist, out_counts, &out);
+    if (rc != ORX_OK) return rc;
     CK(ix->fb_dist.ensure(std::max<size_t>(m, 1)));
     // exact by construction: every eligible row is rescored canonically and the k best are selected
     auto list_query = [&](int j) {
@@ -999,61 +1016,22 @@ int filtered_search_locked(orx_index *ix, const FilterOnDevice &f, const float *
                                 out.dist + (size_t)j * k, out.counts + j, st);
         ix->stats.kernel_launches += m ? 2 : 1;
     };
-    const int slots = orx::slots_for_k(k);
-    const uint32_t n_live = (uint32_t)ix->n_live;
-    // the unproven queries of either scan are re-answered exactly from the eligible list
-    auto redo_unproven = [&]() {
+    if (f.bits != nullptr && m > 32u * (uint32_t)orx::slots_for_k(k)) {
+        // many eligible rows: a scan restricted to them, with the candidate proof of orx_search; the rare unproven
+        // query is re-answered by the exact list path
+        ix->cur->scan_ev_used = 0;
+        int path = 1;
+        rc = scan_pass(ix, q_src, nq, k, plain_ctx(out), &path, &f);
+        if (rc != ORX_OK) return rc;
+        CK(cudaStreamSynchronize(st));
+        CK(cudaGetLastError());
+        harvest_scan_events(ix);
+        ix->stats.last_path = path;
         for (int j = 0; j < nq; ++j) {
             if (!(ix->cur->h_flags.p[j] & 1) || (ix->cur->h_flags.p[j] & 2)) continue;
             ix->stats.fallback_exhaustive += 1;
             list_query(j);
         }
-    };
-    if (f.bits != nullptr && m > 32u * (uint32_t)slots && ix->cur->umma &&
-        orx::umma_should_use(ix->cur->umma, nq, k, n_live) && (uint64_t)nq * m >= (uint64_t)n_live) {
-        // a BATCH of filtered queries whose bitmap scans together would read more than the whole table: ONE tcgen05 pass
-        // over all rows instead.  The predicate enters through the per-row scale (a cleared bit -> the "never a candidate"
-        // marker), so the kernel and its candidate proof are those of orx_search.
-        CK(ix->scale_masked.ensure(n_live));
-        orx::launch_mask_scale(ix->scale, f.bits, n_live, ix->scale_masked.p, st);
-        ix->stats.kernel_launches += 1;
-        ix->cur->scan_ev_used = 0;
-        cudaEvent_t e0 = scan_event(ix), e1 = scan_event(ix);
-        rc = orx::umma_search(ix->cur->umma, ix->dtype, ix->table, ix->scale_masked.p, ix->n2, ix->row_ids, n_live, q_src,
-                              ix->cur->qhat.p, ix->cur->qhat16.p, ix->cur->prep.p, nq, k, out, orx::PublishArgs{}, orx::DoneArgs{},
-                              st, &ix->stats.kernel_launches, e0, e1);
-        if (rc != ORX_OK) return fail(rc, "tcgen05 scan failed: %s", orx::umma_last_error());
-        CK(cudaStreamSynchronize(st));
-        CK(cudaGetLastError());
-        harvest_scan_events(ix);
-        ix->stats.last_path = 2;
-        redo_unproven();
-    } else if (f.bits != nullptr && m > 32u * (uint32_t)slots) {
-        // many eligible rows: the predicate is a row bitmap and the sequential scan skips the rows whose
-        // bit is clear (HBM traffic = eligible rows only); same candidate proof as orx_search, the rare
-        // unproven query is re-answered by the exact list path.
-        const uint32_t n_rows = (uint32_t)ix->n_live;
-        const int grid = orx::scan_gemv_grid(ix->device, n_rows);
-        const double eps = ix->dtype == ORX_DTYPE_F32 ? orx::EPS_GEMV_F32 : orx::EPS_GEMV_BF16;
-        ix->cur->scan_ev_used = 0;
-        for (int s0 = 0; s0 < nq; s0 += GEMV_QCHUNK) {
-            const int mq = std::min(GEMV_QCHUNK, nq - s0);
-            CK(ix->cur->partial.ensure((size_t)mq * grid * 32 * slots));
-            cudaEvent_t e0 = scan_event(ix), e1 = scan_event(ix);
-            if (e0 && e1) CK(cudaEventRecord(e0, st));
-            orx::launch_scan_gemv_filtered(ix->dtype, ix->table, ix->scale, n_rows, f.bits,
-                                           ix->cur->qhat.p + (size_t)s0 * ORX_DIM, mq, slots, ix->cur->partial.p, grid, st);
-            if (e0 && e1) CK(cudaEventRecord(e1, st));
-            // n_rows argument = the eligible count: "every eligible row is a candidate" when it fits the list
-            orx::launch_finalize(ix->dtype, ix->table, ix->n2, ix->row_ids, q_src + (size_t)s0 * ORX_DIM, ix->cur->prep.p + s0,
-                                 ix->cur->partial.p, grid, slots, mq, k, m, eps, out, s0, orx::PublishArgs{}, orx::DoneArgs{}, st);
-            ix->stats.kernel_launches += 2;
-        }
-        CK(cudaStreamSynchronize(st));
-        CK(cudaGetLastError());
-        harvest_scan_events(ix);
-        ix->stats.last_path = 1;
-        redo_unproven();
     } else {
         // few rows: no scan at all
         for (int j = 0; j < nq; ++j) list_query(j);
@@ -1063,11 +1041,7 @@ int filtered_search_locked(orx_index *ix, const FilterOnDevice &f, const float *
     for (int j = 0; j < nq; ++j)
         if (ix->cur->h_prep.p[j].nonfinite)
             return fail(ORX_ERR_NONFINITE, "NaN or infinite value not allowed in vector (query %d)", j);
-    if (!out_on_dev) {
-        memcpy(out_ids, ix->cur->h_ids.p, nk * sizeof(orx_id));
-        memcpy(out_dist, ix->cur->h_dist.p, nk * sizeof(double));
-        memcpy(out_counts, ix->cur->h_counts.p, nq * sizeof(int));
-    }
+    deliver_results(ix->cur, nq, k, out_on_dev, out_ids, out_dist, out_counts);
     ix->stats.searches += 1;
     ix->stats.queries += nq;
     return ORX_OK;
@@ -1077,15 +1051,12 @@ int filtered_search_locked(orx_index *ix, const FilterOnDevice &f, const float *
 // import)
 int filter_on_device(orx_index *ix, orx_filter *f, FilterOnDevice *out) {
     if (!f->resolved || f->generation != ix->generation) {
-        std::vector<uint32_t> rows;
-        resolve_allow_ids(ix, f->ids.data(), f->ids.size(), rows);
-        int rc = upload_filter(ix, rows, f->d_list, f->d_count, f->d_bits);
+        int rc = resolve_filter(ix, f->ids.data(), f->ids.size(), f->d_list, f->d_count, f->d_bits, &f->dev);
         if (rc != ORX_OK) return rc;
-        f->m = (uint32_t)rows.size();
         f->generation = ix->generation;
         f->resolved = true;
     }
-    *out = FilterOnDevice{f->m, f->d_list.p, f->d_count.p, f->m >= FILTER_SCAN_MIN_ROWS ? f->d_bits.p : nullptr};
+    *out = f->dev;
     return ORX_OK;
 }
 
@@ -1101,14 +1072,11 @@ using MmrGather = std::function<int(const orx_id *ids, const int *cnt, int m, co
 
 int check_mmr_args(orx_index *ix, const float *queries, int nq, int dim, int k, int fetch_k, double lam,
                    orx_id *out_ids, double *out_dist, int *out_counts) {
-    if (!ix) return fail(ORX_ERR_INVALID, "index is null");
-    if (dim != ORX_DIM) return fail(ORX_ERR_DIM, "different vector dimensions %d and %d", ORX_DIM, dim);
     if (k < 1 || fetch_k < k || fetch_k > ORX_MAX_K)
         return fail(ORX_ERR_INVALID, "need 1 <= k <= fetch_k <= %d, got k = %d, fetch_k = %d", ORX_MAX_K, k, fetch_k);
     if (!(lam >= 0.0 && lam <= 1.0)) return fail(ORX_ERR_INVALID, "lambda_mult must be a number in [0, 1], got %g", lam);
-    if (nq < 0) return fail(ORX_ERR_INVALID, "nq must be >= 0");
-    if (nq == 0) return ORX_OK;
-    if (!queries || !out_ids || !out_dist || !out_counts) return fail(ORX_ERR_INVALID, "null argument");
+    int rc = check_query_args(ix, queries, nq, dim, k, out_ids, out_dist, out_counts);
+    if (rc != ORX_OK || nq == 0) return rc;
     if (is_device_ptr(queries) || is_device_ptr(out_ids) || is_device_ptr(out_dist) || is_device_ptr(out_counts))
         return fail(ORX_ERR_INVALID, "MMR search takes host queries and host outputs");
     return ORX_OK;
@@ -1190,18 +1158,43 @@ int mmr_local(orx_index *ix, const float *queries, int nq, int k, int fetch_k, d
 }
 
 // =========================================================================== sharded search
-// Layout of one rank's result block for (nq, k): ids | dist | counts | flags (16-byte padded).
-struct SlotLayout {
-    size_t dist_off, counts_off, flags_off, bytes;
-};
-SlotLayout slot_layout(int nq, int k) {
-    SlotLayout L;
-    L.dist_off = (size_t)nq * k * sizeof(orx_id);
-    L.counts_off = L.dist_off + (size_t)nq * k * sizeof(double);
-    L.flags_off = L.counts_off + (size_t)nq * sizeof(int);
-    L.bytes = (L.flags_off + (size_t)nq * sizeof(int) + 15) & ~(size_t)15;
-    return L;
+// The gather buffer of `world` ranks: two sets of `world` slots (one slot = a rank's block of up to XQ_MAX x 32
+// results), then 2 x world arrival words.  Returns its size.
+size_t exchange_layout(Exchange *x, int world, int rank) {
+    x->world = world;
+    x->rank = rank;
+    x->slot_bytes = slot_layout(XQ_MAX, 32).bytes;          // nq * k <= XQ_MAX * 32 per exchange round
+    x->set_bytes = x->slot_bytes * world;
+    x->flags_off = 2 * x->set_bytes;
+    return x->flags_off + 2 * (size_t)world * XFLAG_STRIDE;
 }
+// d_peer_slot / d_peer_flag of both sets: my slot and my arrival word inside each target's gather buffer (every rank's,
+// or the group root's), allocated on the current device
+cudaError_t upload_peer_tables(Exchange *x, const std::vector<char *> &targets) {
+    const int n = (int)targets.size();
+    x->n_targets = n;
+    std::vector<void *> slots(n);
+    std::vector<uint32_t *> flags(n);
+    for (int s = 0; s < 2; ++s) {
+        for (int t = 0; t < n; ++t) {
+            slots[t] = targets[t] + (size_t)s * x->set_bytes + (size_t)x->rank * x->slot_bytes;
+            flags[t] = reinterpret_cast<uint32_t *>(targets[t] + x->flags_off + ((size_t)s * x->world + x->rank) * XFLAG_STRIDE);
+        }
+        cudaError_t e = cudaMalloc(&x->d_peer_slot[s], n * sizeof(void *));
+        if (e == cudaSuccess) e = cudaMalloc(&x->d_peer_flag[s], n * sizeof(uint32_t *));
+        if (e == cudaSuccess) e = cudaMemcpy(x->d_peer_slot[s], slots.data(), n * sizeof(void *), cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) e = cudaMemcpy(x->d_peer_flag[s], flags.data(), n * sizeof(uint32_t *), cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+// Queries per exchange round at this k (a slot holds XQ_MAX of them at k <= 32), or 0 when one round cannot hold
+// world x k candidates per query.
+int exchange_queries(size_t world, int k) {
+    if (world * k > 1024) return 0;
+    return k <= 32 ? XQ_MAX : XQ_MAX * 32 / k;
+}
+
 // merge what every rank published under `seq` into the caller's result arrays; the last merge CTA writes `token`
 int launch_shard_merge(orx_index *ix, Exchange *x, int nq, int k, const orx::ResultOut &final_out, const SlotLayout &L,
                        uint32_t seq, uint32_t token) {
@@ -1226,6 +1219,23 @@ int launch_shard_publish(orx_index *ix, Exchange *x, const SlotLayout &L, uint32
     return ORX_OK;
 }
 
+// Publish a zeroed block from the slot's scratch (the shard may own no local slot) in place of this shard's results
+// under `seq`.  Its flags carry the query check (`prep`: an empty shard) or, with prep null, bit 3 (this shard failed:
+// whoever merges fails fast instead of waiting for it).
+cudaError_t publish_substitute(orx_index *ix, Exchange *x, const SlotLayout &L, int nq, uint32_t seq,
+                               const orx::QueryPrep *prep) {
+    cudaStream_t st = ix->stream;
+    cudaError_t e = ix->cur->blk.ensure((L.bytes + 7) / 8);
+    if (e != cudaSuccess) return e;
+    char *blk = reinterpret_cast<char *>(ix->cur->blk.p);
+    int *flags = reinterpret_cast<int *>(blk + L.flags_off);
+    cudaMemsetAsync(blk, 0, L.bytes, st);
+    if (prep) orx::launch_flags_from_prep(prep, nq, flags, st);
+    else orx::launch_fill_flags(flags, nq, 8, st);
+    orx::launch_publish(blk, x->d_peer_slot[seq & 1], x->d_peer_flag[seq & 1], x->n_targets, L.bytes, seq, st);
+    return cudaGetLastError();
+}
+
 // Round 1 of a row-sharded search on ONE shard, launches only (no wait): stage the batch, scan, finalize pushes the
 // shard's block into its targets' gather buffers under `seq`.  On failure the shard still publishes a block whose flags
 // carry bit 3, so that whoever merges fails fast instead of waiting for it.
@@ -1239,13 +1249,9 @@ int shard_round1(orx_index *ix, Exchange *x, const float *queries, bool src_pinn
     if (rc == ORX_OK) {
         if (ix->n_live == 0) {
             // an empty shard contributes nothing (its peers may still hold rows); flags carry the query check
-            CK(ix->cur->blk.ensure((L.bytes + 7) / 8));         // scratch block: the shard may own no local slot
-            char *blk = reinterpret_cast<char *>(ix->cur->blk.p);
-            cudaMemsetAsync(blk, 0, L.bytes, st);
-            orx::launch_flags_from_prep(ix->cur->prep.p, nq, reinterpret_cast<int *>(blk + L.flags_off), st);
-            orx::launch_publish(blk, x->d_peer_slot[set], x->d_peer_flag[set], x->n_targets, L.bytes, seq, st);
+            if (publish_substitute(ix, x, L, nq, seq, ix->cur->prep.p) != cudaSuccess)
+                rc = fail(ORX_ERR_CUDA, "publishing an empty shard's block failed");
             ix->stats.kernel_launches += 2;
-            if (cudaGetLastError() != cudaSuccess) rc = fail(ORX_ERR_CUDA, "publishing an empty shard's block failed");
         } else {
             SearchCtx ctx{};
             ctx.pub = orx::PublishArgs{reinterpret_cast<char *const *>(x->d_peer_slot[set]), x->d_peer_flag[set],
@@ -1258,12 +1264,7 @@ int shard_round1(orx_index *ix, Exchange *x, const float *queries, bool src_pinn
         const std::string why = g_err;
         cudaStreamSynchronize(st);
         if (ix->cur->d_counters.p) cudaMemsetAsync(ix->cur->d_counters.p, 0, 2 * sizeof(unsigned int), st);
-        if (ix->cur->blk.ensure((L.bytes + 7) / 8) == cudaSuccess) {
-            char *blk = reinterpret_cast<char *>(ix->cur->blk.p);
-            cudaMemsetAsync(blk, 0, L.bytes, st);
-            orx::launch_fill_flags(reinterpret_cast<int *>(blk + L.flags_off), nq, 8, st);
-            orx::launch_publish(blk, x->d_peer_slot[set], x->d_peer_flag[set], x->n_targets, L.bytes, seq, st);
-        }
+        publish_substitute(ix, x, L, nq, seq, nullptr);
         cudaStreamSynchronize(st);
         cudaGetLastError();
         g_err = why;
@@ -1282,126 +1283,114 @@ int sharded_submit_locked(orx_index *ix, Exchange *x, const float *queries, int 
     pd.out_ids = out_ids;
     pd.out_dist = out_dist;
     pd.out_counts = out_counts;
-    const bool out_on_dev = pd.out_on_dev = is_device_ptr(out_ids);
-    if (out_on_dev != is_device_ptr(out_dist) || out_on_dev != is_device_ptr(out_counts))
-        return fail(ORX_ERR_INVALID, "out_ids, out_dist and out_counts must all be host or all be device");
-    const size_t nk = (size_t)nq * k;
-    const SlotLayout L = slot_layout(nq, k);
-    if (L.bytes > x->slot_bytes) return fail(ORX_ERR_INVALID, "sharded search limited to %d queries per call", XQ_MAX);
-    pd.L = SlotLayoutPod{L.dist_off, L.counts_off, L.flags_off, L.bytes};
+    int rc = outputs_on_device(out_ids, out_dist, out_counts, &pd.out_on_dev);
+    if (rc != ORX_OK) return rc;
+    pd.L = slot_layout(nq, k);
+    if (pd.L.bytes > x->slot_bytes) return fail(ORX_ERR_INVALID, "sharded search limited to %d queries per call", XQ_MAX);
 
-    CK(ix->cur->h_flags.ensure(nq));
     CK(ix->cur->h_myflags.ensure(nq));
     CK(ix->cur->h_redo.ensure(1));
-    if (!out_on_dev) {
-        CK(ix->cur->h_ids.ensure(nk));
-        CK(ix->cur->h_dist.ensure(nk));
-        CK(ix->cur->h_counts.ensure(nq));
-    }
-    int rc = ensure_signalling(ix);
+    rc = prepare_results(ix->cur, nq, k, pd.out_on_dev, out_ids, out_dist, out_counts, &pd.out);
     if (rc != ORX_OK) return rc;
-    const orx::ResultOut final_out{out_on_dev ? out_ids : ix->cur->h_ids.p, out_on_dev ? out_dist : ix->cur->h_dist.p,
-                                   out_on_dev ? out_counts : ix->cur->h_counts.p, ix->cur->h_flags.p};
+    rc = ensure_signalling(ix);
+    if (rc != ORX_OK) return rc;
     *ix->cur->h_redo.p = 0;
     ix->cur->h_done.p[1] = 0;
 
     // ---- round 1: scan, finalize pushes my block into every rank's gather buffer, merge what arrives
     pd.seq = ++x->seq;
-    rc = shard_round1(ix, x, queries, false, nq, k, L, pd.seq, &pd.q_src, &pd.path);
+    rc = shard_round1(ix, x, queries, false, nq, k, pd.L, pd.seq, &pd.q_src, &pd.path);
     if (rc != ORX_OK) return rc;
     pd.token = next_token(ix);
-    rc = launch_shard_merge(ix, x, nq, k, final_out, L, pd.seq, pd.token);
+    rc = launch_shard_merge(ix, x, nq, k, pd.out, pd.L, pd.seq, pd.token);
     if (rc != ORX_OK) return rc;
     pd.active = true;
     return ORX_OK;
 }
 
-int sharded_wait_locked(orx_index *ix, Exchange *x) {
+// ---- the wait of a search submitted on `ix->cur` (one GPU, or one rank of the row-sharded search): poll the completion
+//      word, check the flags, settle unproven queries, hand the results over
+int search_wait_locked(orx_index *ix) {
     SearchSlot::Pending &pd = ix->cur->pend;
-    if (!pd.active || !pd.sharded) return fail(ORX_ERR_INVALID, "no sharded search in flight under this ticket");
+    if (!pd.active) return fail(ORX_ERR_INVALID, "no search in flight under this ticket");
     pd.active = false;
     if (pd.settled) {
         if (pd.settled_rc != ORX_OK) g_err = pd.settled_err;
         return pd.settled_rc;
     }
-    cudaStream_t st = ix->stream;
     const int nq = pd.nq, k = pd.k;
-    const size_t nk = (size_t)nq * k;
-    const bool out_on_dev = pd.out_on_dev;
-    SlotLayout L;
-    L.dist_off = pd.L.dist_off; L.counts_off = pd.L.counts_off; L.flags_off = pd.L.flags_off; L.bytes = pd.L.bytes;
-    const orx::ResultOut final_out{out_on_dev ? pd.out_ids : ix->cur->h_ids.p, out_on_dev ? pd.out_dist : ix->cur->h_dist.p,
-                                   out_on_dev ? pd.out_counts : ix->cur->h_counts.p, ix->cur->h_flags.p};
-    char *slot = x->base + (size_t)(pd.seq & 1) * x->set_bytes + (size_t)x->rank * x->slot_bytes;      // my block, local copy
-    int rc = wait_done(ix, pd.token);
-    if (rc != ORX_OK) return rc;
-    if (ix->cur->h_done.p[1]) return fail(ORX_ERR_CUDA, "sharded search: a peer rank did not publish its candidates within 10 s");
-
-    for (int j = 0; j < nq; ++j) {
-        if (ix->cur->h_flags.p[j] & 8) return fail(ORX_ERR_CUDA, "sharded search: a peer rank failed (query %d)", j);
-        if (ix->cur->h_flags.p[j] & 2)
-            return fail(ORX_ERR_NONFINITE, "NaN or infinite value not allowed in vector (query %d)", j);
-    }
-    if (*ix->cur->h_redo.p) {
-        // ---- round 2 (every rank sees the same redo word): ranks with unproven queries re-answer them
-        //      exactly, everybody republishes and merges again under the next sequence number.  (With another search in
-        //      flight that number selects the same buffer set as round 1 did; it is free again by then: this round is
-        //      stream-ordered behind the other search's merge, which needed every peer's publish, which every peer
-        //      issued after finishing ITS merge of round 1.)
-        const uint32_t seq2 = ++x->seq;
-        char *slot2 = x->base + (size_t)(seq2 & 1) * x->set_bytes + (size_t)x->rank * x->slot_bytes;
-        if (slot2 != slot) CK(cudaMemcpyAsync(slot2, slot, L.bytes, cudaMemcpyDeviceToDevice, st));
-        const orx::ResultOut mine2{reinterpret_cast<orx_id *>(slot2), reinterpret_cast<double *>(slot2 + L.dist_off),
-                                   reinterpret_cast<int *>(slot2 + L.counts_off), reinterpret_cast<int *>(slot2 + L.flags_off)};
-        bool mine_unproven = false;
-        for (int j = 0; j < nq; ++j) mine_unproven |= (ix->cur->h_myflags.p[j] & 1) != 0;
-        rc = ORX_OK;
-        if (mine_unproven && ix->n_live > 0)
-            rc = resolve_unproven(ix, pd.q_src, nq, k, mine2, ix->cur->h_myflags.p, pd.path, /*host_readable=*/false);
-        if (rc != ORX_OK) {
-            const std::string why = g_err;
-            orx::launch_fill_flags(mine2.flags, nq, 8, st);
-            launch_shard_publish(ix, x, L, seq2);
-            cudaStreamSynchronize(st);
-            cudaGetLastError();
-            g_err = why;
-            return rc;
+    if (!pd.complete) {
+        const char *peer = pd.sharded ? "sharded search: a peer rank" : nullptr;
+        int rc = wait_done(ix, pd.token);       // the last kernel wrote the completion word; flags are on the host
+        if (rc != ORX_OK) return rc;
+        bool unproven = false;
+        rc = search_verdict(ix->cur, nq, peer, &unproven);
+        if (rc != ORX_OK) return rc;
+        if (!pd.sharded && unproven) {
+            rc = resolve_unproven(ix, pd.q_src, nq, k, pd.out, ix->cur->h_flags.p, pd.path, /*host_readable=*/!pd.out_on_dev);
+            if (rc != ORX_OK) return rc;
         }
-        *ix->cur->h_redo.p = 0;
-        rc = launch_shard_publish(ix, x, L, seq2);
-        if (rc != ORX_OK) return rc;
-        const uint32_t token = next_token(ix);
-        rc = launch_shard_merge(ix, x, nq, k, final_out, L, seq2, token);
-        if (rc != ORX_OK) return rc;
-        rc = wait_done(ix, token);
-        if (rc != ORX_OK) return rc;
-        if (ix->cur->h_done.p[1]) return fail(ORX_ERR_CUDA, "sharded search: a peer rank did not publish its candidates within 10 s");
-        for (int j = 0; j < nq; ++j)
-            if (ix->cur->h_flags.p[j] & 8) return fail(ORX_ERR_CUDA, "sharded search: a peer rank failed (query %d)", j);
-        if (*ix->cur->h_redo.p) return fail(ORX_ERR_CUDA, "sharded search: a rank could not prove its candidates");
+        if (pd.sharded && *ix->cur->h_redo.p) {
+            // ---- round 2 (every rank sees the same redo word): ranks with unproven queries re-answer them
+            //      exactly, everybody republishes and merges again under the next sequence number.  (With another search in
+            //      flight that number selects the same buffer set as round 1 did; it is free again by then: this round is
+            //      stream-ordered behind the other search's merge, which needed every peer's publish, which every peer
+            //      issued after finishing ITS merge of round 1.)
+            Exchange *x = ix->xchg;
+            cudaStream_t st = ix->stream;
+            const SlotLayout &L = pd.L;
+            char *slot = x->base + (size_t)(pd.seq & 1) * x->set_bytes + (size_t)x->rank * x->slot_bytes;  // my block, local copy
+            const uint32_t seq2 = ++x->seq;
+            char *slot2 = x->base + (size_t)(seq2 & 1) * x->set_bytes + (size_t)x->rank * x->slot_bytes;
+            if (slot2 != slot) CK(cudaMemcpyAsync(slot2, slot, L.bytes, cudaMemcpyDeviceToDevice, st));
+            const orx::ResultOut mine2{reinterpret_cast<orx_id *>(slot2), reinterpret_cast<double *>(slot2 + L.dist_off),
+                                       reinterpret_cast<int *>(slot2 + L.counts_off), reinterpret_cast<int *>(slot2 + L.flags_off)};
+            bool mine_unproven = false;
+            for (int j = 0; j < nq; ++j) mine_unproven |= (ix->cur->h_myflags.p[j] & 1) != 0;
+            if (mine_unproven && ix->n_live > 0)
+                rc = resolve_unproven(ix, pd.q_src, nq, k, mine2, ix->cur->h_myflags.p, pd.path, /*host_readable=*/false);
+            if (rc != ORX_OK) {
+                const std::string why = g_err;
+                publish_substitute(ix, x, L, nq, seq2, nullptr);
+                ix->stats.kernel_launches += 1;
+                cudaStreamSynchronize(st);
+                cudaGetLastError();
+                g_err = why;
+                return rc;
+            }
+            *ix->cur->h_redo.p = 0;
+            rc = launch_shard_publish(ix, x, L, seq2);
+            if (rc != ORX_OK) return rc;
+            const uint32_t token = next_token(ix);
+            rc = launch_shard_merge(ix, x, nq, k, pd.out, L, seq2, token);
+            if (rc != ORX_OK) return rc;
+            rc = wait_done(ix, token);
+            if (rc != ORX_OK) return rc;
+            rc = search_verdict(ix->cur, nq, peer, &unproven);
+            if (rc != ORX_OK) return rc;
+            if (*ix->cur->h_redo.p) return fail(ORX_ERR_CUDA, "sharded search: a rank could not prove its candidates");
+        }
+        deliver_results(ix->cur, nq, k, pd.out_on_dev, pd.out_ids, pd.out_dist, pd.out_counts);
+        harvest_scan_events(ix);
+        ix->stats.last_path = pd.path;
     }
-    if (!out_on_dev) {
-        memcpy(pd.out_ids, ix->cur->h_ids.p, nk * sizeof(orx_id));
-        memcpy(pd.out_dist, ix->cur->h_dist.p, nk * sizeof(double));
-        memcpy(pd.out_counts, ix->cur->h_counts.p, nq * sizeof(int));
-    }
-    harvest_scan_events(ix);
     ix->stats.last_search_ms =
         std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - pd.t_begin).count();
-    ix->stats.last_path = pd.path;
     ix->stats.searches += 1;
     ix->stats.queries += nq;
     return ORX_OK;
 }
 
-int search_sharded_locked(orx_index *ix, Exchange *x, const float *queries, int nq, int k, orx_id *out_ids,
-                          double *out_dist, int *out_counts) {
+// one search on a fresh slot, submitted and waited for; x: the row-sharded search over that exchange
+int search_locked(orx_index *ix, Exchange *x, const float *queries, int nq, int k, orx_id *out_ids, double *out_dist,
+                  int *out_counts) {
     int rc = claim_slot(ix, nullptr);
     if (rc != ORX_OK) return rc;
-    rc = sharded_submit_locked(ix, x, queries, nq, k, out_ids, out_dist, out_counts);
+    rc = x ? sharded_submit_locked(ix, x, queries, nq, k, out_ids, out_dist, out_counts)
+           : search_submit_locked(ix, queries, nq, k, out_ids, out_dist, out_counts);
     if (rc != ORX_OK) return rc;
     ix->tickets += 1;
-    return sharded_wait_locked(ix, x);
+    return search_wait_locked(ix);
 }
 
 // A write (upsert / delete / import) is ordered AFTER every search submitted before it: the searches in flight are
@@ -1415,7 +1404,7 @@ void settle_in_flight(orx_index *ix) {
         if (!pd.active || pd.settled) continue;
         ix->cur = sl;
         const std::string keep = g_err;
-        const int rc = pd.sharded ? (ix->xchg ? sharded_wait_locked(ix, ix->xchg) : ORX_ERR_INVALID) : search_wait_locked(ix);
+        const int rc = search_wait_locked(ix);
         pd.settled = true;
         pd.settled_rc = rc;
         pd.settled_err = g_err;
@@ -1486,7 +1475,6 @@ int orx_create(orx_index **out, int dim, int dtype, uint64_t capacity_rows, int 
     orx_index *ix = new orx_index();
     ix->device = device;
     ix->dtype = dtype;
-    ix->scan_grid_sms = prop.multiProcessorCount;
     uint64_t cap = std::max<uint64_t>(capacity_rows, 1024);
     if (cap >= 0xFFFFFFFFull) {
         delete ix;
@@ -1616,7 +1604,7 @@ int orx_get_stats(const orx_index *ix, orx_stats *out) {
 
 int orx_contains(const orx_index *ix, orx_id id) {
     if (!ix) return 0;
-    if (ix->group) return orx_contains(ix->group->shards[shard_of_id(id, (uint32_t)ix->group->shards.size())], id);
+    if (ix->group) return orx_contains(ix->group->shards[orx::shard_of_id(id, (uint32_t)ix->group->shards.size())], id);
     std::lock_guard<std::mutex> lk(ix->mu);
     return ix->map.find(id) != nullptr ? 1 : 0;
 }
@@ -1698,26 +1686,20 @@ int orx_delete(orx_index *ix, const orx_id *ids, uint64_t n, uint64_t *n_removed
 
 int orx_search(orx_index *ix, const float *queries, int nq, int dim, int k, orx_id *out_ids, double *out_dist,
                int *out_counts) {
-    if (!ix) return fail(ORX_ERR_INVALID, "index is null");
-    if (dim != ORX_DIM) return fail(ORX_ERR_DIM, "different vector dimensions %d and %d", ORX_DIM, dim);
-    if (k < 1 || k > ORX_MAX_K) return fail(ORX_ERR_INVALID, "k must be in [1, %d], got %d", ORX_MAX_K, k);
-    if (nq < 0) return fail(ORX_ERR_INVALID, "nq must be >= 0");
-    if (nq == 0) return ORX_OK;
-    if (!queries || !out_ids || !out_dist || !out_counts) return fail(ORX_ERR_INVALID, "null argument");
+    int rc = check_query_args(ix, queries, nq, dim, k, out_ids, out_dist, out_counts);
+    if (rc != ORX_OK || nq == 0) return rc;
     if (ix->group) return group_search(ix->group, queries, nq, k, out_ids, out_dist, out_counts);
     std::lock_guard<std::mutex> lk(ix->mu);
     DeviceGuard g(ix->device);
-    return search_locked(ix, queries, nq, k, out_ids, out_dist, out_counts);
+    return search_locked(ix, nullptr, queries, nq, k, out_ids, out_dist, out_counts);
 }
 
 namespace {
 int check_search_args(orx_index *ix, const float *queries, int nq, int dim, int k, orx_id *out_ids, double *out_dist,
                       int *out_counts) {
-    if (!ix) return fail(ORX_ERR_INVALID, "index is null");
-    if (dim != ORX_DIM) return fail(ORX_ERR_DIM, "different vector dimensions %d and %d", ORX_DIM, dim);
-    if (k < 1 || k > ORX_MAX_K) return fail(ORX_ERR_INVALID, "k must be in [1, %d], got %d", ORX_MAX_K, k);
     if (nq < 1) return fail(ORX_ERR_INVALID, "nq must be >= 1");
-    if (!queries || !out_ids || !out_dist || !out_counts) return fail(ORX_ERR_INVALID, "null argument");
+    int rc = check_query_args(ix, queries, nq, dim, k, out_ids, out_dist, out_counts);
+    if (rc != ORX_OK) return rc;
     if (ix->group) return fail(ORX_ERR_INVALID, "asynchronous searches are per GPU: a multi-GPU index answers orx_search");
     return ORX_OK;
 }
@@ -1748,10 +1730,6 @@ int orx_search_wait(orx_index *ix, int ticket) {
     if (!sl->pend.active || (sl->pend.ticket & 0x7FFFFFFFu) != (uint32_t)ticket)
         return fail(ORX_ERR_INVALID, "ticket %d is not in flight", ticket);
     ix->cur = sl;
-    if (sl->pend.sharded) {
-        if (!ix->xchg || !ix->xchg->connected) return fail(ORX_ERR_INVALID, "shard exchange not connected");
-        return sharded_wait_locked(ix, ix->xchg);
-    }
     return search_wait_locked(ix);
 }
 
@@ -1763,8 +1741,8 @@ int orx_search_sharded_submit(orx_index *ix, const float *queries, int nq, int d
     std::lock_guard<std::mutex> lk(ix->mu);
     DeviceGuard g(ix->device);
     if (!ix->xchg || !ix->xchg->connected) return fail(ORX_ERR_INVALID, "shard exchange not connected (orx_shard_export / orx_shard_connect)");
-    if ((size_t)ix->xchg->world * k > 1024) return fail(ORX_ERR_INVALID, "sharded search: world * k must be <= 1024");
-    const int qchunk = k <= 32 ? XQ_MAX : XQ_MAX * 32 / k;
+    const int qchunk = exchange_queries(ix->xchg->world, k);
+    if (!qchunk) return fail(ORX_ERR_INVALID, "sharded search: world * k must be <= 1024");
     if (nq > qchunk) return fail(ORX_ERR_INVALID, "an asynchronous sharded search takes at most %d queries at k = %d", qchunk, k);
     rc = claim_slot(ix, ticket);
     if (rc != ORX_OK) return rc;
@@ -1777,7 +1755,7 @@ int orx_search_sharded_submit(orx_index *ix, const float *queries, int nq, int d
 
 int orx_search_filtered(orx_index *ix, const float *queries, int nq, int dim, int k, const orx_id *allow_ids,
                         uint64_t n_allow, orx_id *out_ids, double *out_dist, int *out_counts) {
-    int rc = check_filtered_args(ix, queries, nq, dim, k, out_ids, out_dist, out_counts);
+    int rc = check_query_args(ix, queries, nq, dim, k, out_ids, out_dist, out_counts);
     if (rc != ORX_OK || nq == 0) return rc;
     if (n_allow && !allow_ids) return fail(ORX_ERR_INVALID, "null argument");
     if (is_device_ptr(allow_ids)) return fail(ORX_ERR_INVALID, "allow_ids must be a host pointer");
@@ -1785,12 +1763,9 @@ int orx_search_filtered(orx_index *ix, const float *queries, int nq, int dim, in
     std::lock_guard<std::mutex> lk(ix->mu);
     DeviceGuard g(ix->device);
     if (any_in_flight(ix)) return fail(ORX_ERR_INVALID, "wait for the searches in flight (orx_search_wait) first");
-    std::vector<uint32_t> rows;
-    resolve_allow_ids(ix, allow_ids, n_allow, rows);
-    rc = upload_filter(ix, rows, ix->fb_list, ix->fb_count, ix->allow_bits);
+    FilterOnDevice f;
+    rc = resolve_filter(ix, allow_ids, n_allow, ix->fb_list, ix->fb_count, ix->allow_bits, &f);
     if (rc != ORX_OK) return rc;
-    const uint32_t m = (uint32_t)rows.size();
-    const FilterOnDevice f{m, ix->fb_list.p, ix->fb_count.p, m >= FILTER_SCAN_MIN_ROWS ? ix->allow_bits.p : nullptr};
     return filtered_search_locked(ix, f, queries, nq, k, out_ids, out_dist, out_counts);
 }
 
@@ -1821,7 +1796,7 @@ void orx_filter_destroy(orx_filter *f) {
 
 int orx_search_with_filter(orx_index *ix, orx_filter *f, const float *queries, int nq, int dim, int k,
                            orx_id *out_ids, double *out_dist, int *out_counts) {
-    int rc = check_filtered_args(ix, queries, nq, dim, k, out_ids, out_dist, out_counts);
+    int rc = check_query_args(ix, queries, nq, dim, k, out_ids, out_dist, out_counts);
     if (rc != ORX_OK || nq == 0) return rc;
     if (!f || f->ix != ix) return fail(ORX_ERR_INVALID, "filter does not belong to this index");
     std::lock_guard<std::mutex> lk(ix->mu);
@@ -1845,7 +1820,7 @@ int orx_search_mmr(orx_index *ix, const float *queries, int nq, int dim, int k, 
     if (any_in_flight(ix)) return fail(ORX_ERR_INVALID, "wait for the searches in flight (orx_search_wait) first");
     return mmr_local(ix, queries, nq, k, fetch_k, lambda_mult, out_ids, out_dist, out_counts,
                      [&](const float *q, int m, orx_id *ids, double *dist, int *cnt) {
-                         return search_locked(ix, q, m, fetch_k, ids, dist, cnt);
+                         return search_locked(ix, nullptr, q, m, fetch_k, ids, dist, cnt);
                      });
 }
 
@@ -1862,12 +1837,9 @@ int orx_search_mmr_filtered(orx_index *ix, const float *queries, int nq, int dim
     std::lock_guard<std::mutex> lk(ix->mu);
     DeviceGuard g(ix->device);
     if (any_in_flight(ix)) return fail(ORX_ERR_INVALID, "wait for the searches in flight (orx_search_wait) first");
-    std::vector<uint32_t> rows;
-    resolve_allow_ids(ix, allow_ids, n_allow, rows);
-    rc = upload_filter(ix, rows, ix->fb_list, ix->fb_count, ix->allow_bits);
+    FilterOnDevice f;
+    rc = resolve_filter(ix, allow_ids, n_allow, ix->fb_list, ix->fb_count, ix->allow_bits, &f);
     if (rc != ORX_OK) return rc;
-    const uint32_t m_allow = (uint32_t)rows.size();
-    const FilterOnDevice f{m_allow, ix->fb_list.p, ix->fb_count.p, m_allow >= FILTER_SCAN_MIN_ROWS ? ix->allow_bits.p : nullptr};
     return mmr_local(ix, queries, nq, k, fetch_k, lambda_mult, out_ids, out_dist, out_counts,
                      [&](const float *q, int m, orx_id *ids, double *dist, int *cnt) {
                          return filtered_search_locked(ix, f, q, m, fetch_k, ids, dist, cnt);
@@ -2031,15 +2003,9 @@ int orx_shard_export(orx_index *ix, int world, int rank, void *handle_out) {
     DeviceGuard g(ix->device);
     if (ix->xchg) return fail(ORX_ERR_INVALID, "shard exchange already initialised");
     Exchange *x = new Exchange();
-    x->world = world;
-    x->rank = rank;
-    x->n_targets = world;
-    x->slot_bytes = slot_layout(XQ_MAX, 32).bytes;          // nq * k <= XQ_MAX * 32 per exchange round
-    x->set_bytes = x->slot_bytes * world;
-    x->flags_off = 2 * x->set_bytes;
-    x->total_bytes = x->flags_off + 2 * (size_t)world * XFLAG_STRIDE;
-    cudaError_t e = cudaMalloc(&x->base, x->total_bytes);
-    if (e == cudaSuccess) e = cudaMemset(x->base, 0, x->total_bytes);
+    const size_t bytes = exchange_layout(x, world, rank);
+    cudaError_t e = cudaMalloc(&x->base, bytes);
+    if (e == cudaSuccess) e = cudaMemset(x->base, 0, bytes);
     cudaIpcMemHandle_t h;
     if (e == cudaSuccess) e = cudaIpcGetMemHandle(&h, x->base);
     if (e != cudaSuccess) {
@@ -2080,43 +2046,25 @@ int orx_shard_connect(orx_index *ix, const void *handles, int n_handles) {
         }
         x->peer_base[r] = static_cast<char *>(p);
     }
-    for (int s = 0; s < 2; ++s) {
-        std::vector<void *> slots(x->world);
-        std::vector<uint32_t *> flags(x->world);
-        for (int r = 0; r < x->world; ++r) {
-            slots[r] = x->peer_base[r] + (size_t)s * x->set_bytes + (size_t)x->rank * x->slot_bytes;
-            flags[r] = reinterpret_cast<uint32_t *>(x->peer_base[r] + x->flags_off +
-                                                    ((size_t)s * x->world + x->rank) * XFLAG_STRIDE);
-        }
-        CK(cudaMalloc(&x->d_peer_slot[s], x->world * sizeof(void *)));
-        CK(cudaMalloc(&x->d_peer_flag[s], x->world * sizeof(uint32_t *)));
-        CK(cudaMemcpy(x->d_peer_slot[s], slots.data(), x->world * sizeof(void *), cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(x->d_peer_flag[s], flags.data(), x->world * sizeof(uint32_t *), cudaMemcpyHostToDevice));
-    }
+    CK(upload_peer_tables(x, x->peer_base));
     x->connected = true;
     return ORX_OK;
 }
 
 int orx_search_sharded(orx_index *ix, const float *queries, int nq, int dim, int k, orx_id *out_ids,
                        double *out_dist, int *out_counts) {
-    if (!ix) return fail(ORX_ERR_INVALID, "index is null");
-    if (dim != ORX_DIM) return fail(ORX_ERR_DIM, "different vector dimensions %d and %d", ORX_DIM, dim);
-    if (k < 1 || k > ORX_MAX_K) return fail(ORX_ERR_INVALID, "k must be in [1, %d], got %d", ORX_MAX_K, k);
-    if (nq < 0) return fail(ORX_ERR_INVALID, "nq must be >= 0");
-    if (nq == 0) return ORX_OK;
-    if (!queries || !out_ids || !out_dist || !out_counts) return fail(ORX_ERR_INVALID, "null argument");
+    int rc = check_query_args(ix, queries, nq, dim, k, out_ids, out_dist, out_counts);
+    if (rc != ORX_OK || nq == 0) return rc;
     if (ix->group) return fail(ORX_ERR_INVALID, "a multi-GPU index is not a rank of a process group: use orx_search");
     std::lock_guard<std::mutex> lk(ix->mu);
     DeviceGuard g(ix->device);
     if (!ix->xchg || !ix->xchg->connected) return fail(ORX_ERR_INVALID, "shard exchange not connected (orx_shard_export / orx_shard_connect)");
-    const bool q_dev = is_device_ptr(queries), o_dev = is_device_ptr(out_ids);
-    if ((size_t)ix->xchg->world * k > 1024) return fail(ORX_ERR_INVALID, "sharded search: world * k must be <= 1024");
-    const int qchunk = k <= 32 ? XQ_MAX : XQ_MAX * 32 / k;       // a slot holds XQ_MAX queries at k <= 32
+    const int qchunk = exchange_queries(ix->xchg->world, k);
+    if (!qchunk) return fail(ORX_ERR_INVALID, "sharded search: world * k must be <= 1024");
     for (int q0 = 0; q0 < nq; q0 += qchunk) {       // every rank chunks identically
         const int m = std::min(qchunk, nq - q0);
-        (void)q_dev; (void)o_dev;
-        int rc = search_sharded_locked(ix, ix->xchg, queries + (size_t)q0 * ORX_DIM, m, k, out_ids + (size_t)q0 * k,
-                                       out_dist + (size_t)q0 * k, out_counts + q0);
+        rc = search_locked(ix, ix->xchg, queries + (size_t)q0 * ORX_DIM, m, k, out_ids + (size_t)q0 * k,
+                           out_dist + (size_t)q0 * k, out_counts + q0);
         if (rc != ORX_OK) return rc;
     }
     return ORX_OK;

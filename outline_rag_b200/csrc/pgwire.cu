@@ -78,15 +78,6 @@ inline uint32_t be32(const uint8_t *p) { return ((uint32_t)p[0] << 24) | ((uint3
 inline uint16_t be16(const uint8_t *p) { return (uint16_t)(((uint16_t)p[0] << 8) | p[1]); }
 inline uint64_t be64(const uint8_t *p) { return ((uint64_t)be32(p) << 32) | be32(p + 4); }
 
-// the row-shard function of outline_rag_b200/sharded.py:shard_of (SURVEY.md 8e): mix64(hi * GOLD ^ lo) mod G
-inline uint32_t shard_of_id(uint64_t hi, uint64_t lo, uint32_t world) {
-    uint64_t z = hi * 0x9E3779B97F4A7C15ull ^ lo;
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    z ^= z >> 31;
-    return (uint32_t)(z % world);
-}
-
 }  // namespace
 
 struct orx_pgcopy {
@@ -324,7 +315,7 @@ int pg_parse(orx_pgcopy *ld) {
                 }
                 if (have < PG_TUPLE_MAX) return ORX_OK;
                 const orx_id id{be64(p + 6), be64(p + 14)};
-                if (ld->world > 1 && shard_of_id(id.hi, id.lo, ld->world) != ld->rank) {
+                if (ld->world > 1 && orx::shard_of_id(id, ld->world) != ld->rank) {
                     ld->foreign += 1;                                     // another rank's row: not staged
                     ld->pos += PG_TUPLE_MAX;
                     break;

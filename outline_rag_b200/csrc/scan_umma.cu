@@ -1053,7 +1053,6 @@ void umma_plan_destroy(UmmaPlan *p) {
     cudaFree(p->gthr);
     delete p;
 }
-void umma_plan_invalidate(UmmaPlan *) {}      // tensor maps are encoded per search (pointer + live row count)
 const char *umma_last_error() { return g_umma_err.c_str(); }
 
 bool umma_should_use(const UmmaPlan *p, int nq, int k, uint32_t n_rows) {

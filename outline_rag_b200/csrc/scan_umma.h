@@ -11,7 +11,6 @@ struct UmmaPlan;
 
 UmmaPlan *umma_plan_create(int device);
 void umma_plan_destroy(UmmaPlan *p);
-void umma_plan_invalidate(UmmaPlan *p);          // table was reallocated: tensor maps are stale
 constexpr int UMMA_MAX_K = 64;                   // largest k the coarse pass can prove (candidate lists of 160 keys)
 bool umma_should_use(const UmmaPlan *p, int nq, int k, uint32_t n_rows);
 const char *umma_last_error();

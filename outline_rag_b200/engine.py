@@ -87,6 +87,19 @@ def _host_f32(x, what: str) -> np.ndarray:
     return np.ascontiguousarray(a, dtype=np.float32)
 
 
+def _host_result(nq: int, k: int):
+    """Host result triple ``(ids uint64 [nq,k,2], dist float64 [nq,k], counts int32 [nq])``: zero ids, NaN distances."""
+    k = max(k, 0)
+    return np.zeros((nq, k, 2), np.uint64), np.full((nq, k), np.nan, np.float64), np.zeros(nq, np.int32)
+
+
+def _device_result(nq: int, k: int, device):
+    """Uninitialised CUDA result triple ``(ids int64 [nq,k,2], dist float64 [nq,k], counts int32 [nq])``."""
+    return (torch.empty((nq, k, 2), dtype=torch.int64, device=device),
+            torch.empty((nq, k), dtype=torch.float64, device=device),
+            torch.empty((nq,), dtype=torch.int32, device=device))
+
+
 def parse_vector_text(text, dim: int = ORX_DIM) -> np.ndarray:
     """pgvector's text input (``'[0.1, 0.2, ...]'`` -> fp32 ``[dim]``) with its checks: the format the
     reference sends the query vector and the stored embeddings in.  One rounding, decimal -> fp32
@@ -109,6 +122,12 @@ class Filter:
         self._index = index
         ida = ids_to_array(allow_ids)
         check(lib.orx_filter_create(index._h, C.c_void_p(ida.ctypes.data), ida.shape[0], C.byref(self._f)))
+
+    def handle_for(self, index: "Index"):
+        """The C handle, once it is checked to be open and to belong to `index`."""
+        if self._index is not index or not self._f:
+            raise _lib.OrxValueError(_lib.ORX_ERR_INVALID, "filter is closed or belongs to another index")
+        return self._f
 
     def close(self) -> None:
         if getattr(self, "_f", None) is not None and self._f:
@@ -328,20 +347,13 @@ class Index:
             nq, dim = q.shape
             if len(self.devices) > 1:
                 _fence_producer(q)
-            if out is not None:
-                ids, dist, cnt = out
-            else:
-                ids = torch.empty((nq, k, 2), dtype=torch.int64, device=q.device)
-                dist = torch.empty((nq, k), dtype=torch.float64, device=q.device)
-                cnt = torch.empty((nq,), dtype=torch.int32, device=q.device)
+            ids, dist, cnt = out if out is not None else _device_result(nq, k, q.device)
             check(lib.orx_search(self._h, C.c_void_p(q.data_ptr()), nq, dim, int(k), C.c_void_p(ids.data_ptr()),
                                  C.c_void_p(dist.data_ptr()), C.c_void_p(cnt.data_ptr())))
             return ids, dist, cnt
         q = _host_f32(queries, "queries")
         nq, dim = q.shape
-        ids = np.zeros((nq, max(k, 0), 2), np.uint64)
-        dist = np.full((nq, max(k, 0)), np.nan, np.float64)
-        cnt = np.zeros(nq, np.int32)
+        ids, dist, cnt = _host_result(nq, k)
         check(lib.orx_search(self._h, C.c_void_p(q.ctypes.data), nq, dim, int(k), C.c_void_p(ids.ctypes.data),
                              C.c_void_p(dist.ctypes.data), C.c_void_p(cnt.ctypes.data)))
         return ids, dist, cnt
@@ -390,13 +402,9 @@ class Index:
         `allow_ids`: ids (resolved on every call) or a `Filter` (resolved once, kept on the device)."""
         q = _host_f32(queries, "queries")
         nq, dim = q.shape
-        ids = np.zeros((nq, max(k, 0), 2), np.uint64)
-        dist = np.full((nq, max(k, 0)), np.nan, np.float64)
-        cnt = np.zeros(nq, np.int32)
+        ids, dist, cnt = _host_result(nq, k)
         if isinstance(allow_ids, Filter):
-            if allow_ids._index is not self or not allow_ids._f:
-                raise _lib.OrxValueError(_lib.ORX_ERR_INVALID, "filter is closed or belongs to another index")
-            check(lib.orx_search_with_filter(self._h, allow_ids._f, C.c_void_p(q.ctypes.data), nq, dim, int(k),
+            check(lib.orx_search_with_filter(self._h, allow_ids.handle_for(self), C.c_void_p(q.ctypes.data), nq, dim, int(k),
                                              C.c_void_p(ids.ctypes.data), C.c_void_p(dist.ctypes.data),
                                              C.c_void_p(cnt.ctypes.data)))
             return ids, dist, cnt
@@ -414,17 +422,13 @@ class Index:
         row with its query distance.  Not served by the micro-batcher or the row-sharded `ShardedIndex`."""
         q = _host_f32(queries, "queries")
         nq, dim = q.shape
-        ids = np.zeros((nq, max(k, 0), 2), np.uint64)
-        dist = np.full((nq, max(k, 0)), np.nan, np.float64)
-        cnt = np.zeros(nq, np.int32)
+        ids, dist, cnt = _host_result(nq, k)
         outs = (C.c_void_p(ids.ctypes.data), C.c_void_p(dist.ctypes.data), C.c_void_p(cnt.ctypes.data))
         head = (C.c_void_p(q.ctypes.data), nq, dim, int(k), int(fetch_k), float(lambda_mult))
         if allow_ids is None:
             check(lib.orx_search_mmr(self._h, *head, *outs))
         elif isinstance(allow_ids, Filter):
-            if allow_ids._index is not self or not allow_ids._f:
-                raise _lib.OrxValueError(_lib.ORX_ERR_INVALID, "filter is closed or belongs to another index")
-            check(lib.orx_search_mmr_with_filter(self._h, allow_ids._f, *head, *outs))
+            check(lib.orx_search_mmr_with_filter(self._h, allow_ids.handle_for(self), *head, *outs))
         else:
             allow = ids_to_array(allow_ids)
             check(lib.orx_search_mmr_filtered(self._h, *head, C.c_void_p(allow.ctypes.data), allow.shape[0], *outs))
@@ -563,18 +567,14 @@ class Index:
             q = queries if queries.dim() == 2 else queries.unsqueeze(0)
             nq, dim = q.shape
             if out is None:
-                out = (torch.empty((nq, k, 2), dtype=torch.int64, device=q.device),
-                       torch.empty((nq, k), dtype=torch.float64, device=q.device),
-                       torch.empty((nq,), dtype=torch.int32, device=q.device))
+                out = _device_result(nq, k, q.device)
             check(lib.orx_search_sharded(self._h, C.c_void_p(q.data_ptr()), nq, dim, int(k),
                                          C.c_void_p(out[0].data_ptr()), C.c_void_p(out[1].data_ptr()),
                                          C.c_void_p(out[2].data_ptr())))
             return out
         q = _host_f32(queries, "queries")
         nq, dim = q.shape
-        ids = np.zeros((nq, max(k, 0), 2), np.uint64)
-        dist = np.full((nq, max(k, 0)), np.nan, np.float64)
-        cnt = np.zeros(nq, np.int32)
+        ids, dist, cnt = _host_result(nq, k)
         check(lib.orx_search_sharded(self._h, C.c_void_p(q.ctypes.data), nq, dim, int(k), C.c_void_p(ids.ctypes.data),
                                      C.c_void_p(dist.ctypes.data), C.c_void_p(cnt.ctypes.data)))
         return ids, dist, cnt
@@ -583,9 +583,7 @@ class Index:
         """Merge ``[n_lists, nq, k]`` shard results (NumPy or CUDA tensors) into the global top-k."""
         if _is_cuda_tensor(ids):
             n_lists, nq = ids.shape[0], ids.shape[1]
-            oi = torch.empty((nq, k, 2), dtype=torch.int64, device=ids.device)
-            od = torch.empty((nq, k), dtype=torch.float64, device=ids.device)
-            oc = torch.empty((nq,), dtype=torch.int32, device=ids.device)
+            oi, od, oc = _device_result(nq, k, ids.device)
             check(lib.orx_merge_topk(self._h, n_lists, nq, int(k), C.c_void_p(ids.contiguous().data_ptr()),
                                      C.c_void_p(dist.contiguous().data_ptr()),
                                      C.c_void_p(counts.contiguous().data_ptr()), C.c_void_p(oi.data_ptr()),
@@ -595,9 +593,7 @@ class Index:
         dist = np.ascontiguousarray(dist, np.float64)
         counts = np.ascontiguousarray(counts, np.int32)
         n_lists, nq = ids.shape[0], ids.shape[1]
-        oi = np.zeros((nq, k, 2), np.uint64)
-        od = np.full((nq, k), np.nan, np.float64)
-        oc = np.zeros(nq, np.int32)
+        oi, od, oc = _host_result(nq, k)
         check(lib.orx_merge_topk(self._h, n_lists, nq, int(k), C.c_void_p(ids.ctypes.data),
                                  C.c_void_p(dist.ctypes.data), C.c_void_p(counts.ctypes.data),
                                  C.c_void_p(oi.ctypes.data), C.c_void_p(od.ctypes.data),

@@ -21,7 +21,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from .engine import Index, ids_to_array
+from .engine import Index, _device_result, ids_to_array
 
 _GOLD = np.uint64(0x9E3779B97F4A7C15)
 _M1 = np.uint64(0xBF58476D1CE4E5B9)
@@ -170,9 +170,7 @@ class ShardedIndex:
                 key = (q.shape[0], k)
                 out = self._outs.get(key)
                 if out is None:
-                    out = self._outs[key] = (torch.empty((q.shape[0], k, 2), dtype=torch.int64, device=q.device),
-                                             torch.empty((q.shape[0], k), dtype=torch.float64, device=q.device),
-                                             torch.empty((q.shape[0],), dtype=torch.int32, device=q.device))
+                    out = self._outs[key] = _device_result(q.shape[0], k, q.device)
                 return self.local.search_sharded(q, k, out)
             return self.local.search_sharded(queries, k)
         if self.world > 1 and isinstance(queries, torch.Tensor) and queries.is_cuda and hasattr(self.local, "search_into"):
@@ -190,9 +188,7 @@ class ShardedIndex:
             key = (q.shape[0], k)
             out = self._outs.get(key)
             if out is None:
-                out = self._outs[key] = (torch.empty((q.shape[0], k, 2), dtype=torch.int64, device=q.device),
-                                         torch.empty((q.shape[0], k), dtype=torch.float64, device=q.device),
-                                         torch.empty((q.shape[0],), dtype=torch.int32, device=q.device))
+                out = self._outs[key] = _device_result(q.shape[0], k, q.device)
             return self.local.search(q, k, out=out)
         ids, dist_, cnt = self.local.search(queries, k)
         if self.world == 1:
@@ -211,9 +207,7 @@ class ShardedIndex:
         self._submits += 1
         out = self._outs.get(key)
         if out is None:
-            out = self._outs[key] = (torch.empty((q.shape[0], k, 2), dtype=torch.int64, device=q.device),
-                                     torch.empty((q.shape[0], k), dtype=torch.float64, device=q.device),
-                                     torch.empty((q.shape[0],), dtype=torch.int32, device=q.device))
+            out = self._outs[key] = _device_result(q.shape[0], k, q.device)
         if self.world > 1 and self.exchange != "p2p":
             raise RuntimeError("search_submit needs the peer-memory exchange (or a single rank)")
         return self.local.search_submit(q, k, out, sharded=self.world > 1), out
