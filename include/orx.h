@@ -30,9 +30,12 @@ extern "C" {
 #define ORX_MAX_K 128           /* TOP_K is 12 (reference app/config.py:253); up to 128 for a wider
                                    reranker feed (SURVEY.md 8f-4).  Batches with k <= 64 run the tcgen05 scan
                                    (64-key candidate lists up to k = 16, 160-key lists beyond); k > 64 runs
-                                   one fp32 scan per query. */
+                                   one GEMV scan per query (over the bf16 image of a large fp32 table, see
+                                   ORX_OPT_IMAGE_MIN_ROWS). */
 
-#define ORX_DTYPE_F32 0         /* rows stored verbatim (fp32) + per-row 1/norm   */
+#define ORX_DTYPE_F32 0         /* rows stored verbatim (fp32) + per-row 1/norm;
+                                   + a bf16 image of the rows when the device has room
+                                   (see ORX_OPT_IMAGE_MIN_ROWS)                    */
 #define ORX_DTYPE_BF16 1        /* rows stored as RNE-bf16 of the normalised row  */
 
 #define ORX_OK 0
@@ -59,7 +62,8 @@ typedef struct orx_stats {
     uint64_t rows_moved;          /* rows relocated by delete compaction           */
     float    last_scan_ms;        /* device time of the last search's scan kernel(s) */
     float    last_search_ms;      /* host wall time of the last orx_search call     */
-    int      last_path;           /* 0 none, 1 gemv scan, 2 tcgen05 scan           */
+    int      last_path;           /* 0 none, 1 gemv scan, 2 tcgen05 scan,
+                                     3 gemv scan over the bf16 image of an fp32 table */
     int      reserved;
     uint64_t scan_launches;       /* scan kernel launches (gemv or tcgen05)        */
     double   scan_ms_total;       /* sum of their device times (CUDA events around each launch) */
@@ -90,8 +94,21 @@ int orx_shard_count(const orx_index *idx);      /* 1 for orx_create, n_devices f
 int orx_set_stream(orx_index *idx, void *cuda_stream);
 
 /* Options.  ORX_OPT_SCAN_TIMING (default 1): record a CUDA event pair around every scan launch so that orx_get_stats
- * can report the scan kernel's own device time (bench.py's roofline); 0 saves the two event records per search. */
+ * can report the scan kernel's own device time (bench.py's roofline); 0 saves the two event records per search.
+ * ORX_OPT_IMAGE_MIN_ROWS (default 1048576 = 2^20): live rows from which an fp32 table's GEMV scans (one query, batches
+ * with k > 64, filtered bitmap scans) read the table's bf16 IMAGE instead of its fp32 rows.  The image holds RNE-bf16 of
+ * every stored element (not normalised: 2 bytes per element, +50 % device memory, e.g. +20.5 GB at 10M rows) and is kept
+ * in step by upsert, delete, import and growth.  It is allocated only for a capacity of at least this many rows -- when
+ * the table is created or grows, or by the first search that would read it (after the option was lowered) -- so small
+ * tables pay nothing for it; an fp32 table for which the device has no room simply has none (scans read the fp32 rows).
+ * The image takes device memory other allocations (search scratch, the caller's tensors) might want; only growth of
+ * the table itself takes it back.  The re-scan of queries the tcgen05 batch pass could not prove always reads the fp32
+ * rows.  The image scan halves
+ * the bytes a query streams; its candidates are still rescored canonically from the fp32 rows and the completeness proof
+ * uses the image's error bound, so the answers are the same ids and distance bits (last_path reports 3).  0 = always
+ * (when an image exists), a negative value = never.  bf16 tables have no image.  A multi-GPU handle sets every shard. */
 #define ORX_OPT_SCAN_TIMING 1
+#define ORX_OPT_IMAGE_MIN_ROWS 2
 int orx_set_option(orx_index *idx, int option, int value);
 
 uint64_t orx_size(const orx_index *idx);       /* live rows */
@@ -242,6 +259,12 @@ int orx_debug_coarse_scores(orx_index *idx, const float *queries, int nq, int us
  * sequence).  Irregular rows (norm outside [2^-40, 2^40]) come out +-inf or NaN, zero-norm rows NaN.  out_device
  * [live rows, nq] fp32 in table row order.  1 <= nq <= 65535. */
 int orx_debug_fast_scores(orx_index *idx, const float *queries, int nq, float *out_device);
+
+/* The same diagnostic for the scans over the bf16 image of an fp32 table (ORX_OPT_IMAGE_MIN_ROWS): the fp32 FMA-chain dot
+ * of every live row's IMAGE with every normalised query, times the fp32 row's 1/|x| -- the value the image scans key
+ * their candidates on.  ORX_ERR_INVALID when the index has no image (bf16 table, or no device memory for it).
+ * out_device [live rows, nq] fp32 in table row order.  1 <= nq <= 65535. */
+int orx_debug_image_scores(orx_index *idx, const float *queries, int nq, float *out_device);
 
 /* Read back stored rows (as fp32) by id -- snapshot / debugging / tests.
  * out_vecs [n, dim] host; out_found [n] host (1/0). */

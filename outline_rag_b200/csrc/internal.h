@@ -9,6 +9,12 @@ namespace orx {
 // Rigorous bounds on |fast score - canonical cosine| per scan path (DESIGN.md, "Exactness").
 constexpr double EPS_GEMV_F32 = 3.0e-6;   // fp32 FMA chain of depth 32 + 5 shuffle adds
 constexpr double EPS_GEMV_BF16 = 3.0e-6;  // same arithmetic on exactly-converted bf16 rows
+// the same scans over the bf16 image of an fp32 table (RNE of every element, not normalised, scored with the fp32 row's
+// 1/|x|): |img_i - x_i| <= 2^-8 |x_i| (+ 2^-134 for subnormals) -> |q^.(img - x)| * scale <= 2^-8 (1 + 2^-20), plus the
+// fp32 arithmetic of the bf16 dot (EPS_GEMV_BF16); 3.9093e-3 rounded up (DESIGN.md section 2)
+constexpr double EPS_GEMV_IMAGE = 3.92e-3;
+// live rows from which an fp32 table's single-query / k > 64 batch / bitmap scans read the image (ORX_OPT_IMAGE_MIN_ROWS)
+constexpr uint64_t IMAGE_MIN_ROWS = 1ull << 20;
 // kind::tf32 truncates both operands to 10 mantissa bits (measured on sm_100a, tests/test_epsilon_adversarial_gpu.py):
 // worst case (1+2^-10)^2-1 = 1.96e-3; a worst-case query against its own row measures 1.927e-3 (DESIGN.md section 2)
 constexpr double EPS_UMMA_TF32 = 2.5e-3;
@@ -18,6 +24,10 @@ constexpr double EPS_UMMA_BF16 = 2.5e-3;
 // candidate list = 32 * slots keys per query: k <= 16 -> 32 candidates, k <= 32 -> 64
 // candidate list = 32 * slots keys per query: k <= 16 -> 32, k <= 32 -> 64, k <= 128 -> 32 more than k at least
 inline int slots_for_k(int k) { return k <= 16 ? 1 : k <= 32 ? 2 : k <= 96 ? 4 : 5; }
+// the scans over an fp32 table's bf16 image: one width up.  Their eps is ~1300x the fp32 scan's, so more rows have fast
+// scores within eps of the k-th (measured at 10M rows, k = 12: 21-49 rows within 2 eps); finalize's proof needs the
+// list's K-th fast score to lie eps below the k-th cosine, and a list of 32 keys left ~6 % of queries unproven
+inline int image_slots_for_k(int k) { return k <= 16 ? 2 : k <= 32 ? 4 : 5; }
 constexpr int SCAN_THREADS = 256;
 constexpr int SCAN_WARPS = SCAN_THREADS / 32;
 
@@ -114,13 +124,15 @@ void launch_scan_gemv_filtered(int dtype, const void *table, const float *scale,
 
 // ---- table_ops.cu
 void launch_validate_rows(const float *src, uint64_t n, int *flag, cudaStream_t st);
+// image: the bf16 image of an fp32 table ([cap, ORX_DIM] __nv_bfloat16), kept in step with the rows; nullptr = none
 void launch_commit_rows(int dtype, const float *src, const uint32_t *src_idx, const uint32_t *dst_row,
                         const orx_id *ids, uint32_t n, void *table, float *scale, double *n2,
-                        orx_id *row_ids, const int *abort_flag, cudaStream_t st);
+                        orx_id *row_ids, const int *abort_flag, void *image, cudaStream_t st);
 void launch_adopt_rows(int dtype, const void *table, uint32_t row0, uint32_t n, const orx_id *ids, float *scale,
-                       double *n2, orx_id *row_ids, int *flag, cudaStream_t st);
+                       double *n2, orx_id *row_ids, int *flag, void *image, cudaStream_t st);
 void launch_move_rows(int dtype, const uint32_t *src_row, const uint32_t *dst_row, uint32_t n,
-                      void *table, float *scale, double *n2, orx_id *row_ids, cudaStream_t st);
+                      void *table, float *scale, double *n2, orx_id *row_ids, void *image, cudaStream_t st);
+void launch_image_rows(const float *table, uint64_t n, void *image, cudaStream_t st);     // image of rows [0, n)
 void launch_gather_rows(int dtype, const void *table, const uint32_t *rows, uint32_t n, float *out,
                         cudaStream_t st);
 

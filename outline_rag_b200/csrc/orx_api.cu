@@ -296,6 +296,13 @@ struct orx_index {
     float *scale = nullptr;
     double *n2 = nullptr;
     orx_id *row_ids = nullptr;
+    // fp32 tables: the bf16 image of the rows ([capacity, ORX_DIM], RNE of every element) that the GEMV scans read from
+    // image_min_rows live rows on -- half the bytes of the fp32 rows; finalize still rescores the fp32 rows.  Allocated
+    // only for a capacity of image_min_rows rows or more (at create / growth, or by the first search that needs it),
+    // and best effort: null when the device has no room (the scans then read the fp32 rows; bf16 tables never have one)
+    __nv_bfloat16 *image = nullptr;
+    uint64_t image_min_rows = orx::IMAGE_MIN_ROWS;    // ORX_OPT_IMAGE_MIN_ROWS
+    uint64_t image_failed_cap = 0;                    // capacity at which allocating the image failed (no retry until it changes)
 
     // host mirror of the id column + id -> row map
     std::vector<orx_id> host_row_ids;
@@ -371,11 +378,50 @@ struct DeviceGuard {
     }
 };
 
+// the bf16 image of an fp32 table with room for `cap` rows, or nullptr: a bf16 table, a capacity below the row count from
+// which the scans would read it (small tables pay no memory for it), or no room left on the device
+__nv_bfloat16 *alloc_image(orx_index *ix, uint64_t cap) {
+    if (ix->dtype != ORX_DTYPE_F32 || cap < ix->image_min_rows) return nullptr;
+    void *p = nullptr;
+    if (cudaMalloc(&p, cap * ORX_DIM * sizeof(__nv_bfloat16)) != cudaSuccess) {
+        cudaGetLastError();
+        ix->image_failed_cap = cap;
+        return nullptr;
+    }
+    return static_cast<__nv_bfloat16 *>(p);
+}
+bool use_image(const orx_index *ix) { return ix->image != nullptr && ix->n_live >= ix->image_min_rows; }
+
+// an fp32 table that has reached image_min_rows live rows (or whose option was lowered below its size) without an image:
+// allocate one and build it from the live rows, once per capacity.  Best effort: without it the scans read the fp32 rows.
+// force: the diagnostic hook, which wants the image whatever the threshold.
+void ensure_image(orx_index *ix, bool force = false) {
+    if (ix->image || ix->dtype != ORX_DTYPE_F32 || ix->n_live == 0 || ix->image_failed_cap == ix->capacity) return;
+    if (!force && ix->n_live < ix->image_min_rows) return;
+    const uint64_t keep = ix->image_min_rows;
+    ix->image_min_rows = 0;                       // the capacity test of alloc_image is this function's own decision
+    __nv_bfloat16 *im = alloc_image(ix, ix->capacity);
+    ix->image_min_rows = keep;
+    if (!im) {
+        ix->image_failed_cap = ix->capacity;
+        return;
+    }
+    orx::launch_image_rows(static_cast<const float *>(ix->table), ix->n_live, im, ix->stream);
+    ix->stats.kernel_launches += 1;
+    if (cudaGetLastError() != cudaSuccess) {      // nothing was launched: stay without an image
+        cudaFree(im);
+        ix->image_failed_cap = ix->capacity;
+        return;
+    }
+    ix->image = im;                               // stream order: every later scan sees the built rows
+}
+
 int alloc_table(orx_index *ix, uint64_t cap) {
     CK(cudaMalloc(&ix->table, cap * ORX_DIM * elem_size(ix->dtype)));
     CK(cudaMalloc(&ix->scale, cap * sizeof(float)));
     CK(cudaMalloc(&ix->n2, cap * sizeof(double)));
     CK(cudaMalloc(&ix->row_ids, cap * sizeof(orx_id)));
+    ix->image = alloc_image(ix, cap);             // after the table: the image never takes the table's room
     ix->capacity = cap;
     return ORX_OK;
 }
@@ -390,23 +436,47 @@ int grow_table(orx_index *ix, uint64_t need) {
     double *n = nullptr;
     orx_id *r = nullptr;
     const size_t rb = ORX_DIM * elem_size(ix->dtype);
-    cudaError_t e = cudaMalloc(&t, cap * rb);
-    if (e == cudaSuccess) e = cudaMalloc(&s, cap * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc(&n, cap * sizeof(double));
-    if (e == cudaSuccess) e = cudaMalloc(&r, cap * sizeof(orx_id));
-    if (e != cudaSuccess) {
+    cudaError_t e = cudaSuccess;
+    for (int attempt = 0; attempt < 2; ++attempt) {
+        e = cudaMalloc(&t, cap * rb);
+        if (e == cudaSuccess) e = cudaMalloc(&s, cap * sizeof(float));
+        if (e == cudaSuccess) e = cudaMalloc(&n, cap * sizeof(double));
+        if (e == cudaSuccess) e = cudaMalloc(&r, cap * sizeof(orx_id));
+        if (e == cudaSuccess) break;
         cudaGetLastError();
         if (t) cudaFree(t);
         if (s) cudaFree(s);
         if (n) cudaFree(n);
         if (r) cudaFree(r);
+        t = nullptr, s = nullptr, n = nullptr, r = nullptr;
+        if (!ix->image) break;
+        cudaFree(ix->image);                // the image is best effort: it gives its room to the table's growth
+        ix->image = nullptr;
+    }
+    if (e != cudaSuccess)
         return fail(ORX_ERR_CAPACITY, "cannot grow table to %llu rows: %s", (unsigned long long)cap,
                     cudaGetErrorString(e));
+    __nv_bfloat16 *im = nullptr;
+    if (ix->image) {                        // an image that exists is carried over whatever the threshold
+        const uint64_t keep = ix->image_min_rows;
+        ix->image_min_rows = 0;
+        im = alloc_image(ix, cap);
+        ix->image_min_rows = keep;
+    } else {
+        im = alloc_image(ix, cap);
     }
     e = cudaMemcpyAsync(t, ix->table, ix->n_live * rb, cudaMemcpyDeviceToDevice, ix->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(s, ix->scale, ix->n_live * sizeof(float), cudaMemcpyDeviceToDevice, ix->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(n, ix->n2, ix->n_live * sizeof(double), cudaMemcpyDeviceToDevice, ix->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(r, ix->row_ids, ix->n_live * sizeof(orx_id), cudaMemcpyDeviceToDevice, ix->stream);
+    if (e == cudaSuccess && im) {
+        if (ix->image)
+            e = cudaMemcpyAsync(im, ix->image, ix->n_live * ORX_DIM * sizeof(__nv_bfloat16), cudaMemcpyDeviceToDevice,
+                                ix->stream);
+        else
+            orx::launch_image_rows(static_cast<const float *>(ix->table), ix->n_live, im, ix->stream);
+        if (e == cudaSuccess) e = cudaGetLastError();
+    }
     if (e == cudaSuccess) e = cudaStreamSynchronize(ix->stream);
     if (e != cudaSuccess) {                 // the old table stays in place and valid
         cudaGetLastError();
@@ -414,16 +484,19 @@ int grow_table(orx_index *ix, uint64_t need) {
         cudaFree(s);
         cudaFree(n);
         cudaFree(r);
+        if (im) cudaFree(im);
         return fail(ORX_ERR_CUDA, "copying the table to its grown allocation failed: %s", cudaGetErrorString(e));
     }
     cudaFree(ix->table);
     cudaFree(ix->scale);
     cudaFree(ix->n2);
     cudaFree(ix->row_ids);
+    if (ix->image) cudaFree(ix->image);
     ix->table = t;
     ix->scale = s;
     ix->n2 = n;
     ix->row_ids = r;
+    ix->image = im;
     ix->capacity = cap;
     return ORX_OK;
 }
@@ -537,7 +610,7 @@ int upsert_locked(orx_index *ix, const orx_id *ids, const float *vecs, uint64_t 
         CK(cudaMemcpyAsync(ix->d_dst_row.p, ix->h_u32b.p, np * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(ix->d_ids.p, ids + s, m * sizeof(orx_id), cudaMemcpyHostToDevice, st));
         orx::launch_commit_rows(ix->dtype, src, ix->d_src_idx.p, ix->d_dst_row.p, ix->d_ids.p, np, ix->table,
-                                ix->scale, ix->n2, ix->row_ids, ix->d_flag.p, st);
+                                ix->scale, ix->n2, ix->row_ids, ix->d_flag.p, ix->image, st);
         ix->stats.kernel_launches += 1;
         CK(cudaMemcpyAsync(ix->h_flag.p, ix->d_flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));     // the ONE sync of a chunk: scratch + the caller's buffers are reusable after it
@@ -623,13 +696,20 @@ int exhaustive_query(orx_index *ix, const float *q_src, int qi, int k, double dk
     return ORX_OK;
 }
 
-// f: a filter with a bitmap -- the sequential scan skips the rows whose bit is clear (HBM traffic = eligible rows only)
+// f: a filter with a bitmap -- the sequential scan skips the rows whose bit is clear (HBM traffic = eligible rows only).
+// allow_image: a large fp32 table with an image is scanned over the image (the bf16 instantiation of the same kernels,
+// the fp32 row's 1/|x|, EPS_GEMV_IMAGE); finalize rescores the fp32 rows either way, so the answer is the same.  The
+// re-scan of queries the tcgen05 pass could not prove passes false: it reads the fp32 rows with EPS_GEMV_F32, whose
+// bound is ~800x tighter than the tensor pass's, and so settles them; the image's bound would be looser than it.
 int gemv_pass(orx_index *ix, const float *q_src, int q0, int nq, int k, const SearchCtx &ctx,
-              const FilterOnDevice *f = nullptr) {
+              const FilterOnDevice *f = nullptr, bool allow_image = true) {
     const uint32_t n_rows = (uint32_t)ix->n_live;
     const int grid = orx::scan_gemv_grid(ix->device, n_rows);
-    const double eps = ix->dtype == ORX_DTYPE_F32 ? orx::EPS_GEMV_F32 : orx::EPS_GEMV_BF16;
-    const int slots = orx::slots_for_k(k);
+    const bool img = allow_image && use_image(ix);
+    const int scan_dtype = img ? ORX_DTYPE_BF16 : ix->dtype;      // the element type the scan reads
+    const void *scan_rows = img ? static_cast<const void *>(ix->image) : ix->table;
+    const double eps = img ? orx::EPS_GEMV_IMAGE : ix->dtype == ORX_DTYPE_F32 ? orx::EPS_GEMV_F32 : orx::EPS_GEMV_BF16;
+    const int slots = img ? orx::image_slots_for_k(k) : orx::slots_for_k(k);
     for (int s = 0; s < nq; s += GEMV_QCHUNK) {
         const int m = std::min(GEMV_QCHUNK, nq - s);
         const int qa = q0 + s;
@@ -639,14 +719,14 @@ int gemv_pass(orx_index *ix, const float *q_src, int q0, int nq, int k, const Se
         cudaEvent_t e0 = scan_event(ix), e1 = scan_event(ix);
         if (e0 && e1) CK(cudaEventRecord(e0, ix->stream));
         if (f)
-            orx::launch_scan_gemv_filtered(ix->dtype, ix->table, ix->scale, n_rows, f->bits,
+            orx::launch_scan_gemv_filtered(scan_dtype, scan_rows, ix->scale, n_rows, f->bits,
                                            ix->cur->qhat.p + (size_t)qa * ORX_DIM, m, slots, ix->cur->partial.p, grid,
                                            ix->stream);
         else if (m >= 2)
-            orx::launch_scan_gemv_batch(ix->dtype, ix->table, ix->scale, n_rows, ix->cur->qhat.p + (size_t)qa * ORX_DIM, m,
+            orx::launch_scan_gemv_batch(scan_dtype, scan_rows, ix->scale, n_rows, ix->cur->qhat.p + (size_t)qa * ORX_DIM, m,
                                         slots, ix->cur->partial.p, parts, ix->stream);
         else
-            orx::launch_scan_gemv(ix->dtype, ix->table, ix->scale, n_rows, ix->cur->qhat.p + (size_t)qa * ORX_DIM, m,
+            orx::launch_scan_gemv(scan_dtype, scan_rows, ix->scale, n_rows, ix->cur->qhat.p + (size_t)qa * ORX_DIM, m,
                                   slots, ix->cur->partial.p, grid, ix->stream);
         if (e0 && e1) CK(cudaEventRecord(e1, ix->stream));
         // a filter's row bound is the eligible count: "every eligible row is a candidate" when it fits the list
@@ -706,7 +786,7 @@ int stage_queries(orx_index *ix, const float *queries, int nq, const float **q_s
     return ORX_OK;
 }
 
-// ---- the scan + finalize of all nq queries (tcgen05 for batches, GEMV otherwise); *path = 1 / 2
+// ---- the scan + finalize of all nq queries (tcgen05 for batches, GEMV otherwise); *path = 1 / 2 / 3 (GEMV over the image)
 //      f: a filter with a bitmap.  A BATCH of filtered queries whose bitmap scans together would read more than the
 //      whole table takes ONE tcgen05 pass over all rows instead: the predicate enters through the per-row scale (a
 //      cleared bit -> the "never a candidate" marker), so the kernel and its candidate proof are those of orx_search.
@@ -729,7 +809,8 @@ int scan_pass(orx_index *ix, const float *q_src, int nq, int k, const SearchCtx 
         if (rc != ORX_OK) return fail(rc, "tcgen05 scan failed: %s", orx::umma_last_error());
         return ORX_OK;
     }
-    *path = 1;
+    ensure_image(ix);
+    *path = use_image(ix) ? 3 : 1;
     return gemv_pass(ix, q_src, 0, nq, k, ctx, f);
 }
 
@@ -829,7 +910,7 @@ int resolve_unproven(orx_index *ix, const float *q_src, int nq, int k, const orx
             int j1 = j + 1;                                    // a run of flagged neighbours shares its table passes
             while (j1 < nq && (hflags[j1] & 1)) ++j1;
             ix->stats.fallback_gemv += (uint64_t)(j1 - j);
-            int rc = gemv_pass(ix, q_src, j, j1 - j, k, ctx);
+            int rc = gemv_pass(ix, q_src, j, j1 - j, k, ctx, nullptr, /*allow_image=*/false);
             if (rc != ORX_OK) return rc;
             j = j1;
         }
@@ -1523,6 +1604,7 @@ void orx_destroy(orx_index *ix) {
     cudaFree(ix->scale);
     cudaFree(ix->n2);
     cudaFree(ix->row_ids);
+    if (ix->image) cudaFree(ix->image);
     ix->fb_list.release(); ix->fb_count.release(); ix->fb_dist.release();
     ix->mmr_rows.release(); ix->mmr_stage.release(); ix->mmr_idx.release(); ix->mmr_dist.release();
     ix->mmr_cnt.release(); ix->mmr_sel.release();
@@ -1556,13 +1638,15 @@ int orx_set_stream(orx_index *ix, void *cuda_stream) {
 
 int orx_set_option(orx_index *ix, int option, int value) {
     if (!ix) return fail(ORX_ERR_INVALID, "index is null");
-    if (option != ORX_OPT_SCAN_TIMING) return fail(ORX_ERR_INVALID, "unknown option %d", option);
+    if (option != ORX_OPT_SCAN_TIMING && option != ORX_OPT_IMAGE_MIN_ROWS)
+        return fail(ORX_ERR_INVALID, "unknown option %d", option);
     if (ix->group) {
         for (orx_index *s : ix->group->shards) orx_set_option(s, option, value);
         return ORX_OK;
     }
     std::lock_guard<std::mutex> lk(ix->mu);
-    ix->scan_timing = value != 0;
+    if (option == ORX_OPT_SCAN_TIMING) ix->scan_timing = value != 0;
+    else ix->image_min_rows = value < 0 ? UINT64_MAX : (uint64_t)value;
     return ORX_OK;
 }
 
@@ -1674,7 +1758,7 @@ int orx_delete(orx_index *ix, const orx_id *ids, uint64_t n, uint64_t *n_removed
         CK(cudaMemcpyAsync(ix->d_src_idx.p, ix->h_u32a.p, hmv * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(ix->d_dst_row.p, ix->h_u32b.p, hmv * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
         orx::launch_move_rows(ix->dtype, ix->d_src_idx.p, ix->d_dst_row.p, (uint32_t)hmv, ix->table, ix->scale,
-                              ix->n2, ix->row_ids, st);
+                              ix->n2, ix->row_ids, ix->image, st);
         ix->stats.kernel_launches += 1;
         ix->stats.rows_moved += hmv;
         CK(cudaStreamSynchronize(st));
@@ -1978,7 +2062,7 @@ int orx_import_rows(orx_index *ix, const orx_id *ids, const void *rows_raw, uint
                        is_device_ptr(rows_raw) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(ix->d_ids.p, ids, n * sizeof(orx_id), cudaMemcpyHostToDevice, st));
     orx::launch_adopt_rows(ix->dtype, ix->table, (uint32_t)row0, (uint32_t)n, ix->d_ids.p, ix->scale, ix->n2,
-                           ix->row_ids, ix->d_flag.p, st);
+                           ix->row_ids, ix->d_flag.p, ix->image, st);
     ix->stats.kernel_launches += 1;
     CK(cudaMemcpyAsync(ix->h_flag.p, ix->d_flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
@@ -2104,6 +2188,28 @@ int orx_debug_fast_scores(orx_index *ix, const float *queries, int nq, float *ou
     if (rc != ORX_OK) return rc;
     orx::launch_dump_fast_scores(ix->dtype, ix->table, ix->scale, (uint32_t)ix->n_live, ix->cur->qhat.p, nq, out_device,
                                  ix->stream);
+    ix->stats.kernel_launches += 1;
+    CK(cudaStreamSynchronize(ix->stream));
+    CK(cudaGetLastError());
+    return ORX_OK;
+}
+
+int orx_debug_image_scores(orx_index *ix, const float *queries, int nq, float *out_device) {
+    if (!ix || !queries || !out_device) return fail(ORX_ERR_INVALID, "null argument");
+    if (ix->group) return fail(ORX_ERR_INVALID, "per-GPU diagnostic: call it on a single-GPU index");
+    if (!is_device_ptr(out_device)) return fail(ORX_ERR_INVALID, "out must be device memory");
+    if (nq < 1 || nq > 65535) return fail(ORX_ERR_INVALID, "1 <= nq <= 65535, got %d", nq);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    DeviceGuard g(ix->device);
+    if (any_in_flight(ix)) return fail(ORX_ERR_INVALID, "wait for the searches in flight (orx_search_wait) first");
+    if (ix->n_live == 0) return fail(ORX_ERR_INVALID, "empty table");
+    ensure_image(ix, /*force=*/true);
+    if (!ix->image) return fail(ORX_ERR_INVALID, "this index has no bf16 image (bf16 table, or no device memory for it)");
+    const float *q_src = nullptr;
+    int rc = stage_queries(ix, queries, nq, &q_src);
+    if (rc != ORX_OK) return rc;
+    orx::launch_dump_fast_scores(ORX_DTYPE_BF16, ix->image, ix->scale, (uint32_t)ix->n_live, ix->cur->qhat.p, nq,
+                                 out_device, ix->stream);
     ix->stats.kernel_launches += 1;
     CK(cudaStreamSynchronize(ix->stream));
     CK(cudaGetLastError());

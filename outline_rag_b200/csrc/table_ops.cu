@@ -5,6 +5,9 @@
 //           canonical binary64 |x|^2 (`n2`) are computed HERE, once, so a query never touches norms.
 //           fp32 tables keep the row bits verbatim (so the canonical rescore sees exactly what the
 //           caller stored); bf16 tables store RNE_bf16(x/|x|) and the norm of that rounded row.
+//           An fp32 table may also keep a bf16 IMAGE: RNE_bf16(x) of every element, not normalised (the
+//           row's fp32 `scale` applies to it unchanged).  The large-table GEMV scans read it instead of the
+//           fp32 rows (half the bytes); every kernel here that writes or moves rows keeps it in step.
 // delete  = `vector_store.adelete` -> DELETE ... WHERE langchain_id IN (...) (app/rag.py:231, :371);
 //           the host plans disjoint (last live row -> hole) moves, so the table stays dense and the
 //           scan needs no tombstone test.
@@ -45,7 +48,8 @@ __global__ void __launch_bounds__(256)
 commit_rows_kernel(const float *__restrict__ src, const uint32_t *__restrict__ src_idx,
                    const uint32_t *__restrict__ dst_row, const orx_id *__restrict__ ids, uint32_t n,
                    T *__restrict__ table, float *__restrict__ scale, double *__restrict__ n2_out,
-                   orx_id *__restrict__ row_ids, const int *__restrict__ abort_flag) {
+                   orx_id *__restrict__ row_ids, const int *__restrict__ abort_flag,
+                   __nv_bfloat16 *__restrict__ image) {
     // the batch's element check (validate_rows, earlier on this stream) found a NaN / Inf: nothing is written --
     // the whole batch is rejected and the table stays as it was, without a host round trip in between
     if (abort_flag != nullptr && *abort_flag != 0) return;
@@ -68,6 +72,11 @@ commit_rows_kernel(const float *__restrict__ src, const uint32_t *__restrict__ s
         if constexpr (sizeof(T) == 4) {
 #pragma unroll
             for (int j = 0; j < 32; ++j) row[lane + 32 * j] = v[j];
+            if (image != nullptr) {
+                __nv_bfloat16 *img = image + (size_t)dst * ORX_DIM;
+#pragma unroll
+                for (int j = 0; j < 32; ++j) img[lane + 32 * j] = __float2bfloat16_rn(v[j]);
+            }
         } else {
             const double inv = (n2 > 0.0) ? __ddiv_rn(1.0, __dsqrt_rn(n2)) : 0.0;
 #pragma unroll
@@ -89,33 +98,36 @@ commit_rows_kernel(const float *__restrict__ src, const uint32_t *__restrict__ s
 
 void launch_commit_rows(int dtype, const float *src, const uint32_t *src_idx, const uint32_t *dst_row,
                         const orx_id *ids, uint32_t n, void *table, float *scale, double *n2,
-                        orx_id *row_ids, const int *abort_flag, cudaStream_t st) {
+                        orx_id *row_ids, const int *abort_flag, void *image, cudaStream_t st) {
     if (n == 0) return;
     uint32_t blocks = (n + 7) / 8;
     blocks = cap_grid(blocks, 8);
     if (dtype == ORX_DTYPE_F32)
         commit_rows_kernel<float><<<blocks, 256, 0, st>>>(src, src_idx, dst_row, ids, n,
-                                                          static_cast<float *>(table), scale, n2, row_ids, abort_flag);
+                                                          static_cast<float *>(table), scale, n2, row_ids, abort_flag,
+                                                          static_cast<__nv_bfloat16 *>(image));
     else
         commit_rows_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>(
-            src, src_idx, dst_row, ids, n, static_cast<__nv_bfloat16 *>(table), scale, n2, row_ids, abort_flag);
+            src, src_idx, dst_row, ids, n, static_cast<__nv_bfloat16 *>(table), scale, n2, row_ids, abort_flag, nullptr);
 }
 
 // Bulk load (snapshot restore / cold start): the rows were copied VERBATIM (table dtype) to the
 // table tail [row0, row0+n); this computes what upsert would have: finite check, canonical |x|^2 of
 // the row as stored, 1/|x|, the id column.  Nothing is visible to searches until the host bumps
-// the live row count, so a NaN/Inf batch is rejected without side effects.
+// the live row count, so a NaN/Inf batch is rejected without side effects.  An fp32 table's image rows are
+// built from the verbatim rows here (snapshots do not store the image).
 template <typename T>
 __global__ void __launch_bounds__(256)
 adopt_rows_kernel(const T *__restrict__ table, uint32_t row0, uint32_t n, const orx_id *__restrict__ ids,
                   float *__restrict__ scale, double *__restrict__ n2_out, orx_id *__restrict__ row_ids,
-                  int *__restrict__ flag) {
+                  int *__restrict__ flag, __nv_bfloat16 *__restrict__ image) {
     const int lane = threadIdx.x & 31;
     const uint32_t gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const uint32_t n_gw = gridDim.x * (blockDim.x >> 5);
     for (uint32_t i = gw; i < n; i += n_gw) {
         const uint32_t r = row0 + i;
         const T *row = table + (size_t)r * ORX_DIM;
+        __nv_bfloat16 *img = image != nullptr ? image + (size_t)r * ORX_DIM : nullptr;
         double p[32];
         bool bad = false;
 #pragma unroll
@@ -123,6 +135,7 @@ adopt_rows_kernel(const T *__restrict__ table, uint32_t row0, uint32_t n, const 
             const float v = row_elem<T>(row, lane + 32 * j);
             bad |= !isfinite(v);
             p[j] = __dmul_rn((double)v, (double)v);
+            if (img != nullptr) img[lane + 32 * j] = __float2bfloat16_rn(v);
         }
         const double n2 = bcast_lane0(canon_tree_1024(p));
         if (__any_sync(FULL_MASK, bad) && lane == 0) atomicOr(flag, 1);
@@ -135,16 +148,34 @@ adopt_rows_kernel(const T *__restrict__ table, uint32_t row0, uint32_t n, const 
 }
 
 void launch_adopt_rows(int dtype, const void *table, uint32_t row0, uint32_t n, const orx_id *ids, float *scale,
-                       double *n2, orx_id *row_ids, int *flag, cudaStream_t st) {
+                       double *n2, orx_id *row_ids, int *flag, void *image, cudaStream_t st) {
     if (n == 0) return;
     uint32_t blocks = (n + 7) / 8;
     blocks = cap_grid(blocks, 8);
     if (dtype == ORX_DTYPE_F32)
         adopt_rows_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float *>(table), row0, n, ids, scale, n2,
-                                                         row_ids, flag);
+                                                         row_ids, flag, static_cast<__nv_bfloat16 *>(image));
     else
         adopt_rows_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>(static_cast<const __nv_bfloat16 *>(table), row0, n,
-                                                                 ids, scale, n2, row_ids, flag);
+                                                                 ids, scale, n2, row_ids, flag, nullptr);
+}
+
+// the image of fp32 rows [0, n) that are already in the table (a grown table whose earlier allocation had no image)
+__global__ void __launch_bounds__(256)
+image_rows_kernel(const float4 *__restrict__ table, uint64_t n_vec4, uint2 *__restrict__ image) {
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n_vec4; i += (uint64_t)gridDim.x * blockDim.x) {
+        const float4 v = table[i];
+        const __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
+        image[i] = make_uint2(*reinterpret_cast<const uint32_t *>(&lo), *reinterpret_cast<const uint32_t *>(&hi));
+    }
+}
+
+void launch_image_rows(const float *table, uint64_t n, void *image, cudaStream_t st) {
+    if (n == 0) return;
+    const uint64_t n4 = n * (ORX_DIM / 4);
+    const uint64_t blocks = cap_grid((n4 + 255) / 256, 16);
+    image_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>(reinterpret_cast<const float4 *>(table), n4,
+                                                       static_cast<uint2 *>(image));
 }
 
 // one warp per relocated row; sources (>= new live count) and destinations (< new live count)
@@ -152,7 +183,7 @@ void launch_adopt_rows(int dtype, const void *table, uint32_t row0, uint32_t n, 
 __global__ void __launch_bounds__(256)
 move_rows_kernel(const uint32_t *__restrict__ src_row, const uint32_t *__restrict__ dst_row, uint32_t n,
                  uint4 *__restrict__ table, int vec_per_row, float *__restrict__ scale,
-                 double *__restrict__ n2, orx_id *__restrict__ row_ids) {
+                 double *__restrict__ n2, orx_id *__restrict__ row_ids, uint4 *__restrict__ image) {
     const int lane = threadIdx.x & 31;
     const uint32_t gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const uint32_t n_gw = gridDim.x * (blockDim.x >> 5);
@@ -161,6 +192,12 @@ move_rows_kernel(const uint32_t *__restrict__ src_row, const uint32_t *__restric
         const uint4 *sp = table + (size_t)s * vec_per_row;
         uint4 *dp = table + (size_t)d * vec_per_row;
         for (int j = lane; j < vec_per_row; j += 32) dp[j] = sp[j];
+        if (image != nullptr) {                  // 2048 B of image per row = 128 x 16 B
+            const uint4 *si = image + (size_t)s * 128;
+            uint4 *di = image + (size_t)d * 128;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) di[lane + 32 * j] = si[lane + 32 * j];
+        }
         if (lane == 0) {
             scale[d] = scale[s];
             n2[d] = n2[s];
@@ -170,13 +207,13 @@ move_rows_kernel(const uint32_t *__restrict__ src_row, const uint32_t *__restric
 }
 
 void launch_move_rows(int dtype, const uint32_t *src_row, const uint32_t *dst_row, uint32_t n,
-                      void *table, float *scale, double *n2, orx_id *row_ids, cudaStream_t st) {
+                      void *table, float *scale, double *n2, orx_id *row_ids, void *image, cudaStream_t st) {
     if (n == 0) return;
     uint32_t blocks = (n + 7) / 8;
     blocks = cap_grid(blocks, 8);
     const int vpr = dtype == ORX_DTYPE_F32 ? 256 : 128;
     move_rows_kernel<<<blocks, 256, 0, st>>>(src_row, dst_row, n, static_cast<uint4 *>(table), vpr,
-                                             scale, n2, row_ids);
+                                             scale, n2, row_ids, static_cast<uint4 *>(image));
 }
 
 template <typename T>
