@@ -63,7 +63,8 @@ typedef struct orx_stats {
     float    last_scan_ms;        /* device time of the last search's scan kernel(s) */
     float    last_search_ms;      /* host wall time of the last orx_search call     */
     int      last_path;           /* 0 none, 1 gemv scan, 2 tcgen05 scan,
-                                     3 gemv scan over the bf16 image of an fp32 table */
+                                     3 gemv scan over the bf16 image of an fp32 table,
+                                     4 gemv scan over the 8-bit image of an fp32 table */
     int      reserved;
     uint64_t scan_launches;       /* scan kernel launches (gemv or tcgen05)        */
     double   scan_ms_total;       /* sum of their device times (CUDA events around each launch) */
@@ -107,8 +108,19 @@ int orx_set_stream(orx_index *idx, void *cuda_stream);
  * the bytes a query streams; its candidates are still rescored canonically from the fp32 rows and the completeness proof
  * uses the image's error bound, so the answers are the same ids and distance bits (last_path reports 3).  0 = always
  * (when an image exists), a negative value = never.  bf16 tables have no image.  A multi-GPU handle sets every shard. */
+/* ORX_OPT_IMAGE8_MIN_ROWS (default 4194304 = 2^22): capacities from which an fp32 table's image is an 8-bit one INSTEAD of
+ * the bf16 one (a table holds at most one image; the kind is chosen when the image is allocated -- create, growth or the
+ * first search that needs it -- and growth past this capacity replaces a bf16 image by an 8-bit one).  Each row is kept
+ * as 1024 int8 X_i = rint(x_i / d), d = max|x_i| / 127, plus one fp32 d / |x|: 1 byte per element + 4 per row (10.3 GB
+ * at 10M rows instead of 20.5 GB for the bf16 image).  The single-query and filtered bitmap scans with k <= 12 read it
+ * (last_path 4) once ORX_OPT_IMAGE_MIN_ROWS live rows are reached, scoring each row by an exact integer dot with a
+ * 15-bit quantisation of the query: a quarter of the fp32 rows' bytes.  The candidates are rescored canonically from
+ * the fp32 rows, so ids and distance bits are those of the fp32 scan.  A row whose quantisation residual exceeds 2^-6
+ * of its norm is always a candidate; a table with more than 16 such rows, batches of GEMV queries (k > 64) and k > 12
+ * read the fp32 rows (last_path 1).  0 = every fp32 table that gets an image, a negative value = never. */
 #define ORX_OPT_SCAN_TIMING 1
 #define ORX_OPT_IMAGE_MIN_ROWS 2
+#define ORX_OPT_IMAGE8_MIN_ROWS 3
 int orx_set_option(orx_index *idx, int option, int value);
 
 uint64_t orx_size(const orx_index *idx);       /* live rows */
@@ -265,6 +277,11 @@ int orx_debug_fast_scores(orx_index *idx, const float *queries, int nq, float *o
  * their candidates on.  ORX_ERR_INVALID when the index has no image (bf16 table, or no device memory for it).
  * out_device [live rows, nq] fp32 in table row order.  1 <= nq <= 65535. */
 int orx_debug_image_scores(orx_index *idx, const float *queries, int nq, float *out_device);
+
+/* The same for the 8-bit image (ORX_OPT_IMAGE8_MIN_ROWS): (float(D) * dq) * scale8 of every live row, D the exact integer
+ * dot of the row's int8 image with the query's 15-bit quantisation -- the value the 8-bit scans key their candidates on.
+ * ORX_ERR_INVALID when the index has no 8-bit image (bf16 table, a bf16 image, or no device memory for it). */
+int orx_debug_image8_scores(orx_index *idx, const float *queries, int nq, float *out_device);
 
 /* Read back stored rows (as fp32) by id -- snapshot / debugging / tests.
  * out_vecs [n, dim] host; out_found [n] host (1/0). */

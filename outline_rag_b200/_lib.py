@@ -24,6 +24,7 @@ ORX_DIM = 1024
 ORX_MAX_K = 128
 ORX_OPT_SCAN_TIMING = 1
 ORX_OPT_IMAGE_MIN_ROWS = 2
+ORX_OPT_IMAGE8_MIN_ROWS = 3
 ORX_IPC_HANDLE_BYTES = 64
 DTYPE_F32 = 0
 DTYPE_BF16 = 1
@@ -112,6 +113,7 @@ SIGNATURES = {
     "orx_debug_coarse_scores": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp]),
     "orx_debug_fast_scores": (C.c_int, [_vp, _vp, C.c_int, _vp]),
     "orx_debug_image_scores": (C.c_int, [_vp, _vp, C.c_int, _vp]),
+    "orx_debug_image8_scores": (C.c_int, [_vp, _vp, C.c_int, _vp]),
     "orx_pgcopy_open": (C.c_int, [_vp, C.POINTER(_vp)]),
     "orx_pgcopy_open_sharded": (C.c_int, [_vp, C.c_int, C.c_int, C.POINTER(_vp)]),
     "orx_pgcopy_feed": (C.c_int, [_vp, _vp, C.c_uint64]),

@@ -13,11 +13,13 @@ namespace orx {
 
 // --------------------------------------------------------------- prep_queries
 // One warp per query: pgvector's input check (NaN/Inf -> error), canonical |q|^2,
-// normalised fp32 copy qhat (and its RNE bf16 image for the tcgen05 bf16 scan).
+// normalised fp32 copy qhat (and its RNE bf16 image for the tcgen05 bf16 scan, and its 15-bit quantisation for the
+// scan over an 8-bit image: Q_i = rint(qhat_i / dq), dq = max|qhat_i| / 16383, so |Q_i| <= 16383 and
+// |qhat_i - dq Q_i| <= dq / 2 (the division is binary64), i.e. |qhat - dq Q| <= 16 dq <= 9.7662e-4; DESIGN.md section 2).
 __global__ void __launch_bounds__(128)
 prep_queries_kernel(const float *__restrict__ q_all, int nq, float *__restrict__ q_copy,
                     float *__restrict__ qhat_all, __nv_bfloat16 *__restrict__ qhat16_all,
-                    QueryPrep *__restrict__ prep) {
+                    int8_t *__restrict__ qhat8_all, QueryPrep *__restrict__ prep) {
     const int lane = threadIdx.x & 31;
     const int qi = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     pdl_launch_dependents();            // the scan's CTAs may take their SMs now; they wait for this grid before reading qhat
@@ -37,24 +39,40 @@ prep_queries_kernel(const float *__restrict__ q_all, int nq, float *__restrict__
     const bool any_bad = __any_sync(FULL_MASK, bad);
     const bool zero = !(n2q > 0.0);
     const double inv = (any_bad || zero) ? 0.0 : __ddiv_rn(1.0, __dsqrt_rn(n2q));
+    float amax = 0.f;
 #pragma unroll
     for (int j = 0; j < 32; ++j) {
         const float h = (any_bad || zero) ? 0.f : __double2float_rn(__dmul_rn((double)x[j], inv));
+        x[j] = h;
+        amax = fmaxf(amax, fabsf(h));
         qhat_all[(size_t)qi * ORX_DIM + lane + 32 * j] = h;
         if (qhat16_all) qhat16_all[(size_t)qi * ORX_DIM + lane + 32 * j] = __float2bfloat16_rn(h);
+    }
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) amax = fmaxf(amax, __shfl_xor_sync(FULL_MASK, amax, d));
+    const float dq = __fdiv_rn(amax, 16383.f);
+    if (qhat8_all) {
+        int8_t *q8 = qhat8_all + (size_t)qi * 2 * ORX_DIM;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+            const int Q = dq > 0.f ? __double2int_rn(__ddiv_rn((double)x[j], (double)dq)) : 0;
+            q8[lane + 32 * j] = (int8_t)(Q >> 7);                  // arithmetic shift: floor(Q / 128) in [-128, 127]
+            q8[ORX_DIM + lane + 32 * j] = (int8_t)(Q & 127);       // Q - 128 (Q >> 7) in [0, 127]
+        }
     }
     if (lane == 0) {
         prep[qi].n2q = n2q;
         prep[qi].nonfinite = any_bad ? 1 : 0;
         prep[qi].zero = zero ? 1 : 0;
+        prep[qi].dq8 = dq;
     }
 }
 
-void launch_prep_queries(const float *q, int nq, float *q_copy, float *qhat, void *qhat_bf16,
+void launch_prep_queries(const float *q, int nq, float *q_copy, float *qhat, void *qhat_bf16, int8_t *qhat8,
                          QueryPrep *prep, cudaStream_t st) {
     if (nq <= 0) return;
     prep_queries_kernel<<<(nq + 3) / 4, 128, 0, st>>>(q, nq, q_copy, qhat,
-                                                      static_cast<__nv_bfloat16 *>(qhat_bf16), prep);
+                                                      static_cast<__nv_bfloat16 *>(qhat_bf16), qhat8, prep);
 }
 
 __global__ void flags_from_prep_kernel(const QueryPrep *__restrict__ prep, int nq, int *__restrict__ flags) {

@@ -15,6 +15,24 @@ constexpr double EPS_GEMV_BF16 = 3.0e-6;  // same arithmetic on exactly-converte
 constexpr double EPS_GEMV_IMAGE = 3.92e-3;
 // live rows from which an fp32 table's single-query / k > 64 batch / bitmap scans read the image (ORX_OPT_IMAGE_MIN_ROWS)
 constexpr uint64_t IMAGE_MIN_ROWS = 1ull << 20;
+// the 8-bit image of a large fp32 table (ORX_OPT_IMAGE8_MIN_ROWS; DESIGN.md section 2): X_i = rint(x_i / d) with
+// d = max|x_i| / 127, scored as the exact integer dot with the query's 15-bit quantisation Q (step dq, residual
+// r_q <= 16 dq <= 9.7662e-4) times scale8 = d / |x| and dq.  A row whose relative residual |x - d X| / |x| exceeds
+// R8_CAP is an always-candidate (+inf marker), so with r_x <= R8_CAP:
+//   |s - cos| <= R8_CAP + (1 + R8_CAP) (r_q + 6e-8) + 2.5e-7 = 1.66172e-2, rounded up
+constexpr double R8_CAP = 1.0 / 64;
+constexpr double EPS_GEMV_IMAGE8 = 1.662e-2;
+// capacities from which an fp32 table's image is the 8-bit one instead of the bf16 one (ORX_OPT_IMAGE8_MIN_ROWS)
+constexpr uint64_t IMAGE8_MIN_ROWS = 1ull << 22;
+// rows over R8_CAP a table may hold before its searches read the fp32 rows again: every such row takes a slot of every
+// candidate list it reaches, and the 8-bit scan's lists keep at least this many keys beyond k
+constexpr uint64_t IMAGE8_MAX_CAPPED = 16;
+// the 8-bit scan's candidate lists: 160 keys (slots 5) for k <= IMAGE8_MAX_K.  Its eps puts ~200 rows of a 10M-row
+// table within 2 eps of the 12th best; a 160-key list proves every query of a 10M-row CPU emulation at k = 12 (least
+// margin 1.1e-3), a 128-key one leaves 4 of 32 unproven, and at k = 16 even 160 keys leave 1 of 32 (DESIGN.md section
+// 4).  Searches with a wider k read the fp32 rows.
+constexpr int IMAGE8_MAX_K = 12;
+constexpr int IMAGE8_SLOTS = 5;
 // kind::tf32 truncates both operands to 10 mantissa bits (measured on sm_100a, tests/test_epsilon_adversarial_gpu.py):
 // worst case (1+2^-10)^2-1 = 1.96e-3; a worst-case query against its own row measures 1.927e-3 (DESIGN.md section 2)
 constexpr double EPS_UMMA_TF32 = 2.5e-3;
@@ -35,6 +53,13 @@ struct QueryPrep {            // per query, written by prep_queries
     double n2q;               // canonical |q|^2
     int nonfinite;            // 1 if any element is NaN/Inf
     int zero;                 // 1 if |q| == 0 (every distance is NaN)
+    float dq8;                // step of the 15-bit quantisation of qhat the 8-bit scan reads (max|qhat_i| / 16383)
+};
+
+// the 8-bit image of an fp32 table, as the kernels that write or move rows see it; rows == nullptr: none
+struct Image8 {
+    int8_t *rows;             // [cap, ORX_DIM] X_i = rint(x_i / d)
+    float *scale8;            // [cap] d / |x|, or the row's scale marker (NaN zero row, +inf irregular or over R8_CAP)
 };
 
 // ---- where a search's results go and how its completion is signalled (finalize.cu, exchange.cu)
@@ -67,7 +92,9 @@ struct DoneArgs {
 };
 
 // ---- finalize.cu
-void launch_prep_queries(const float *q, int nq, float *q_copy, float *qhat, void *qhat_bf16,
+// qhat8 (nullptr: none): [nq, 2 * ORX_DIM] int8, the 15-bit quantisation Q of qhat split into Q >> 7 (elements 0..1023)
+// and Q & 127 (elements 1024..2047), for the 8-bit scan; its step goes to prep->dq8
+void launch_prep_queries(const float *q, int nq, float *q_copy, float *qhat, void *qhat_bf16, int8_t *qhat8,
                          QueryPrep *prep, cudaStream_t st);
 // q / prep / partial / floor are launch-relative (query 0 of this launch); results are written at q_base + query
 void launch_finalize(int dtype, const void *table, const double *n2, const orx_id *row_ids,
@@ -86,6 +113,9 @@ void launch_collect(int dtype, const void *table, const float *scale, uint32_t n
 // diagnostic: fast scores of every row for nq staged queries, out [n_rows, nq] (orx_debug_fast_scores)
 void launch_dump_fast_scores(int dtype, const void *table, const float *scale, uint32_t n_rows, const float *qhat,
                              int nq, float *out, cudaStream_t st);
+// the same diagnostic for the 8-bit scan (orx_debug_image8_scores)
+void launch_dump_image8_scores(const int8_t *image, const float *scale8, uint32_t n_rows, const int8_t *qhat8,
+                               const QueryPrep *prep, int nq, float *out, cudaStream_t st);
 void launch_rescore_list(int dtype, const void *table, const double *n2, const orx_id *row_ids,
                          const float *q, const QueryPrep *prep, const uint32_t *list,
                          const uint32_t *count, double *dist_out, cudaStream_t st);
@@ -121,18 +151,27 @@ void launch_scan_gemv_batch(int dtype, const void *table, const float *scale, ui
 void launch_scan_gemv_filtered(int dtype, const void *table, const float *scale, uint32_t n_rows,
                                const uint32_t *allow_bits, const float *qhat, int nq, int slots,
                                uint64_t *partial, int grid, cudaStream_t st);
+// the single-query and bitmap scans over the 8-bit image (IMAGE8_SLOTS lists); allow_bits == nullptr: every row
+void launch_scan_gemv8(const int8_t *image, const float *scale8, uint32_t n_rows, const uint32_t *allow_bits,
+                       const int8_t *qhat8, const QueryPrep *prep, int nq, uint64_t *partial, int grid, cudaStream_t st);
 
 // ---- table_ops.cu
 void launch_validate_rows(const float *src, uint64_t n, int *flag, cudaStream_t st);
 // image: the bf16 image of an fp32 table ([cap, ORX_DIM] __nv_bfloat16), kept in step with the rows; nullptr = none
+//        image8: the 8-bit image (Image8::rows == nullptr: none); a table has at most one of the two
 void launch_commit_rows(int dtype, const float *src, const uint32_t *src_idx, const uint32_t *dst_row,
                         const orx_id *ids, uint32_t n, void *table, float *scale, double *n2,
-                        orx_id *row_ids, const int *abort_flag, void *image, cudaStream_t st);
+                        orx_id *row_ids, const int *abort_flag, void *image, const Image8 &image8, cudaStream_t st);
 void launch_adopt_rows(int dtype, const void *table, uint32_t row0, uint32_t n, const orx_id *ids, float *scale,
-                       double *n2, orx_id *row_ids, int *flag, void *image, cudaStream_t st);
+                       double *n2, orx_id *row_ids, int *flag, void *image, const Image8 &image8, cudaStream_t st);
 void launch_move_rows(int dtype, const uint32_t *src_row, const uint32_t *dst_row, uint32_t n,
-                      void *table, float *scale, double *n2, orx_id *row_ids, void *image, cudaStream_t st);
+                      void *table, float *scale, double *n2, orx_id *row_ids, void *image, const Image8 &image8,
+                      cudaStream_t st);
 void launch_image_rows(const float *table, uint64_t n, void *image, cudaStream_t st);     // image of rows [0, n)
+void launch_image8_rows(const float *table, const double *n2, const float *scale, uint64_t n, const Image8 &image8,
+                        cudaStream_t st);                                                 // 8-bit image of rows [0, n)
+// *count <- live rows [0, n) over R8_CAP (scale8 +inf while scale is regular)
+void launch_count_capped8(const float *scale, const float *scale8, uint64_t n, uint32_t *count, cudaStream_t st);
 void launch_gather_rows(int dtype, const void *table, const uint32_t *rows, uint32_t n, float *out,
                         cudaStream_t st);
 

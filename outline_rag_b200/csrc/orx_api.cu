@@ -244,6 +244,7 @@ struct Exchange {   // peer-memory exchange state of one rank (orx_shard_*) or o
 struct SearchSlot {         // everything ONE search in flight owns
     DevBuf<float> q_dev, qhat;
     DevBuf<__nv_bfloat16> qhat16;
+    DevBuf<int8_t> qhat8;               // fp32 tables: the 15-bit quantised queries of the 8-bit scan [nq, 2 * ORX_DIM]
     DevBuf<orx::QueryPrep> prep;
     DevBuf<uint64_t> partial;
     DevBuf<double> blk;                 // scratch result block (empty shard / error block of the row-sharded search)
@@ -274,7 +275,7 @@ struct SearchSlot {         // everything ONE search in flight owns
         std::chrono::steady_clock::time_point t_begin;
     } pend;
     void release() {
-        q_dev.release(); qhat.release(); qhat16.release(); prep.release(); partial.release(); blk.release();
+        q_dev.release(); qhat.release(); qhat16.release(); qhat8.release(); prep.release(); partial.release(); blk.release();
         h_q.release(); h_prep.release(); h_ids.release(); h_dist.release(); h_counts.release(); h_flags.release();
         h_myflags.release(); h_redo.release(); h_done.release(); d_counters.release();
         for (auto &e : scan_ev) cudaEventDestroy(e);
@@ -301,8 +302,16 @@ struct orx_index {
     // only for a capacity of image_min_rows rows or more (at create / growth, or by the first search that needs it),
     // and best effort: null when the device has no room (the scans then read the fp32 rows; bf16 tables never have one)
     __nv_bfloat16 *image = nullptr;
+    // ... or, for a capacity of image8_min_rows rows or more, the 8-bit image instead (never both): a quarter of the
+    // fp32 rows' bytes.  capped8 = live rows over R8_CAP, recounted by every write; more than IMAGE8_MAX_CAPPED of them
+    // and the scans read the fp32 rows again
+    orx::Image8 image8{nullptr, nullptr};
     uint64_t image_min_rows = orx::IMAGE_MIN_ROWS;    // ORX_OPT_IMAGE_MIN_ROWS
+    uint64_t image8_min_rows = orx::IMAGE8_MIN_ROWS;  // ORX_OPT_IMAGE8_MIN_ROWS
     uint64_t image_failed_cap = 0;                    // capacity at which allocating the image failed (no retry until it changes)
+    uint64_t capped8 = 0;
+    DevBuf<uint32_t> d_capped8;
+    PinBuf<uint32_t> h_capped8;
 
     // host mirror of the id column + id -> row map
     std::vector<orx_id> host_row_ids;
@@ -378,42 +387,97 @@ struct DeviceGuard {
     }
 };
 
-// the bf16 image of an fp32 table with room for `cap` rows, or nullptr: a bf16 table, a capacity below the row count from
-// which the scans would read it (small tables pay no memory for it), or no room left on the device
-__nv_bfloat16 *alloc_image(orx_index *ix, uint64_t cap) {
-    if (ix->dtype != ORX_DTYPE_F32 || cap < ix->image_min_rows) return nullptr;
-    void *p = nullptr;
-    if (cudaMalloc(&p, cap * ORX_DIM * sizeof(__nv_bfloat16)) != cudaSuccess) {
-        cudaGetLastError();
-        ix->image_failed_cap = cap;
-        return nullptr;
-    }
-    return static_cast<__nv_bfloat16 *>(p);
+// the image a capacity gets: 2 the 8-bit one (from image8_min_rows rows), 1 the bf16 one (from image_min_rows rows), 0
+// none (bf16 tables, small capacities: small tables pay no memory for it)
+int image_kind_for(const orx_index *ix, uint64_t cap) {
+    if (ix->dtype != ORX_DTYPE_F32) return 0;
+    return cap >= ix->image8_min_rows ? 2 : cap >= ix->image_min_rows ? 1 : 0;
 }
-bool use_image(const orx_index *ix) { return ix->image != nullptr && ix->n_live >= ix->image_min_rows; }
+int image_kind(const orx_index *ix) { return ix->image8.rows ? 2 : ix->image ? 1 : 0; }
 
-// an fp32 table that has reached image_min_rows live rows (or whose option was lowered below its size) without an image:
-// allocate one and build it from the live rows, once per capacity.  Best effort: without it the scans read the fp32 rows.
-// force: the diagnostic hook, which wants the image whatever the threshold.
-void ensure_image(orx_index *ix, bool force = false) {
-    if (ix->image || ix->dtype != ORX_DTYPE_F32 || ix->n_live == 0 || ix->image_failed_cap == ix->capacity) return;
-    if (!force && ix->n_live < ix->image_min_rows) return;
-    const uint64_t keep = ix->image_min_rows;
-    ix->image_min_rows = 0;                       // the capacity test of alloc_image is this function's own decision
-    __nv_bfloat16 *im = alloc_image(ix, ix->capacity);
-    ix->image_min_rows = keep;
-    if (!im) {
-        ix->image_failed_cap = ix->capacity;
-        return;
+struct ImageAlloc {
+    __nv_bfloat16 *bf16 = nullptr;
+    orx::Image8 i8{nullptr, nullptr};
+    bool ok() const { return bf16 || i8.rows; }
+    void release() {
+        if (bf16) cudaFree(bf16);
+        if (i8.rows) cudaFree(i8.rows);
+        if (i8.scale8) cudaFree(i8.scale8);
+        *this = ImageAlloc{};
     }
-    orx::launch_image_rows(static_cast<const float *>(ix->table), ix->n_live, im, ix->stream);
+};
+// an image of `kind` with room for `cap` rows; best effort: none when the device has no room
+ImageAlloc alloc_image(orx_index *ix, uint64_t cap, int kind) {
+    ImageAlloc a;
+    if (kind == 0) return a;
+    cudaError_t e = kind == 1 ? cudaMalloc(&a.bf16, cap * ORX_DIM * sizeof(__nv_bfloat16))
+                              : cudaMalloc(&a.i8.rows, cap * ORX_DIM * sizeof(int8_t));
+    if (e == cudaSuccess && kind == 2) e = cudaMalloc(&a.i8.scale8, cap * sizeof(float));
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        a.release();
+        ix->image_failed_cap = cap;
+    }
+    return a;
+}
+void free_image(orx_index *ix) {
+    ImageAlloc{ix->image, ix->image8}.release();
+    ix->image = nullptr;
+    ix->image8 = orx::Image8{nullptr, nullptr};
+}
+// build image a of the first n rows from a table's fp32 rows (and their n2 / scale)
+void build_image(const ImageAlloc &a, const void *table, const double *n2, const float *scale, uint64_t n,
+                 cudaStream_t st) {
+    if (a.bf16) orx::launch_image_rows(static_cast<const float *>(table), n, a.bf16, st);
+    else orx::launch_image8_rows(static_cast<const float *>(table), n2, scale, n, a.i8, st);
+}
+// the 8-bit image's over-cap count of rows [0, n) into h_capped8, stream-ordered (read it after the next sync)
+cudaError_t launch_recount8(orx_index *ix, uint64_t n) {
+    cudaError_t e = ix->d_capped8.ensure(1);
+    if (e == cudaSuccess) e = ix->h_capped8.ensure(1);
+    if (e != cudaSuccess) return e;
+    orx::launch_count_capped8(ix->scale, ix->image8.scale8, n, ix->d_capped8.p, ix->stream);
     ix->stats.kernel_launches += 1;
-    if (cudaGetLastError() != cudaSuccess) {      // nothing was launched: stay without an image
-        cudaFree(im);
+    return cudaMemcpyAsync(ix->h_capped8.p, ix->d_capped8.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, ix->stream);
+}
+
+// rows a GEMV launch of m queries reads: 4 the 8-bit image (one query or a bitmap scan, k <= IMAGE8_MAX_K, few rows
+// over R8_CAP), 3 the bf16 image, 1 the table's own rows (also below image_min_rows live rows)
+int gemv_source(const orx_index *ix, int m, int k, bool filtered) {
+    if (ix->n_live < ix->image_min_rows) return 1;
+    if (ix->image) return 3;
+    if (ix->image8.rows && (filtered || m == 1) && k <= orx::IMAGE8_MAX_K && ix->capped8 <= orx::IMAGE8_MAX_CAPPED)
+        return 4;
+    return 1;
+}
+
+// an fp32 table that has reached image_min_rows live rows (or whose options were changed) without the image its capacity
+// gets: allocate that one and build it from the live rows, once per capacity (an image of the other kind is dropped
+// first).  Best effort: without it the scans read the fp32 rows.  force_kind: the diagnostic hooks, which want an image
+// whatever the thresholds (and keep one of either kind).
+void ensure_image(orx_index *ix, int force_kind = 0) {
+    if (ix->dtype != ORX_DTYPE_F32 || ix->n_live == 0) return;
+    if (!force_kind && ix->n_live < ix->image_min_rows) return;
+    const int kind = force_kind ? force_kind : ix->capacity >= ix->image8_min_rows ? 2 : 1;
+    if (image_kind(ix) == kind || (force_kind && image_kind(ix)) || ix->image_failed_cap == ix->capacity) return;
+    free_image(ix);
+    ImageAlloc a = alloc_image(ix, ix->capacity, kind);
+    if (!a.ok()) return;
+    build_image(a, ix->table, ix->n2, ix->scale, ix->n_live, ix->stream);
+    ix->stats.kernel_launches += 1;
+    ix->image = a.bf16;
+    ix->image8 = a.i8;
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess && kind == 2) e = launch_recount8(ix, ix->n_live);
+    if (e == cudaSuccess && kind == 2) e = cudaStreamSynchronize(ix->stream);
+    if (e != cudaSuccess) {                       // stay without an image
+        cudaGetLastError();
+        cudaStreamSynchronize(ix->stream);
+        free_image(ix);
         ix->image_failed_cap = ix->capacity;
         return;
     }
-    ix->image = im;                               // stream order: every later scan sees the built rows
+    if (kind == 2) ix->capped8 = *ix->h_capped8.p;  // stream order: every later scan sees the built rows
 }
 
 int alloc_table(orx_index *ix, uint64_t cap) {
@@ -421,7 +485,9 @@ int alloc_table(orx_index *ix, uint64_t cap) {
     CK(cudaMalloc(&ix->scale, cap * sizeof(float)));
     CK(cudaMalloc(&ix->n2, cap * sizeof(double)));
     CK(cudaMalloc(&ix->row_ids, cap * sizeof(orx_id)));
-    ix->image = alloc_image(ix, cap);             // after the table: the image never takes the table's room
+    const ImageAlloc a = alloc_image(ix, cap, image_kind_for(ix, cap));   // after the table: never takes the table's room
+    ix->image = a.bf16;
+    ix->image8 = a.i8;
     ix->capacity = cap;
     return ORX_OK;
 }
@@ -449,32 +515,33 @@ int grow_table(orx_index *ix, uint64_t need) {
         if (n) cudaFree(n);
         if (r) cudaFree(r);
         t = nullptr, s = nullptr, n = nullptr, r = nullptr;
-        if (!ix->image) break;
-        cudaFree(ix->image);                // the image is best effort: it gives its room to the table's growth
-        ix->image = nullptr;
+        if (!image_kind(ix)) break;
+        free_image(ix);                     // the image is best effort: it gives its room to the table's growth
     }
     if (e != cudaSuccess)
         return fail(ORX_ERR_CAPACITY, "cannot grow table to %llu rows: %s", (unsigned long long)cap,
                     cudaGetErrorString(e));
-    __nv_bfloat16 *im = nullptr;
-    if (ix->image) {                        // an image that exists is carried over whatever the threshold
-        const uint64_t keep = ix->image_min_rows;
-        ix->image_min_rows = 0;
-        im = alloc_image(ix, cap);
-        ix->image_min_rows = keep;
-    } else {
-        im = alloc_image(ix, cap);
-    }
+    const int kind_was = image_kind(ix);
+    int kind = image_kind_for(ix, cap);
+    if (kind == 0) kind = kind_was;         // an image that exists is carried over whatever the thresholds
+    ImageAlloc im = alloc_image(ix, cap, kind);
     e = cudaMemcpyAsync(t, ix->table, ix->n_live * rb, cudaMemcpyDeviceToDevice, ix->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(s, ix->scale, ix->n_live * sizeof(float), cudaMemcpyDeviceToDevice, ix->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(n, ix->n2, ix->n_live * sizeof(double), cudaMemcpyDeviceToDevice, ix->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(r, ix->row_ids, ix->n_live * sizeof(orx_id), cudaMemcpyDeviceToDevice, ix->stream);
-    if (e == cudaSuccess && im) {
-        if (ix->image)
-            e = cudaMemcpyAsync(im, ix->image, ix->n_live * ORX_DIM * sizeof(__nv_bfloat16), cudaMemcpyDeviceToDevice,
+    if (e == cudaSuccess && im.ok()) {
+        if (kind == kind_was && im.bf16)
+            e = cudaMemcpyAsync(im.bf16, ix->image, ix->n_live * ORX_DIM * sizeof(__nv_bfloat16), cudaMemcpyDeviceToDevice,
                                 ix->stream);
-        else
-            orx::launch_image_rows(static_cast<const float *>(ix->table), ix->n_live, im, ix->stream);
+        else if (kind == kind_was) {
+            e = cudaMemcpyAsync(im.i8.rows, ix->image8.rows, ix->n_live * ORX_DIM, cudaMemcpyDeviceToDevice, ix->stream);
+            if (e == cudaSuccess)
+                e = cudaMemcpyAsync(im.i8.scale8, ix->image8.scale8, ix->n_live * sizeof(float), cudaMemcpyDeviceToDevice,
+                                    ix->stream);
+        } else {                            // none yet, or bf16 -> 8-bit at image8_min_rows
+            build_image(im, ix->table, ix->n2, ix->scale, ix->n_live, ix->stream);
+            ix->stats.kernel_launches += 1;
+        }
         if (e == cudaSuccess) e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(ix->stream);
@@ -484,20 +551,26 @@ int grow_table(orx_index *ix, uint64_t need) {
         cudaFree(s);
         cudaFree(n);
         cudaFree(r);
-        if (im) cudaFree(im);
+        im.release();
         return fail(ORX_ERR_CUDA, "copying the table to its grown allocation failed: %s", cudaGetErrorString(e));
     }
     cudaFree(ix->table);
     cudaFree(ix->scale);
     cudaFree(ix->n2);
     cudaFree(ix->row_ids);
-    if (ix->image) cudaFree(ix->image);
+    free_image(ix);
     ix->table = t;
     ix->scale = s;
     ix->n2 = n;
     ix->row_ids = r;
-    ix->image = im;
+    ix->image = im.bf16;
+    ix->image8 = im.i8;
     ix->capacity = cap;
+    if (kind == 2 && kind_was != 2) {       // a rebuilt 8-bit image: count its rows over R8_CAP
+        CK(launch_recount8(ix, ix->n_live));
+        CK(cudaStreamSynchronize(ix->stream));
+        ix->capped8 = *ix->h_capped8.p;
+    }
     return ORX_OK;
 }
 
@@ -610,12 +683,14 @@ int upsert_locked(orx_index *ix, const orx_id *ids, const float *vecs, uint64_t 
         CK(cudaMemcpyAsync(ix->d_dst_row.p, ix->h_u32b.p, np * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(ix->d_ids.p, ids + s, m * sizeof(orx_id), cudaMemcpyHostToDevice, st));
         orx::launch_commit_rows(ix->dtype, src, ix->d_src_idx.p, ix->d_dst_row.p, ix->d_ids.p, np, ix->table,
-                                ix->scale, ix->n2, ix->row_ids, ix->d_flag.p, ix->image, st);
+                                ix->scale, ix->n2, ix->row_ids, ix->d_flag.p, ix->image, ix->image8, st);
         ix->stats.kernel_launches += 1;
+        if (ix->image8.rows) CK(launch_recount8(ix, next_row));
         CK(cudaMemcpyAsync(ix->h_flag.p, ix->d_flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));     // the ONE sync of a chunk: scratch + the caller's buffers are reusable after it
         CK(cudaGetLastError());
         if (*ix->h_flag.p) return fail(ORX_ERR_NONFINITE, "NaN or infinite value not allowed in vector");
+        if (ix->image8.rows) ix->capped8 = *ix->h_capped8.p;
         // ---- the device holds the rows: publish them
         if (!pending_list.empty()) {
             if (ix->host_row_ids.size() < next_row) ix->host_row_ids.resize(next_row);
@@ -698,27 +773,34 @@ int exhaustive_query(orx_index *ix, const float *q_src, int qi, int k, double dk
 
 // f: a filter with a bitmap -- the sequential scan skips the rows whose bit is clear (HBM traffic = eligible rows only).
 // allow_image: a large fp32 table with an image is scanned over the image (the bf16 instantiation of the same kernels,
-// the fp32 row's 1/|x|, EPS_GEMV_IMAGE); finalize rescores the fp32 rows either way, so the answer is the same.  The
+// the fp32 row's 1/|x|, EPS_GEMV_IMAGE; or the 8-bit scan, EPS_GEMV_IMAGE8, see gemv_source); finalize rescores the fp32
+// rows either way, so the answer is the same.  The
 // re-scan of queries the tcgen05 pass could not prove passes false: it reads the fp32 rows with EPS_GEMV_F32, whose
 // bound is ~800x tighter than the tensor pass's, and so settles them; the image's bound would be looser than it.
 int gemv_pass(orx_index *ix, const float *q_src, int q0, int nq, int k, const SearchCtx &ctx,
               const FilterOnDevice *f = nullptr, bool allow_image = true) {
     const uint32_t n_rows = (uint32_t)ix->n_live;
     const int grid = orx::scan_gemv_grid(ix->device, n_rows);
-    const bool img = allow_image && use_image(ix);
-    const int scan_dtype = img ? ORX_DTYPE_BF16 : ix->dtype;      // the element type the scan reads
-    const void *scan_rows = img ? static_cast<const void *>(ix->image) : ix->table;
-    const double eps = img ? orx::EPS_GEMV_IMAGE : ix->dtype == ORX_DTYPE_F32 ? orx::EPS_GEMV_F32 : orx::EPS_GEMV_BF16;
-    const int slots = img ? orx::image_slots_for_k(k) : orx::slots_for_k(k);
     for (int s = 0; s < nq; s += GEMV_QCHUNK) {
         const int m = std::min(GEMV_QCHUNK, nq - s);
         const int qa = q0 + s;
+        const int src = allow_image ? gemv_source(ix, m, k, f != nullptr) : 1;
+        const bool img = src == 3;
+        const int scan_dtype = img ? ORX_DTYPE_BF16 : ix->dtype;      // the element type the scan reads
+        const void *scan_rows = img ? static_cast<const void *>(ix->image) : ix->table;
+        const double eps = src == 4 ? orx::EPS_GEMV_IMAGE8 : img ? orx::EPS_GEMV_IMAGE
+                           : ix->dtype == ORX_DTYPE_F32 ? orx::EPS_GEMV_F32 : orx::EPS_GEMV_BF16;
+        const int slots = src == 4 ? orx::IMAGE8_SLOTS : img ? orx::image_slots_for_k(k) : orx::slots_for_k(k);
         // several queries: the batched kernel (8 queries share every row through shared memory); one: the streaming kernel
         const int parts = !f && m >= 2 ? orx::scan_gemv_batch_parts(ix->device, n_rows, m) : grid;
         CK(ix->cur->partial.ensure((size_t)m * parts * 32 * slots));
         cudaEvent_t e0 = scan_event(ix), e1 = scan_event(ix);
         if (e0 && e1) CK(cudaEventRecord(e0, ix->stream));
-        if (f)
+        if (src == 4)
+            orx::launch_scan_gemv8(ix->image8.rows, ix->image8.scale8, n_rows, f ? f->bits : nullptr,
+                                   ix->cur->qhat8.p + (size_t)qa * 2 * ORX_DIM, ix->cur->prep.p + qa, m,
+                                   ix->cur->partial.p, grid, ix->stream);
+        else if (f)
             orx::launch_scan_gemv_filtered(scan_dtype, scan_rows, ix->scale, n_rows, f->bits,
                                            ix->cur->qhat.p + (size_t)qa * ORX_DIM, m, slots, ix->cur->partial.p, grid,
                                            ix->stream);
@@ -752,6 +834,11 @@ int stage_queries(orx_index *ix, const float *queries, int nq, const float **q_s
     CK(ix->cur->qhat.ensure(nq_pad * ORX_DIM));
     CK(ix->cur->qhat16.ensure(nq_pad * ORX_DIM));
     CK(ix->cur->prep.ensure(nq));
+    int8_t *q8 = nullptr;                 // quantised for the 8-bit scan (fp32 tables: a search may build the image)
+    if (ix->dtype == ORX_DTYPE_F32) {
+        CK(ix->cur->qhat8.ensure((size_t)nq * 2 * ORX_DIM));
+        q8 = ix->cur->qhat8.p;
+    }
     if (nq_pad != (size_t)nq && nq > 1) {
         CK(cudaMemsetAsync(ix->cur->qhat.p + (size_t)nq * ORX_DIM, 0, (nq_pad - nq) * ORX_DIM * sizeof(float), st));
         CK(cudaMemsetAsync(ix->cur->qhat16.p + (size_t)nq * ORX_DIM, 0, (nq_pad - nq) * ORX_DIM * sizeof(__nv_bfloat16), st));
@@ -759,13 +846,13 @@ int stage_queries(orx_index *ix, const float *queries, int nq, const float **q_s
     const int qdev = ptr_device(queries);
     if (qdev == ix->device) {
         *q_src = queries;
-        orx::launch_prep_queries(queries, nq, nullptr, ix->cur->qhat.p, ix->cur->qhat16.p, ix->cur->prep.p, st);
+        orx::launch_prep_queries(queries, nq, nullptr, ix->cur->qhat.p, ix->cur->qhat16.p, q8, ix->cur->prep.p, st);
     } else if (qdev >= 0) {
         // the batch lives on ANOTHER GPU (a group's shards all receive the root's pointer): the prep kernel reads it
         // over NVLink once and leaves a local copy for the rescoring kernels
         CK(ix->cur->q_dev.ensure((size_t)nq * ORX_DIM));
         *q_src = ix->cur->q_dev.p;
-        orx::launch_prep_queries(queries, nq, ix->cur->q_dev.p, ix->cur->qhat.p, ix->cur->qhat16.p, ix->cur->prep.p, st);
+        orx::launch_prep_queries(queries, nq, ix->cur->q_dev.p, ix->cur->qhat.p, ix->cur->qhat16.p, q8, ix->cur->prep.p, st);
     } else {
         CK(ix->cur->q_dev.ensure((size_t)nq * ORX_DIM));
         const float *pinned = queries;
@@ -776,17 +863,18 @@ int stage_queries(orx_index *ix, const float *queries, int nq, const float **q_s
         }
         *q_src = ix->cur->q_dev.p;
         if (nq <= ZERO_COPY_MAX_Q) {
-            orx::launch_prep_queries(pinned, nq, ix->cur->q_dev.p, ix->cur->qhat.p, ix->cur->qhat16.p, ix->cur->prep.p, st);
+            orx::launch_prep_queries(pinned, nq, ix->cur->q_dev.p, ix->cur->qhat.p, ix->cur->qhat16.p, q8, ix->cur->prep.p, st);
         } else {
             CK(cudaMemcpyAsync(ix->cur->q_dev.p, pinned, (size_t)nq * ORX_DIM * sizeof(float), cudaMemcpyHostToDevice, st));
-            orx::launch_prep_queries(ix->cur->q_dev.p, nq, nullptr, ix->cur->qhat.p, ix->cur->qhat16.p, ix->cur->prep.p, st);
+            orx::launch_prep_queries(ix->cur->q_dev.p, nq, nullptr, ix->cur->qhat.p, ix->cur->qhat16.p, q8, ix->cur->prep.p, st);
         }
     }
     ix->stats.kernel_launches += 1;
     return ORX_OK;
 }
 
-// ---- the scan + finalize of all nq queries (tcgen05 for batches, GEMV otherwise); *path = 1 / 2 / 3 (GEMV over the image)
+// ---- the scan + finalize of all nq queries (tcgen05 for batches, GEMV otherwise); *path = 1 / 2 / 3 (GEMV over the bf16
+//      image) / 4 (GEMV over the 8-bit image)
 //      f: a filter with a bitmap.  A BATCH of filtered queries whose bitmap scans together would read more than the
 //      whole table takes ONE tcgen05 pass over all rows instead: the predicate enters through the per-row scale (a
 //      cleared bit -> the "never a candidate" marker), so the kernel and its candidate proof are those of orx_search.
@@ -810,7 +898,7 @@ int scan_pass(orx_index *ix, const float *q_src, int nq, int k, const SearchCtx 
         return ORX_OK;
     }
     ensure_image(ix);
-    *path = use_image(ix) ? 3 : 1;
+    *path = gemv_source(ix, f ? 1 : std::min(nq, GEMV_QCHUNK), k, f != nullptr);
     return gemv_pass(ix, q_src, 0, nq, k, ctx, f);
 }
 
@@ -1604,7 +1692,7 @@ void orx_destroy(orx_index *ix) {
     cudaFree(ix->scale);
     cudaFree(ix->n2);
     cudaFree(ix->row_ids);
-    if (ix->image) cudaFree(ix->image);
+    free_image(ix);
     ix->fb_list.release(); ix->fb_count.release(); ix->fb_dist.release();
     ix->mmr_rows.release(); ix->mmr_stage.release(); ix->mmr_idx.release(); ix->mmr_dist.release();
     ix->mmr_cnt.release(); ix->mmr_sel.release();
@@ -1638,7 +1726,7 @@ int orx_set_stream(orx_index *ix, void *cuda_stream) {
 
 int orx_set_option(orx_index *ix, int option, int value) {
     if (!ix) return fail(ORX_ERR_INVALID, "index is null");
-    if (option != ORX_OPT_SCAN_TIMING && option != ORX_OPT_IMAGE_MIN_ROWS)
+    if (option != ORX_OPT_SCAN_TIMING && option != ORX_OPT_IMAGE_MIN_ROWS && option != ORX_OPT_IMAGE8_MIN_ROWS)
         return fail(ORX_ERR_INVALID, "unknown option %d", option);
     if (ix->group) {
         for (orx_index *s : ix->group->shards) orx_set_option(s, option, value);
@@ -1646,7 +1734,8 @@ int orx_set_option(orx_index *ix, int option, int value) {
     }
     std::lock_guard<std::mutex> lk(ix->mu);
     if (option == ORX_OPT_SCAN_TIMING) ix->scan_timing = value != 0;
-    else ix->image_min_rows = value < 0 ? UINT64_MAX : (uint64_t)value;
+    else if (option == ORX_OPT_IMAGE_MIN_ROWS) ix->image_min_rows = value < 0 ? UINT64_MAX : (uint64_t)value;
+    else ix->image8_min_rows = value < 0 ? UINT64_MAX : (uint64_t)value;
     return ORX_OK;
 }
 
@@ -1758,11 +1847,15 @@ int orx_delete(orx_index *ix, const orx_id *ids, uint64_t n, uint64_t *n_removed
         CK(cudaMemcpyAsync(ix->d_src_idx.p, ix->h_u32a.p, hmv * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(ix->d_dst_row.p, ix->h_u32b.p, hmv * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
         orx::launch_move_rows(ix->dtype, ix->d_src_idx.p, ix->d_dst_row.p, (uint32_t)hmv, ix->table, ix->scale,
-                              ix->n2, ix->row_ids, ix->image, st);
+                              ix->n2, ix->row_ids, ix->image, ix->image8, st);
         ix->stats.kernel_launches += 1;
         ix->stats.rows_moved += hmv;
+    }
+    if (ix->image8.rows) CK(launch_recount8(ix, new_live));
+    if (hmv > 0 || ix->image8.rows) {
         CK(cudaStreamSynchronize(st));
         CK(cudaGetLastError());
+        if (ix->image8.rows) ix->capped8 = *ix->h_capped8.p;
     }
     if (n_removed) *n_removed = d;
     return ORX_OK;
@@ -2062,12 +2155,14 @@ int orx_import_rows(orx_index *ix, const orx_id *ids, const void *rows_raw, uint
                        is_device_ptr(rows_raw) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(ix->d_ids.p, ids, n * sizeof(orx_id), cudaMemcpyHostToDevice, st));
     orx::launch_adopt_rows(ix->dtype, ix->table, (uint32_t)row0, (uint32_t)n, ix->d_ids.p, ix->scale, ix->n2,
-                           ix->row_ids, ix->d_flag.p, ix->image, st);
+                           ix->row_ids, ix->d_flag.p, ix->image, ix->image8, st);
     ix->stats.kernel_launches += 1;
+    if (ix->image8.rows) CK(launch_recount8(ix, row0 + n));
     CK(cudaMemcpyAsync(ix->h_flag.p, ix->d_flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     CK(cudaGetLastError());
     if (*ix->h_flag.p) return fail(ORX_ERR_NONFINITE, "NaN or infinite value not allowed in vector");
+    if (ix->image8.rows) ix->capped8 = *ix->h_capped8.p;
     ix->host_row_ids.resize(row0 + n);
     for (uint64_t i = 0; i < n; ++i) {
         ix->host_row_ids[row0 + i] = ids[i];
@@ -2194,7 +2289,8 @@ int orx_debug_fast_scores(orx_index *ix, const float *queries, int nq, float *ou
     return ORX_OK;
 }
 
-int orx_debug_image_scores(orx_index *ix, const float *queries, int nq, float *out_device) {
+// kind 1: the bf16 image's scores, 2: the 8-bit image's
+int debug_image_scores(orx_index *ix, const float *queries, int nq, float *out_device, int kind) {
     if (!ix || !queries || !out_device) return fail(ORX_ERR_INVALID, "null argument");
     if (ix->group) return fail(ORX_ERR_INVALID, "per-GPU diagnostic: call it on a single-GPU index");
     if (!is_device_ptr(out_device)) return fail(ORX_ERR_INVALID, "out must be device memory");
@@ -2203,17 +2299,29 @@ int orx_debug_image_scores(orx_index *ix, const float *queries, int nq, float *o
     DeviceGuard g(ix->device);
     if (any_in_flight(ix)) return fail(ORX_ERR_INVALID, "wait for the searches in flight (orx_search_wait) first");
     if (ix->n_live == 0) return fail(ORX_ERR_INVALID, "empty table");
-    ensure_image(ix, /*force=*/true);
-    if (!ix->image) return fail(ORX_ERR_INVALID, "this index has no bf16 image (bf16 table, or no device memory for it)");
+    ensure_image(ix, kind);
+    if (image_kind(ix) != kind)
+        return fail(ORX_ERR_INVALID, "this index has no %s image (bf16 table, an image of the other kind, or no device "
+                    "memory for it)", kind == 1 ? "bf16" : "8-bit");
     const float *q_src = nullptr;
     int rc = stage_queries(ix, queries, nq, &q_src);
     if (rc != ORX_OK) return rc;
-    orx::launch_dump_fast_scores(ORX_DTYPE_BF16, ix->image, ix->scale, (uint32_t)ix->n_live, ix->cur->qhat.p, nq,
-                                 out_device, ix->stream);
+    if (kind == 1)
+        orx::launch_dump_fast_scores(ORX_DTYPE_BF16, ix->image, ix->scale, (uint32_t)ix->n_live, ix->cur->qhat.p, nq,
+                                     out_device, ix->stream);
+    else
+        orx::launch_dump_image8_scores(ix->image8.rows, ix->image8.scale8, (uint32_t)ix->n_live, ix->cur->qhat8.p,
+                                       ix->cur->prep.p, nq, out_device, ix->stream);
     ix->stats.kernel_launches += 1;
     CK(cudaStreamSynchronize(ix->stream));
     CK(cudaGetLastError());
     return ORX_OK;
+}
+int orx_debug_image_scores(orx_index *ix, const float *queries, int nq, float *out_device) {
+    return debug_image_scores(ix, queries, nq, out_device, 1);
+}
+int orx_debug_image8_scores(orx_index *ix, const float *queries, int nq, float *out_device) {
+    return debug_image_scores(ix, queries, nq, out_device, 2);
 }
 
 int orx_fetch(orx_index *ix, const orx_id *ids, uint64_t n, float *out_vecs, int *out_found) {

@@ -8,6 +8,7 @@
 //           An fp32 table may also keep a bf16 IMAGE: RNE_bf16(x) of every element, not normalised (the
 //           row's fp32 `scale` applies to it unchanged).  The large-table GEMV scans read it instead of the
 //           fp32 rows (half the bytes); every kernel here that writes or moves rows keeps it in step.
+//           A large fp32 table keeps an 8-bit image instead (quantise8_row): a quarter of the bytes.
 // delete  = `vector_store.adelete` -> DELETE ... WHERE langchain_id IN (...) (app/rag.py:231, :371);
 //           the host plans disjoint (last live row -> hole) moves, so the table stays dense and the
 //           scan needs no tombstone test.
@@ -43,13 +44,47 @@ __device__ __forceinline__ float scale_from_n2(double n2) {
     return __double2float_rn(__ddiv_rn(1.0, __dsqrt_rn(n2)));
 }
 
+// The 8-bit image of one fp32 row (warp-wide, lane l holds elements l + 32 j in v[j]): d = max|x_i| / 127,
+// X_i = rint(x_i / d) in [-127, 127], scale8 = d / |x| (binary64, rounded once).  The relative residual
+// |x - d X| / |x| is computed in binary64 from the stored X_i; a row over R8_CAP (with a 2^-30 margin for the binary64
+// sums) gets the +inf marker, so it is an always-candidate that only the canonical rescore settles.  Zero rows and rows
+// of irregular magnitude keep the marker of their fp32 `scale` (sc).  No fp32 operation here sees a subnormal result
+// that matters: the residual is measured, whatever rounding produced X.
+__device__ __forceinline__ void quantise8_row(const float (&v)[32], double n2, float sc, int lane,
+                                              int8_t *__restrict__ xrow, float *__restrict__ scale8_out) {
+    float m = 0.f;
+#pragma unroll
+    for (int j = 0; j < 32; ++j) m = fmaxf(m, fabsf(v[j]));
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) m = fmaxf(m, __shfl_xor_sync(FULL_MASK, m, d));
+    const bool regular = isfinite(sc);                 // not a marker
+    const float d = __fdiv_rn(m, 127.f);
+    double e2 = 0.0;
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+        const int8_t X = regular ? (int8_t)__float2int_rn(__fdiv_rn(v[j], d)) : (int8_t)0;
+        xrow[lane + 32 * j] = X;
+        const double e = __dsub_rn((double)v[j], (double)d * (double)X);    // d * X is exact in binary64
+        e2 = __fma_rn(e, e, e2);
+    }
+#pragma unroll
+    for (int o = 16; o >= 1; o >>= 1) e2 += __shfl_xor_sync(FULL_MASK, e2, o);
+    if (lane == 0) {
+        float s8 = sc;
+        if (regular)
+            s8 = e2 * (1.0 + 0x1p-30) <= R8_CAP * R8_CAP * n2 ? __double2float_rn(__ddiv_rn((double)d, __dsqrt_rn(n2)))
+                                                               : __int_as_float(0x7f800000);
+        *scale8_out = s8;
+    }
+}
+
 template <typename T>
 __global__ void __launch_bounds__(256)
 commit_rows_kernel(const float *__restrict__ src, const uint32_t *__restrict__ src_idx,
                    const uint32_t *__restrict__ dst_row, const orx_id *__restrict__ ids, uint32_t n,
                    T *__restrict__ table, float *__restrict__ scale, double *__restrict__ n2_out,
                    orx_id *__restrict__ row_ids, const int *__restrict__ abort_flag,
-                   __nv_bfloat16 *__restrict__ image) {
+                   __nv_bfloat16 *__restrict__ image, Image8 image8) {
     // the batch's element check (validate_rows, earlier on this stream) found a NaN / Inf: nothing is written --
     // the whole batch is rejected and the table stays as it was, without a host round trip in between
     if (abort_flag != nullptr && *abort_flag != 0) return;
@@ -77,6 +112,8 @@ commit_rows_kernel(const float *__restrict__ src, const uint32_t *__restrict__ s
 #pragma unroll
                 for (int j = 0; j < 32; ++j) img[lane + 32 * j] = __float2bfloat16_rn(v[j]);
             }
+            if (image8.rows != nullptr)
+                quantise8_row(v, n2, scale_from_n2(n2), lane, image8.rows + (size_t)dst * ORX_DIM, image8.scale8 + dst);
         } else {
             const double inv = (n2 > 0.0) ? __ddiv_rn(1.0, __dsqrt_rn(n2)) : 0.0;
 #pragma unroll
@@ -98,17 +135,18 @@ commit_rows_kernel(const float *__restrict__ src, const uint32_t *__restrict__ s
 
 void launch_commit_rows(int dtype, const float *src, const uint32_t *src_idx, const uint32_t *dst_row,
                         const orx_id *ids, uint32_t n, void *table, float *scale, double *n2,
-                        orx_id *row_ids, const int *abort_flag, void *image, cudaStream_t st) {
+                        orx_id *row_ids, const int *abort_flag, void *image, const Image8 &image8, cudaStream_t st) {
     if (n == 0) return;
     uint32_t blocks = (n + 7) / 8;
     blocks = cap_grid(blocks, 8);
     if (dtype == ORX_DTYPE_F32)
         commit_rows_kernel<float><<<blocks, 256, 0, st>>>(src, src_idx, dst_row, ids, n,
                                                           static_cast<float *>(table), scale, n2, row_ids, abort_flag,
-                                                          static_cast<__nv_bfloat16 *>(image));
+                                                          static_cast<__nv_bfloat16 *>(image), image8);
     else
         commit_rows_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>(
-            src, src_idx, dst_row, ids, n, static_cast<__nv_bfloat16 *>(table), scale, n2, row_ids, abort_flag, nullptr);
+            src, src_idx, dst_row, ids, n, static_cast<__nv_bfloat16 *>(table), scale, n2, row_ids, abort_flag, nullptr,
+            Image8{nullptr, nullptr});
 }
 
 // Bulk load (snapshot restore / cold start): the rows were copied VERBATIM (table dtype) to the
@@ -120,7 +158,7 @@ template <typename T>
 __global__ void __launch_bounds__(256)
 adopt_rows_kernel(const T *__restrict__ table, uint32_t row0, uint32_t n, const orx_id *__restrict__ ids,
                   float *__restrict__ scale, double *__restrict__ n2_out, orx_id *__restrict__ row_ids,
-                  int *__restrict__ flag, __nv_bfloat16 *__restrict__ image) {
+                  int *__restrict__ flag, __nv_bfloat16 *__restrict__ image, Image8 image8) {
     const int lane = threadIdx.x & 31;
     const uint32_t gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const uint32_t n_gw = gridDim.x * (blockDim.x >> 5);
@@ -128,17 +166,20 @@ adopt_rows_kernel(const T *__restrict__ table, uint32_t row0, uint32_t n, const 
         const uint32_t r = row0 + i;
         const T *row = table + (size_t)r * ORX_DIM;
         __nv_bfloat16 *img = image != nullptr ? image + (size_t)r * ORX_DIM : nullptr;
+        float v[32];
         double p[32];
         bool bad = false;
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
-            const float v = row_elem<T>(row, lane + 32 * j);
-            bad |= !isfinite(v);
-            p[j] = __dmul_rn((double)v, (double)v);
-            if (img != nullptr) img[lane + 32 * j] = __float2bfloat16_rn(v);
+            v[j] = row_elem<T>(row, lane + 32 * j);
+            bad |= !isfinite(v[j]);
+            p[j] = __dmul_rn((double)v[j], (double)v[j]);
+            if (img != nullptr) img[lane + 32 * j] = __float2bfloat16_rn(v[j]);
         }
         const double n2 = bcast_lane0(canon_tree_1024(p));
         if (__any_sync(FULL_MASK, bad) && lane == 0) atomicOr(flag, 1);
+        if (image8.rows != nullptr)             // a rejected batch is never published: its image rows do not matter
+            quantise8_row(v, n2, scale_from_n2(n2), lane, image8.rows + (size_t)r * ORX_DIM, image8.scale8 + r);
         if (lane == 0) {
             scale[r] = scale_from_n2(n2);
             n2_out[r] = n2;
@@ -148,16 +189,17 @@ adopt_rows_kernel(const T *__restrict__ table, uint32_t row0, uint32_t n, const 
 }
 
 void launch_adopt_rows(int dtype, const void *table, uint32_t row0, uint32_t n, const orx_id *ids, float *scale,
-                       double *n2, orx_id *row_ids, int *flag, void *image, cudaStream_t st) {
+                       double *n2, orx_id *row_ids, int *flag, void *image, const Image8 &image8, cudaStream_t st) {
     if (n == 0) return;
     uint32_t blocks = (n + 7) / 8;
     blocks = cap_grid(blocks, 8);
     if (dtype == ORX_DTYPE_F32)
         adopt_rows_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float *>(table), row0, n, ids, scale, n2,
-                                                         row_ids, flag, static_cast<__nv_bfloat16 *>(image));
+                                                         row_ids, flag, static_cast<__nv_bfloat16 *>(image), image8);
     else
         adopt_rows_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>(static_cast<const __nv_bfloat16 *>(table), row0, n,
-                                                                 ids, scale, n2, row_ids, flag, nullptr);
+                                                                 ids, scale, n2, row_ids, flag, nullptr,
+                                                                 Image8{nullptr, nullptr});
 }
 
 // the image of fp32 rows [0, n) that are already in the table (a grown table whose earlier allocation had no image)
@@ -178,12 +220,53 @@ void launch_image_rows(const float *table, uint64_t n, void *image, cudaStream_t
                                                        static_cast<uint2 *>(image));
 }
 
+// the 8-bit image of fp32 rows [0, n) that are already in the table, from their stored n2 and scale
+__global__ void __launch_bounds__(256)
+image8_rows_kernel(const float *__restrict__ table, const double *__restrict__ n2, const float *__restrict__ scale,
+                   uint64_t n, Image8 image8) {
+    const int lane = threadIdx.x & 31;
+    const uint64_t gw = blockIdx.x * (uint64_t)(blockDim.x >> 5) + (threadIdx.x >> 5);
+    const uint64_t n_gw = (uint64_t)gridDim.x * (blockDim.x >> 5);
+    for (uint64_t r = gw; r < n; r += n_gw) {
+        const float *row = table + r * ORX_DIM;
+        float v[32];
+#pragma unroll
+        for (int j = 0; j < 32; ++j) v[j] = row[lane + 32 * j];
+        quantise8_row(v, n2[r], scale[r], lane, image8.rows + r * ORX_DIM, image8.scale8 + r);
+    }
+}
+
+void launch_image8_rows(const float *table, const double *n2, const float *scale, uint64_t n, const Image8 &image8,
+                        cudaStream_t st) {
+    if (n == 0) return;
+    const uint64_t blocks = cap_grid((n + 7) / 8, 8);
+    image8_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>(table, n2, scale, n, image8);
+}
+
+__global__ void __launch_bounds__(256)
+count_capped8_kernel(const float *__restrict__ scale, const float *__restrict__ scale8, uint64_t n,
+                     uint32_t *__restrict__ count) {
+    uint32_t mine = 0;
+    for (uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; r < n; r += (uint64_t)gridDim.x * blockDim.x)
+        mine += (scale8[r] == __int_as_float(0x7f800000) && isfinite(scale[r])) ? 1u : 0u;
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) mine += __shfl_xor_sync(FULL_MASK, mine, d);
+    if ((threadIdx.x & 31) == 0 && mine) atomicAdd(count, mine);
+}
+
+void launch_count_capped8(const float *scale, const float *scale8, uint64_t n, uint32_t *count, cudaStream_t st) {
+    cudaMemsetAsync(count, 0, sizeof(uint32_t), st);
+    if (n == 0) return;
+    const uint64_t blocks = cap_grid((n + 255) / 256, 8);
+    count_capped8_kernel<<<(unsigned)blocks, 256, 0, st>>>(scale, scale8, n, count);
+}
+
 // one warp per relocated row; sources (>= new live count) and destinations (< new live count)
 // are disjoint sets, so all moves run in parallel.
 __global__ void __launch_bounds__(256)
 move_rows_kernel(const uint32_t *__restrict__ src_row, const uint32_t *__restrict__ dst_row, uint32_t n,
                  uint4 *__restrict__ table, int vec_per_row, float *__restrict__ scale,
-                 double *__restrict__ n2, orx_id *__restrict__ row_ids, uint4 *__restrict__ image) {
+                 double *__restrict__ n2, orx_id *__restrict__ row_ids, uint4 *__restrict__ image, Image8 image8) {
     const int lane = threadIdx.x & 31;
     const uint32_t gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const uint32_t n_gw = gridDim.x * (blockDim.x >> 5);
@@ -198,6 +281,13 @@ move_rows_kernel(const uint32_t *__restrict__ src_row, const uint32_t *__restric
 #pragma unroll
             for (int j = 0; j < 4; ++j) di[lane + 32 * j] = si[lane + 32 * j];
         }
+        if (image8.rows != nullptr) {            // 1024 B = 64 x 16 B
+            const uint4 *si = reinterpret_cast<const uint4 *>(image8.rows) + (size_t)s * 64;
+            uint4 *di = reinterpret_cast<uint4 *>(image8.rows) + (size_t)d * 64;
+            di[lane] = si[lane];
+            di[lane + 32] = si[lane + 32];
+            if (lane == 0) image8.scale8[d] = image8.scale8[s];
+        }
         if (lane == 0) {
             scale[d] = scale[s];
             n2[d] = n2[s];
@@ -207,13 +297,14 @@ move_rows_kernel(const uint32_t *__restrict__ src_row, const uint32_t *__restric
 }
 
 void launch_move_rows(int dtype, const uint32_t *src_row, const uint32_t *dst_row, uint32_t n,
-                      void *table, float *scale, double *n2, orx_id *row_ids, void *image, cudaStream_t st) {
+                      void *table, float *scale, double *n2, orx_id *row_ids, void *image, const Image8 &image8,
+                      cudaStream_t st) {
     if (n == 0) return;
     uint32_t blocks = (n + 7) / 8;
     blocks = cap_grid(blocks, 8);
     const int vpr = dtype == ORX_DTYPE_F32 ? 256 : 128;
     move_rows_kernel<<<blocks, 256, 0, st>>>(src_row, dst_row, n, static_cast<uint4 *>(table), vpr,
-                                             scale, n2, row_ids, static_cast<uint4 *>(image));
+                                             scale, n2, row_ids, static_cast<uint4 *>(image), image8);
 }
 
 template <typename T>

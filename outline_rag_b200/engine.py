@@ -388,6 +388,16 @@ class Index:
         check(lib.orx_debug_image_scores(self._h, C.c_void_p(ptr), nq, C.c_void_p(out.data_ptr())))
         return out
 
+    def debug_image8_scores(self, queries):
+        """Diagnostic (`orx_debug_image8_scores`): float32 CUDA tensor [live rows, nq] of the scores the scans over an fp32
+        table's 8-bit image key on, rows in table order.  Raises when the index has no 8-bit image."""
+        q = _host_f32(queries, "queries") if not _is_cuda_tensor(queries) else queries.contiguous()
+        nq = q.shape[0]
+        out = torch.empty((len(self), nq), dtype=torch.float32, device=f"cuda:{self.device}")
+        ptr = q.data_ptr() if _is_cuda_tensor(q) else q.ctypes.data
+        check(lib.orx_debug_image8_scores(self._h, C.c_void_p(ptr), nq, C.c_void_p(out.data_ptr())))
+        return out
+
     # -- two searches in flight (orx_search_submit / orx_search_wait)
     def search_submit(self, queries, k: int, out, sharded: bool = False) -> int:
         """Launch a search of a float32 CUDA tensor `queries` into the caller-owned CUDA tensors `out` =

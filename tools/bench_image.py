@@ -1,14 +1,17 @@
-"""The single-query exact scan of a large fp32 table over its bf16 image vs over its fp32 rows, on ONE index and one GPU.
+"""The single-query exact scan of a large fp32 table over its 8-bit image, over its bf16 image and over its fp32 rows, on
+ONE index and one GPU.
 
     python tools/bench_image.py [--rows 10000000] [--steps 200] [--reps 3] [--k 12]
 
-Builds rows x 1024 fp32 synthetic rows (bench.py's generator), then alternates ORX_OPT_IMAGE_MIN_ROWS between 0 (the
-GEMV scans read the bf16 image, last_path 3) and -1 (they read the fp32 rows, last_path 1) `reps` times.  Per arm: step
-time of a closed loop of batch-1 searches (device queries and outputs, CUDA events), the scan kernel's own device time
-(the library's per-launch event pair), the bytes one query actually streams (image: 2 B/element + 4 B scale; fp32:
-4 B/element + 4 B scale) and the bandwidth that makes, the fallback counters, and how many rows a query's finalize
-may rescore (rows whose fast score is within 2 eps + 1e-6 of the k-th best fast score -- an upper bound, measured with
-the debug hooks on a few queries).  Both arms must return the same ids and distance bits.  The card's name, power
+Builds rows x 1024 fp32 synthetic rows (bench.py's generator), then cycles `reps` times through three arms:
+ORX_OPT_IMAGE8_MIN_ROWS 0 (the GEMV scans read the 8-bit image, last_path 4), ORX_OPT_IMAGE8_MIN_ROWS -1 (the bf16
+image, last_path 3; a search rebuilds the image when the option changes its kind, outside the timed window) and
+ORX_OPT_IMAGE_MIN_ROWS -1 (the fp32 rows, last_path 1).  Per arm: step time of a closed loop of batch-1 searches
+(device queries and outputs, CUDA events), the scan kernel's own device time (the library's per-launch event pair), the
+bytes one query actually streams (8-bit: 1 B/element + 4 B scale8; bf16: 2 B/element + 4 B scale; fp32: 4 B/element +
+4 B scale) and the bandwidth that makes, the fallback counters, and how many rows a query's finalize rescores (rows
+whose fast score is within 2 eps + 1e-6 of the k-th best fast score, at most the candidate list's width -- measured
+with the debug hooks on a few queries).  All arms must return the same ids and distance bits.  The card's name, power
 limit and clocks are read in the same run.  Prints one JSON line."""
 import argparse
 import json
@@ -22,7 +25,8 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
-EPS = {"image": 3.92e-3, "fp32": 3.0e-6}            # csrc/internal.h EPS_GEMV_IMAGE / EPS_GEMV_F32
+EPS = {"image8": 1.662e-2, "image": 3.92e-3, "fp32": 3.0e-6}   # csrc/internal.h EPS_GEMV_IMAGE8 / _IMAGE / _F32
+LIST = {"image8": 160, "image": 64, "fp32": 32}                 # candidate keys per query at k <= 12
 
 
 def card(dev):
@@ -73,21 +77,26 @@ def main():
     out = (torch.empty((1, a.k, 2), dtype=torch.int64, device=Q.device),
            torch.empty((1, a.k), dtype=torch.float64, device=Q.device),
            torch.empty((1,), dtype=torch.int32, device=Q.device))
-    arms = {"image": 0, "fp32": -1}
+    arms = {"image8": (0, 0), "image": (-1, 0), "fp32": (0, -1)}    # (IMAGE8_MIN_ROWS, IMAGE_MIN_ROWS)
+
+    def arm(mode):
+        ix.set_option(_lib.ORX_OPT_IMAGE8_MIN_ROWS, arms[mode][0])
+        ix.set_option(_lib.ORX_OPT_IMAGE_MIN_ROWS, arms[mode][1])
 
     def answers(mode):
-        ix.set_option(_lib.ORX_OPT_IMAGE_MIN_ROWS, arms[mode])
+        arm(mode)
         got = [ix.search(Q[i:i + 1], a.k) for i in range(nq)]
         return (torch.cat([g[0] for g in got]).cpu().numpy(), torch.cat([g[1] for g in got]).cpu().numpy(),
                 ix.stats()["last_path"])
 
-    a_img, a_f32 = answers("image"), answers("fp32")
-    same = bool(np.array_equal(a_img[0], a_f32[0]) and np.array_equal(a_img[1].view(np.uint64), a_f32[1].view(np.uint64)))
+    ans = {m: answers(m) for m in arms}
+    same = all(bool(np.array_equal(ans[m][0], ans["fp32"][0]) and
+                    np.array_equal(ans[m][1].view(np.uint64), ans["fp32"][1].view(np.uint64))) for m in arms)
 
     runs = {m: [] for m in arms}
     for _ in range(a.reps):
         for mode in arms:
-            ix.set_option(_lib.ORX_OPT_IMAGE_MIN_ROWS, arms[mode])
+            arm(mode)
             for i in range(a.warmup):
                 ix.search(Q[i % nq:i % nq + 1], a.k, out=out)
             torch.cuda.synchronize()
@@ -109,17 +118,19 @@ def main():
     # rows finalize may rescore: fast score >= k-th best fast score - 2 eps - 1e-6 (finalize.cu, round 2 cut)
     rq = Q[:a.rescore_queries]
     rescore = {}
-    for mode, fn in (("image", ix.debug_image_scores), ("fp32", ix.debug_fast_scores)):
+    for mode, fn in (("image8", ix.debug_image8_scores), ("image", ix.debug_image_scores), ("fp32", ix.debug_fast_scores)):
+        arm(mode)
+        ix.search(Q[0:1], a.k, out=out)                # the image this arm reads
         s = fn(rq)
         kth = torch.topk(s, a.k, dim=0).values[-1]
         rescore[mode] = [int(c) for c in (s >= kth - (2 * EPS[mode] + 1e-6)).sum(dim=0).tolist()]
         del s
 
     elems = a.rows * 1024
-    bytes_q = {"image": elems * 2 + a.rows * 4, "fp32": elems * 4 + a.rows * 4}
-    res = {"what": "bf16 image vs fp32 rows, single-query exact scan", "rows": a.rows, "k": a.k, "steps": a.steps,
-           "reps": a.reps, "card": card(dev), "table_build_s": round(build_s, 2),
-           "same_ids_and_distance_bits": same, "paths": {"image": a_img[2], "fp32": a_f32[2]}, "arms": {}}
+    bytes_q = {"image8": elems + a.rows * 4, "image": elems * 2 + a.rows * 4, "fp32": elems * 4 + a.rows * 4}
+    res = {"what": "8-bit image vs bf16 image vs fp32 rows, single-query exact scan", "rows": a.rows, "k": a.k,
+           "steps": a.steps, "reps": a.reps, "card": card(dev), "table_build_s": round(build_s, 2),
+           "same_ids_and_distance_bits": same, "paths": {m: ans[m][2] for m in arms}, "arms": {}}
     for mode in arms:
         st = np.array([r["step_ms"] for r in runs[mode]])
         km = np.array([r["kernel_ms"] for r in runs[mode]])
@@ -131,9 +142,14 @@ def main():
             "TBps_kernel": round(bytes_q[mode] / (float(np.median(km)) * 1e-3) / 1e12, 3),
             "fallbacks": {"gemv": sum(r["fallback_gemv"] for r in runs[mode]),
                           "exhaustive": sum(r["fallback_exhaustive"] for r in runs[mode])},
-            "rows_within_2eps_of_kth": rescore[mode]}
-    res["speedup_step"] = round(res["arms"]["fp32"]["step_ms_median"] / res["arms"]["image"]["step_ms_median"], 3)
-    res["speedup_kernel"] = round(res["arms"]["fp32"]["kernel_ms_median"] / res["arms"]["image"]["kernel_ms_median"], 3)
+            "rows_within_2eps_of_kth": rescore[mode],
+            "rows_rescored": [min(c, LIST[mode]) for c in rescore[mode]]}
+    for mode in ("image8", "image"):
+        for what in ("step", "kernel"):
+            res[f"speedup_{what}_{mode}_vs_fp32"] = round(res["arms"]["fp32"][f"{what}_ms_median"] /
+                                                          res["arms"][mode][f"{what}_ms_median"], 3)
+    res["speedup_step_image8_vs_image"] = round(res["arms"]["image"]["step_ms_median"] /
+                                                res["arms"]["image8"]["step_ms_median"], 3)
     print(json.dumps(res), flush=True)
     ix.close()
 
