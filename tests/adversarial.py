@@ -87,11 +87,16 @@ def _fma32(a, b, c):
     return (a.astype(np.float64) * b.astype(np.float64) + c.astype(np.float64)).astype(np.float32)
 
 
-def gemv_fast(rows, qhat, dtype):
+def gemv_fast(rows, qhat, dtype, image=False):
     """Emulation of warp_row_dot (scan_common.cuh) times the row scale: lane l runs an fp32 FMA chain over its 32
-    elements in load order, then the xor butterfly 16, 8, 4, 2, 1.  rows: stored values as fp32 [n, D]."""
+    elements in load order, then the xor butterfly 16, 8, 4, 2, 1.  rows: stored values as fp32 [n, D].
+    image=True: the scan over the bf16 image of fp32 rows -- the chain runs over RNE-bf16 of the rows (8 elements per
+    vector), the scale is still the fp32 row's."""
     X = np.asarray(rows, np.float32).reshape(-1, D)
     qh = np.asarray(qhat, np.float32)
+    scale = row_scale(X)
+    if image:
+        X, dtype = bf16_exact(X), "bf16"
     w = 4 if dtype == "fp32" else 8                      # elements per lane per 16-byte vector
     # element order of lane l: vectors v = l + 32 j, elements w*v .. w*v + w-1
     lanes = np.arange(32)[:, None, None]
@@ -105,7 +110,7 @@ def gemv_fast(rows, qhat, dtype):
     for d in (16, 8, 4, 2, 1):
         acc = (acc + acc[:, np.arange(32) ^ d]).astype(np.float32)
     with np.errstate(invalid="ignore", over="ignore"):
-        return (acc[:, 0] * row_scale(X)).astype(np.float32)
+        return (acc[:, 0] * scale).astype(np.float32)
 
 
 def coarse_conversion_only(rows, qhat, dtype, mode=TF32_MODE):
@@ -247,3 +252,100 @@ def import_stored(ix, ids, rows):
     ids = np.ascontiguousarray(ids, np.uint64).reshape(-1, 2)
     assert ids.shape[0] == rows.shape[0]
     _lib.check(_lib.lib.orx_import_rows(ix._h, C.c_void_p(ids.ctypes.data), C.c_void_p(raw.ctypes.data), rows.shape[0]))
+
+
+# ------------------------------------------------------------------- inversions that only the image's eps can catch
+# The rank inversions above tie the winner's score bit for bit, so ANY positive eps fails their proof.  These make the
+# proof depend on the size of eps: the winner w's image score lies `deficit` below its cosine; k "strong" decoys are
+# exact in the image (score == cosine to ~1e-6) at cosines a little below w's; more fillers than a candidate list holds
+# score just above w, so w is not listed.  finalize then proves the decoys with any eps below the path's own (a wrong
+# answer) and fails with the path's eps (the exact fallback answers w first).
+EPS_UMMA = 2.5e-3                     # csrc/internal.h EPS_UMMA_TF32 / EPS_UMMA_BF16: the next bound below EPS_GEMV_IMAGE
+
+
+def proof_holds(scores, cos, k, K, eps):
+    """finalize's completeness proof (finalize.cu, GEMV scan) on emulated fast scores and exact cosines of every row:
+    the list is the K best scores; cut = s_k - 2 eps - 1e-6 drops listed rows from the rescore; the proof holds iff the
+    k-th best rescored cosine exceeds max(s_K, cut) + eps.  Returns (holds, listed rows)."""
+    s = np.asarray(scores, np.float32)
+    order = np.lexsort((np.arange(len(s)), -s.astype(np.float64)))
+    top = order[:K]
+    cut = np.float32(s[top[k - 1]] - np.float32(2.0 * eps + 1e-6))
+    resc = top[s[top] > cut]
+    cos_k = np.sort(np.asarray(cos, np.float64)[resc])[::-1][k - 1]
+    return bool(cos_k > max(float(s[top[-1]]), float(cut)) + eps), top
+
+
+def _toward(qh, c, rng):
+    """a random direction at cosine ~c to the unit vector qh (float64)"""
+    n = rng.standard_normal(D)
+    n -= (n @ qh) * qh
+    return c * qh + np.sqrt(1.0 - c * c) * n / np.linalg.norm(n)
+
+
+def _exact_rows(q, score, lo, hi, n, rng, make):
+    """n rows `make(direction)` whose score (`score(rows)`) lies in [lo, hi]: drawn at the band's centre, kept if in"""
+    qh = q.astype(np.float64) / np.linalg.norm(q.astype(np.float64))
+    out = []
+    for _ in range(200):
+        cand = np.stack([make(_toward(qh, (lo + hi) / 2, rng)) for _ in range(4 * n)])
+        s = score(cand)
+        out += list(cand[(s >= lo) & (s <= hi)])
+        if len(out) >= n:
+            return np.stack(out[:n])
+    raise AssertionError("band too narrow")
+
+
+def image8_inversion(k, seed=0, n_fillers=200, n_bulk=5000):
+    """(rows, q, w_row) for the 8-bit image: w = 2^-7 (X + f) with integer X (one element 127, the rest +-20..45) and
+    |f_i| = 0.484375 (just under half a step, so X is its 8-bit image) -- a relative residual ~0.0150, just under R8_CAP;
+    q = w^ + t f^ leans on that residual so that w's 8-bit score is ~1.25e-2 below its cosine.  Decoys and fillers are
+    2^-7 times integer vectors with max 127: their own image."""
+    from tests.test_image8_scan import image8_scores
+    rng = np.random.default_rng(seed)
+    X = rng.integers(20, 46, D) * rng.choice([-1, 1], D)
+    X[0] = 127
+    f = np.float32(0.5 - 2.0 ** -6) * rng.choice([-1.0, 1.0], D).astype(np.float32)
+    f[0] = 0
+    w = ((X + f) * 2.0 ** -7).astype(np.float32)
+    wh = w.astype(np.float64) / np.linalg.norm(w.astype(np.float64))
+    fh = f.astype(np.float64) / np.linalg.norm(f.astype(np.float64))
+    q = (wh + 1.5 * fh).astype(np.float32)
+    cw = float(cosine(w[None], q)[0])
+    sw = float(image8_scores(w[None], q)[0])
+
+    def exact(v):
+        return (np.rint(v * (127 / np.abs(v).max())) * 2.0 ** -7).astype(np.float32)
+
+    def score(rows):
+        return image8_scores(rows, q)
+    dec = _exact_rows(q, score, cw - 0.0045, cw - 0.0035, k, rng, exact)
+    fil = _exact_rows(q, score, sw + 0.0003, sw + 0.0015, n_fillers, rng, exact)
+    bulk = rng.standard_normal((n_bulk, D)).astype(np.float32)
+    rows = np.concatenate([dec, fil, bulk, w[None]]).astype(np.float32)   # the winner is the LAST row
+    return rows, q, w
+
+
+def image_inversion(k, seed=0, n_fillers=100, n_bulk=5000):
+    """(rows, q, w_row) for the bf16 image: every element of w is +-(1 + 2^-8) 2^e, the RNE tie that rounds down to the
+    even neighbour, so w's image is w / (1 + 2^-8) and its image score ~3.7e-3 below a cosine of ~0.95; decoys and
+    fillers are bf16-exact rows (their own image)."""
+    rng = np.random.default_rng(seed)
+    w = (np.float32(1 + 2.0 ** -8) * np.float32(2.0) ** rng.integers(-7, -3, D).astype(np.float32)
+         * rng.choice([-1.0, 1.0], D).astype(np.float32)).astype(np.float32)
+    wh = w.astype(np.float64) / np.linalg.norm(w.astype(np.float64))
+    q = _toward(wh, 0.95, rng).astype(np.float32)
+    qh, _ = prep_qhat(q)
+    cw = float(cosine(w[None], q)[0])
+    sw = float(gemv_fast(w[None], qh, "fp32", image=True)[0])
+
+    def exact(v):
+        return bf16_exact(v * (0.1 / np.abs(v).max()))
+
+    def score(rows):
+        return gemv_fast(rows, qh, "fp32", image=True)
+    dec = _exact_rows(q, score, cw - 0.0006, cw - 0.0002, k, rng, exact)
+    fil = _exact_rows(q, score, sw + 0.00005, sw + 0.0002, n_fillers, rng, exact)
+    bulk = rng.standard_normal((n_bulk, D)).astype(np.float32)
+    rows = np.concatenate([dec, fil, bulk, w[None]]).astype(np.float32)
+    return rows, q, w

@@ -173,3 +173,22 @@ def test_option_and_debug_hook_are_declared_and_bound():
     assert "int orx_debug_image8_scores(" in h and "orx_debug_image8_scores" in _lib.SIGNATURES
     assert _constexpr("IMAGE8_MIN_ROWS") == 1 << 22
     assert _constexpr("IMAGE8_MAX_K") == 12 and _constexpr("IMAGE8_SLOTS") == 5
+
+
+def test_eps_carries_the_answer_of_the_8bit_inversion():
+    """The construction of tests/test_image_property_gpu.py (adversarial.image8_inversion): finalize's proof over the
+    emulated 8-bit scores must FAIL with EPS_GEMV_IMAGE8 (the fallback then answers) and HOLD with the bf16 image's
+    EPS_GEMV_IMAGE -- which would prove k decoys in place of the winner.  So a search that handed the 8-bit scan a
+    smaller eps than its own returns a wrong answer there."""
+    for k in (1, 12):
+        rows, q, w = A.image8_inversion(k, seed=k)
+        s, cos = image8_scores(rows, q), A.cosine(rows, q)
+        n = len(rows)
+        assert np.argmax(cos) == n - 1 and np.isfinite(s).all()
+        assert 1.15e-2 < cos[-1] - s[-1] < EPS_GEMV_IMAGE8            # the winner's score is far below its cosine
+        assert np.abs(s[:k] - cos[:k]).max() < 1e-4                     # the decoys are their own 8-bit image
+        assert np.sum(s > s[-1]) > 160                                  # the winner is not listed
+        holds, top = A.proof_holds(s, cos, k, 160, EPS_GEMV_IMAGE8)
+        assert not holds and n - 1 not in top
+        holds, top = A.proof_holds(s, cos, k, 160, _constexpr("EPS_GEMV_IMAGE"))
+        assert holds and set(range(k)) <= set(top.tolist())

@@ -65,3 +65,26 @@ def test_option_and_debug_hook_are_declared_and_bound():
     assert m and int(m.group(1)) == _lib.ORX_OPT_IMAGE_MIN_ROWS != _lib.ORX_OPT_SCAN_TIMING
     assert "int orx_debug_image_scores(" in h and "orx_debug_image_scores" in _lib.SIGNATURES
     assert _constexpr("IMAGE_MIN_ROWS") == 1 << 20
+
+
+def test_eps_carries_the_answer_of_the_bf16_image_inversion():
+    """The construction of tests/test_image_property_gpu.py (adversarial.image_inversion): finalize's proof over the
+    emulated image scores must FAIL with EPS_GEMV_IMAGE and HOLD with the tensor pass's 2.5e-3 -- which would prove k
+    decoys in place of the winner."""
+    from tests import adversarial as A
+    eps_img = _constexpr("EPS_GEMV_IMAGE")
+    assert _constexpr("EPS_UMMA_TF32") == A.EPS_UMMA < eps_img
+    for k in (1, 12):
+        rows, q, w = A.image_inversion(k, seed=k)
+        qh, _ = A.prep_qhat(q)
+        s, cos = A.gemv_fast(rows, qh, "fp32", image=True), A.cosine(rows, q)
+        n = len(rows)
+        assert np.argmax(cos) == n - 1
+        assert 3.5e-3 < cos[-1] - s[-1] < eps_img                       # the winner's score is far below its cosine
+        assert np.abs(s[:k] - cos[:k]).max() < 1e-6                     # the decoys are their own image
+        width = 32 * (2 if k <= 16 else 4)                              # image_slots_for_k
+        assert np.sum(s > s[-1]) > width
+        holds, top = A.proof_holds(s, cos, k, width, eps_img)
+        assert not holds and n - 1 not in top
+        holds, top = A.proof_holds(s, cos, k, width, A.EPS_UMMA)
+        assert holds and set(range(k)) <= set(top.tolist())

@@ -244,23 +244,6 @@ def _worst_query(seed, n_zero=0):
     return q
 
 
-def image_fast(rows, qhat):
-    """Emulation of the image scans' score (tests/adversarial.py gemv_fast for bf16 rows): lane l runs an fp32 FMA chain
-    over the RNE-bf16 images of its 32 elements (8 per 16-byte vector), then the xor butterfly -- times the FP32 row's
-    scale, not the image's"""
-    X = np.asarray(rows, np.float32).reshape(-1, 1024)
-    img = A.bf16_exact(X)
-    order = (8 * (np.arange(32)[:, None, None] + 32 * np.arange(4)[None, :, None]) + np.arange(8)[None, None, :])
-    order = order.reshape(32, 32)
-    acc = np.zeros((X.shape[0], 32), np.float32)
-    for s in range(32):
-        e = order[:, s]
-        acc = A._fma32(img[:, e], np.asarray(qhat, np.float32)[e][None, :], acc)
-    for d in (16, 8, 4, 2, 1):
-        acc = (acc + acc[:, np.arange(32) ^ d]).astype(np.float32)
-    return (acc[:, 0] * A.row_scale(X)).astype(np.float32)
-
-
 def test_image_error_is_below_eps_and_reaches_its_worst_case():
     import outline_rag_b200 as orx
     qs = [_worst_query(s) for s in range(4)]
@@ -316,7 +299,7 @@ def inversion():
         q = _worst_query(seed, n_zero=64)
         w = A.with_zero_value(q, q)
         qh, _ = A.prep_qhat(q)
-        if A.cosine(w[None], q)[0] - image_fast(w[None], qh)[0] > 1e-3:
+        if A.cosine(w[None], q)[0] - A.gemv_fast(w[None], qh, "fp32", image=True)[0] > 1e-3:
             break
     else:
         raise AssertionError("no seed gives an image score that underestimates the winner's cosine")
