@@ -65,7 +65,8 @@ typedef struct orx_stats {
     int      last_path;           /* 0 none, 1 gemv scan, 2 tcgen05 scan,
                                      3 gemv scan over the bf16 image of an fp32 table,
                                      4 gemv scan over the 8-bit image of an fp32 table */
-    int      reserved;
+    uint32_t shared_scans;        /* searches that scored rows in another search's pass
+                                     (two single-query searches in flight over the 8-bit image) */
     uint64_t scan_launches;       /* scan kernel launches (gemv or tcgen05)        */
     double   scan_ms_total;       /* sum of their device times (CUDA events around each launch) */
 } orx_stats;
@@ -130,6 +131,9 @@ int orx_dtype(const orx_index *idx);
  * consistent iff this value is the same before the first and after the last call (Index.save checks it). */
 uint64_t orx_mutation_count(const orx_index *idx);
 int orx_get_stats(const orx_index *idx, orx_stats *out);
+/* rows scored for a search in another search's pass (the rows of the segments the searches counted by
+ * orx_stats.shared_scans joined); 0 on a multi-GPU handle */
+uint64_t orx_shared_rows(const orx_index *idx);
 
 /* Replaces `vector_store.aadd_documents(chunks)` -> per-row
  * `INSERT ... ON CONFLICT (langchain_id) DO UPDATE` (reference app/rag.py:235).
@@ -161,8 +165,9 @@ int orx_search(orx_index *idx, const float *queries, int nq, int dim, int k,
  * query -- staging, launches -- and its first kernels overlap the tail of the previous one: finalize, exchange, merge,
  * the completion hand-shake).  orx_search_submit launches the whole chain and returns at once with a ticket;
  * orx_search_wait(ticket) blocks until that search is complete, settles whatever the fast path could not prove, and
- * fills the output buffers given at submit (they and, for host queries, nothing else must stay valid until then;
- * the queries are copied at submit).  At most two tickets may be outstanding; wait for them in submission order.
+ * fills the output buffers given at submit (they must stay valid until then).  Host queries are copied at submit;
+ * DEVICE queries are read by the search's kernels, which may run on a stream of the index's own and not behind work
+ * the caller enqueues after the submit: they must stay allocated and unchanged until the wait.  At most two tickets may be outstanding; wait for them in submission order.
  * orx_search == submit + wait.  orx_search_sharded_submit is the same for the collective row-sharded search (every
  * rank submits and waits in the same order; its tickets are waited for with orx_search_wait too). */
 int orx_search_submit(orx_index *idx, const float *queries, int nq, int dim, int k,

@@ -66,7 +66,7 @@ class OrxStats(C.Structure):
         ("last_scan_ms", C.c_float),
         ("last_search_ms", C.c_float),
         ("last_path", C.c_int),
-        ("reserved", C.c_int),
+        ("shared_scans", C.c_uint32),
         ("scan_launches", C.c_uint64),
         ("scan_ms_total", C.c_double),
     ]
@@ -86,6 +86,7 @@ SIGNATURES = {
     "orx_dtype": (C.c_int, [_vp]),
     "orx_mutation_count": (C.c_uint64, [_vp]),
     "orx_get_stats": (C.c_int, [_vp, C.POINTER(OrxStats)]),
+    "orx_shared_rows": (C.c_uint64, [_vp]),
     "orx_upsert": (C.c_int, [_vp, _vp, _vp, C.c_uint64, C.c_int]),
     "orx_delete": (C.c_int, [_vp, _vp, C.c_uint64, C.POINTER(C.c_uint64)]),
     "orx_contains": (C.c_int, [_vp, OrxId]),

@@ -129,7 +129,7 @@ finalize_kernel(const T *__restrict__ table, const double *__restrict__ n2,
                 const QueryPrep *__restrict__ prep, const uint64_t *__restrict__ partial_all,
                 int nparts, int k, uint32_t n_rows, double eps, const ResultOut out, int q_base,
                 const PublishArgs pub, const DoneArgs done, const float *__restrict__ floor_all,
-                int sorted_lists) {
+                int sorted_lists, const uint32_t *__restrict__ covered) {
     constexpr int K = 32 * S;
     __shared__ uint64_t s_keys[FIN_WARPS][K];
     __shared__ double s_dist[K];
@@ -406,6 +406,7 @@ finalize_kernel(const T *__restrict__ table, const double *__restrict__ n2,
                 flag = ((1.0 - dk) > bound && dk < 2.0) ? 0 : 1;
             }
         }
+        if (covered != nullptr && covered[qi] != n_rows) flag |= 1;     // a lap missed or repeated rows: prove nothing
         flag |= (prep[qi].nonfinite ? 2 : 0) | (prep[qi].zero ? 4 : 0);
         for (int o = 0; o < n_out; ++o) {
             char *b = pub.n_targets > 0 ? pub.slot[o] : nullptr;
@@ -443,11 +444,12 @@ template <typename T>
 static void launch_finalize_t(const void *table, const double *n2, const orx_id *row_ids, const float *q,
                               const QueryPrep *prep, const uint64_t *partial, int nparts, int slots, int nq,
                               int k, uint32_t n_rows, double eps, const ResultOut &out, int q_base,
-                              const PublishArgs &pub, const DoneArgs &done, cudaStream_t st, const float *floor) {
+                              const PublishArgs &pub, const DoneArgs &done, cudaStream_t st, const float *floor,
+                              const uint32_t *covered) {
     const T *tab = static_cast<const T *>(table);
 #define ORX_FIN(S_)                                                                                          \
     launch_pdl(finalize_kernel<T, S_>, dim3(nq), dim3(FIN_THREADS), 0, st, tab, n2, row_ids, q, prep, partial, nparts, k, \
-               n_rows, eps, out, q_base, pub, done, floor, (int)(floor == nullptr))
+               n_rows, eps, out, q_base, pub, done, floor, (int)(floor == nullptr), covered)
     switch (slots) {
         case 1: ORX_FIN(1); break;
         case 2: ORX_FIN(2); break;
@@ -460,14 +462,15 @@ static void launch_finalize_t(const void *table, const double *n2, const orx_id 
 void launch_finalize(int dtype, const void *table, const double *n2, const orx_id *row_ids,
                      const float *q, const QueryPrep *prep, const uint64_t *partial, int nparts,
                      int slots, int nq, int k, uint32_t n_rows, double eps, const ResultOut &out, int q_base,
-                     const PublishArgs &pub, const DoneArgs &done, cudaStream_t st, const float *floor) {
+                     const PublishArgs &pub, const DoneArgs &done, cudaStream_t st, const float *floor,
+                     const uint32_t *covered) {
     if (nq <= 0) return;
     if (dtype == ORX_DTYPE_F32)
         launch_finalize_t<float>(table, n2, row_ids, q, prep, partial, nparts, slots, nq, k, n_rows, eps,
-                                 out, q_base, pub, done, st, floor);
+                                 out, q_base, pub, done, st, floor, covered);
     else
         launch_finalize_t<__nv_bfloat16>(table, n2, row_ids, q, prep, partial, nparts, slots, nq, k, n_rows,
-                                         eps, out, q_base, pub, done, st, floor);
+                                         eps, out, q_base, pub, done, st, floor, covered);
 }
 
 __global__ void signal_done_kernel(DoneArgs done) {

@@ -101,7 +101,9 @@ void launch_finalize(int dtype, const void *table, const double *n2, const orx_i
                      const float *q, const QueryPrep *prep, const uint64_t *partial, int nparts,
                      int slots, int nq, int k, uint32_t n_rows, double eps,
                      const ResultOut &out, int q_base, const PublishArgs &pub, const DoneArgs &done,
-                     cudaStream_t st, const float *floor = nullptr);
+                     cudaStream_t st, const float *floor = nullptr, const uint32_t *covered = nullptr);
+// covered (nq == 1): rows the scan offered for the query (LapState::covered); a count other than n_rows leaves the query
+// unproven, so the exhaustive pass answers it
 // list_stride_bytes == 0: three dense [n_lists][...] arrays; otherwise list l of each array is at +l*stride
 void launch_merge_topk(int n_lists, int nq, int k, const orx_id *ids, const double *dist,
                        const int *counts, size_t list_stride_bytes, orx_id *out_ids, double *out_dist,
@@ -154,6 +156,48 @@ void launch_scan_gemv_filtered(int dtype, const void *table, const float *scale,
 // the single-query and bitmap scans over the 8-bit image (IMAGE8_SLOTS lists); allow_bits == nullptr: every row
 void launch_scan_gemv8(const int8_t *image, const float *scale8, uint32_t n_rows, const uint32_t *allow_bits,
                        const int8_t *qhat8, const QueryPrep *prep, int nq, uint64_t *partial, int grid, cudaStream_t st);
+
+// The single-query scan over the 8-bit image of a search submitted with orx_search_submit is a LAP (DESIGN.md section
+// 4, "two searches in flight"; orx_search, which no other search can join, keeps scan_gemv8_kernel): the table is cut
+// into LAP_SEGS segments, warps claim LAP_CHUNK rows at a time from a device-side counter, front to back, and the first
+// claim in a segment SEALS the segment's query-set word.  Until then a second search may JOIN the segment (atomicCAS
+// 0 -> SEG_JOINED, join kernel): every claimer of the segment then scores its rows against both queries.  A sealed word
+// never changes, so all claimers see the same set.  The joiner's CATCH-UP is a lap of its own over the segments it did
+// not get (itself joinable), merged into the lists the joined lap left.  Every lap counts the rows it offered per query
+// into that query's `covered`; finalize marks a query unproven unless covered == n_rows.
+constexpr int LAP_SEGS = 64;
+constexpr uint32_t LAP_CHUNK = 64;
+constexpr uint32_t SEG_SEALED = 1u << 31, SEG_JOINED = 1u;
+struct LapJoiner {               // written by the join kernel before its first atomicCAS
+    const int8_t *q8;            // the joiner's qhat8 (h | l slices) and prep
+    const QueryPrep *prep;
+    uint64_t *partial;           // its per-CTA lists for this lap's grid, zeroed before the join
+    uint32_t *covered;
+};
+struct LapState {                // one per search slot, device memory
+    uint32_t next;               // work queue: chunks claimed so far
+    uint32_t covered;            // rows offered for this slot's query, by its own lap and by a lap it joined
+    uint32_t n_list;             // catch-up: segments to scan, list[0, n_list)
+    uint32_t pad;
+    uint32_t seg[LAP_SEGS];      // query-set word of each segment: SEG_SEALED | SEG_JOINED
+    uint32_t list[LAP_SEGS];
+    LapJoiner joiner;
+};
+// rows per segment (a multiple of LAP_CHUNK, so a chunk never straddles two segments)
+inline uint32_t lap_seg_rows(uint32_t n_rows) {
+    const uint32_t per = (n_rows + LAP_SEGS - 1) / LAP_SEGS;
+    return (per + LAP_CHUNK - 1) / LAP_CHUNK * LAP_CHUNK;
+}
+// the lap of one query (q8 / prep / partial of query 0).  catch_up == 0: every segment, lap->seg all 0 (the caller
+// clears next / covered / seg); catch_up == 1: the segments in lap->list (join kernel), each CTA's list merged with
+// the one partial already holds
+void launch_scan_lap8(const int8_t *image, const float *scale8, uint32_t n_rows, const int8_t *qhat8,
+                      const QueryPrep *prep, uint64_t *partial, LapState *lap, int catch_up, int grid, cudaStream_t st);
+// one CTA: publish `me` on `host`, try to join every segment of host's lap that is still open, and set up `mine` (the
+// joiner's own lap state; next / covered already cleared) for the catch-up over the others.  rows_joined: mapped host
+// word <- rows of the joined segments
+void launch_join_lap8(LapState *host, LapState *mine, const LapJoiner &me, uint32_t n_rows, uint32_t *rows_joined,
+                      cudaStream_t st);
 
 // ---- table_ops.cu
 void launch_validate_rows(const float *src, uint64_t n, int *flag, cudaStream_t st);

@@ -258,6 +258,12 @@ struct SearchSlot {         // everything ONE search in flight owns
     std::vector<cudaEvent_t> scan_ev;   // pairs bracketing each scan launch of the search
     size_t scan_ev_used = 0;
     orx::UmmaPlan *umma = nullptr;
+    // single-query 8-bit scans (lap_search): they run on this slot's own stream, so that the other slot's search can
+    // join a lap while it runs (internal.h LapState).  ev_entry: the index stream at submit; ev_ready: this slot's lap
+    // state is set up (and its join attempt, if any, is over); ev_lap: after its lap; ev_done: after its finalize
+    DevBuf<orx::LapState> lap;
+    cudaStream_t lap_stream = nullptr;
+    cudaEvent_t ev_entry = nullptr, ev_ready = nullptr, ev_lap = nullptr, ev_done = nullptr;
     // the search in flight in this slot (orx_search_submit ... orx_search_wait)
     struct Pending {
         bool active = false, complete = false, sharded = false, out_on_dev = false;
@@ -270,6 +276,9 @@ struct SearchSlot {         // everything ONE search in flight owns
         int *out_counts = nullptr;
         orx::ResultOut out{};               // where the kernels write (prepare_results)
         const float *q_src = nullptr;
+        bool lap = false;                   // ran on lap_stream (lap_search)
+        SearchSlot *join_host = nullptr;    // the other slot, whose lap this search tries to join
+        uint32_t lap_rows = 0;              // live rows its lap scans
         uint32_t token = 0, seq = 0, ticket = 0;
         SlotLayout L;
         std::chrono::steady_clock::time_point t_begin;
@@ -280,6 +289,13 @@ struct SearchSlot {         // everything ONE search in flight owns
         h_myflags.release(); h_redo.release(); h_done.release(); d_counters.release();
         for (auto &e : scan_ev) cudaEventDestroy(e);
         scan_ev.clear();
+        lap.release();
+        for (cudaEvent_t *e : {&ev_entry, &ev_ready, &ev_lap, &ev_done}) {
+            if (*e) cudaEventDestroy(*e);
+            *e = nullptr;
+        }
+        if (lap_stream) cudaStreamDestroy(lap_stream);
+        lap_stream = nullptr;
     }
 };
 
@@ -349,6 +365,7 @@ struct orx_index {
 
     mutable std::mutex mu;
     orx_stats stats{};
+    uint64_t shared_rows = 0;           // orx_shared_rows
 };
 
 struct FilterOnDevice {          // a resolved predicate: the eligible rows, as a sorted list and (when large) a bitmap
@@ -736,6 +753,8 @@ struct SearchCtx {          // where a search's results go and how its completio
     orx::ResultOut out;
     orx::PublishArgs pub;
     orx::DoneArgs done;
+    bool lap = false;                   // a single-query 8-bit scan runs as a lap (lap_search)
+    SearchSlot *join_host = nullptr;    // ... that joins this slot's lap
 };
 SearchCtx plain_ctx(const orx::ResultOut &out) {      // no publish, no completion word
     SearchCtx c{};
@@ -771,6 +790,45 @@ int exhaustive_query(orx_index *ix, const float *q_src, int qi, int k, double dk
     return ORX_OK;
 }
 
+// ---- the lap of a single-query 8-bit scan on ix->stream (internal.h LapState): set up the slot's lap state, and for a
+//      search that joins the other slot's lap (host) run the join, then wait for that lap before the catch-up
+int ensure_lap(SearchSlot *sl) {
+    CK(sl->lap.ensure(1));
+    if (!sl->lap_stream) CK(cudaStreamCreateWithFlags(&sl->lap_stream, cudaStreamNonBlocking));
+    for (cudaEvent_t *e : {&sl->ev_entry, &sl->ev_ready, &sl->ev_lap, &sl->ev_done})
+        if (!*e) CK(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+    return ORX_OK;
+}
+int lap_setup(orx_index *ix, int qa, uint32_t n_rows, int grid, SearchSlot *host) {
+    SearchSlot *sl = ix->cur;
+    SearchSlot *other = &ix->slot[sl == &ix->slot[0] ? 1 : 0];
+    cudaStream_t st = ix->stream;
+    const int rc = ensure_lap(sl);
+    if (rc != ORX_OK) return rc;
+    // the other slot's join kernel may have worked on this slot's state (it joined this slot's previous lap)
+    if (other->ev_ready) CK(cudaStreamWaitEvent(st, other->ev_ready, 0));
+    if (!host) {
+        CK(cudaMemsetAsync(sl->lap.p, 0, offsetof(orx::LapState, list), st));
+        CK(cudaEventRecord(sl->ev_ready, st));
+        return ORX_OK;
+    }
+    // the joined lap writes this query's lists of its grid (same rows, same grid) only in the CTAs that met the join
+    CK(cudaMemsetAsync(sl->partial.p, 0, (size_t)grid * 32 * orx::IMAGE8_SLOTS * sizeof(uint64_t), st));
+    CK(cudaMemsetAsync(sl->lap.p, 0, 2 * sizeof(uint32_t), st));             // next, covered
+    const orx::LapJoiner me{sl->qhat8.p + (size_t)qa * 2 * ORX_DIM, sl->prep.p + qa, sl->partial.p, &sl->lap.p->covered};
+    orx::launch_join_lap8(host->lap.p, sl->lap.p, me, n_rows, sl->h_done.p + 2, st);
+    CK(cudaEventRecord(sl->ev_ready, st));
+    CK(cudaStreamWaitEvent(st, host->ev_lap, 0));                           // the catch-up merges into its lists
+    ix->stats.kernel_launches += 1;
+    return ORX_OK;
+}
+// a submitted search whose scan is a lap: one query over the 8-bit image
+bool lap_search(orx_index *ix, int nq, int k) {
+    if (nq != 1 || ix->n_live == 0) return false;
+    ensure_image(ix);
+    return gemv_source(ix, 1, k, false) == 4;
+}
+
 // f: a filter with a bitmap -- the sequential scan skips the rows whose bit is clear (HBM traffic = eligible rows only).
 // allow_image: a large fp32 table with an image is scanned over the image (the bf16 instantiation of the same kernels,
 // the fp32 row's 1/|x|, EPS_GEMV_IMAGE; or the 8-bit scan, EPS_GEMV_IMAGE8, see gemv_source); finalize rescores the fp32
@@ -791,12 +849,26 @@ int gemv_pass(orx_index *ix, const float *q_src, int q0, int nq, int k, const Se
         const double eps = src == 4 ? orx::EPS_GEMV_IMAGE8 : img ? orx::EPS_GEMV_IMAGE
                            : ix->dtype == ORX_DTYPE_F32 ? orx::EPS_GEMV_F32 : orx::EPS_GEMV_BF16;
         const int slots = src == 4 ? orx::IMAGE8_SLOTS : img ? orx::image_slots_for_k(k) : orx::slots_for_k(k);
-        // several queries: the batched kernel (8 queries share every row through shared memory); one: the streaming kernel
-        const int parts = !f && m >= 2 ? orx::scan_gemv_batch_parts(ix->device, n_rows, m) : grid;
+        const bool lap = src == 4 && !f && ctx.lap;                     // (m == 1: gemv_source)
+        // several queries: the batched kernel (8 queries share every row through shared memory); one: the streaming
+        // kernel.  A lap leaves two CTA slots of the GPU free (2 CTAs of it fill an SM's registers), so that the other
+        // slot's prep, memsets and join kernel -- and the tail of its catch-up or finalize -- find room while it runs; with
+        // every slot taken, none of 20 pairs submitted back to back joined.  Its work queue gives the two half-used SMs
+        // their share of the rows
+        const int parts = lap ? std::max(1, std::min(grid, 2 * orx::device_sms() - 2))
+                          : !f && m >= 2 ? orx::scan_gemv_batch_parts(ix->device, n_rows, m) : grid;
         CK(ix->cur->partial.ensure((size_t)m * parts * 32 * slots));
+        if (lap) {
+            const int rc = lap_setup(ix, qa, n_rows, parts, ctx.join_host);
+            if (rc != ORX_OK) return rc;
+        }
         cudaEvent_t e0 = scan_event(ix), e1 = scan_event(ix);
         if (e0 && e1) CK(cudaEventRecord(e0, ix->stream));
-        if (src == 4)
+        if (lap)
+            orx::launch_scan_lap8(ix->image8.rows, ix->image8.scale8, n_rows, ix->cur->qhat8.p + (size_t)qa * 2 * ORX_DIM,
+                                  ix->cur->prep.p + qa, ix->cur->partial.p, ix->cur->lap.p, ctx.join_host != nullptr,
+                                  parts, ix->stream);
+        else if (src == 4)
             orx::launch_scan_gemv8(ix->image8.rows, ix->image8.scale8, n_rows, f ? f->bits : nullptr,
                                    ix->cur->qhat8.p + (size_t)qa * 2 * ORX_DIM, ix->cur->prep.p + qa, m,
                                    ix->cur->partial.p, grid, ix->stream);
@@ -811,10 +883,11 @@ int gemv_pass(orx_index *ix, const float *q_src, int q0, int nq, int k, const Se
             orx::launch_scan_gemv(scan_dtype, scan_rows, ix->scale, n_rows, ix->cur->qhat.p + (size_t)qa * ORX_DIM, m,
                                   slots, ix->cur->partial.p, grid, ix->stream);
         if (e0 && e1) CK(cudaEventRecord(e1, ix->stream));
+        if (lap) CK(cudaEventRecord(ix->cur->ev_lap, ix->stream));
         // a filter's row bound is the eligible count: "every eligible row is a candidate" when it fits the list
         orx::launch_finalize(ix->dtype, ix->table, ix->n2, ix->row_ids, q_src + (size_t)qa * ORX_DIM,
                              ix->cur->prep.p + qa, ix->cur->partial.p, parts, slots, m, k, f ? f->m : n_rows, eps, ctx.out,
-                             qa, ctx.pub, ctx.done, ix->stream);
+                             qa, ctx.pub, ctx.done, ix->stream, nullptr, lap ? &ix->cur->lap.p->covered : nullptr);
         ix->stats.kernel_launches += 2;
     }
     CK(cudaGetLastError());
@@ -911,10 +984,11 @@ uint32_t next_token(orx_index *ix) {
 }
 int wait_done(orx_index *ix, uint32_t token) {
     volatile uint32_t *w = ix->cur->h_done.p;
+    cudaStream_t st = ix->cur->pend.lap ? ix->cur->lap_stream : ix->stream;
     for (uint64_t it = 0;; ++it) {
         if (*w == token) return ORX_OK;
         if ((it & 0x3FFu) == 0x3FFu) {
-            cudaError_t e = cudaStreamQuery(ix->stream);
+            cudaError_t e = cudaStreamQuery(st);
             if (e == cudaSuccess) {
                 if (*w == token) return ORX_OK;
                 return fail(ORX_ERR_CUDA, "search finished without signalling completion");
@@ -928,9 +1002,10 @@ int wait_done(orx_index *ix, uint32_t token) {
 }
 int ensure_signalling(orx_index *ix) {
     if (!ix->cur->h_done.p) {
-        CK(ix->cur->h_done.ensure(2));
+        CK(ix->cur->h_done.ensure(3));
         ix->cur->h_done.p[0] = 0;
         ix->cur->h_done.p[1] = 0;
+        ix->cur->h_done.p[2] = 0;
     }
     if (!ix->cur->d_counters.p) {
         CK(ix->cur->d_counters.ensure(2));
@@ -1034,8 +1109,10 @@ int resolve_unproven(orx_index *ix, const float *q_src, int nq, int k, const orx
 // ---- a search = submit (launch the whole chain on the slot `ix->cur`, no waiting) + wait (poll the completion word,
 //      settle unproven queries, hand the results over).  orx_search is the two back to back; orx_search_submit /
 //      orx_search_wait let a caller keep two searches in flight.
+// joinable: orx_search_submit -- a single-query 8-bit scan runs as a lap another submit can join (orx_search holds the
+// index mutex until its search is complete, so nothing can join it: it keeps the plain scan on the index stream)
 int search_submit_locked(orx_index *ix, const float *queries, int nq, int k, orx_id *out_ids, double *out_dist,
-                         int *out_counts) {
+                         int *out_counts, bool joinable) {
     SearchSlot::Pending &pd = ix->cur->pend;
     pd = SearchSlot::Pending{};
     pd.t_begin = std::chrono::steady_clock::now();
@@ -1046,6 +1123,29 @@ int search_submit_locked(orx_index *ix, const float *queries, int nq, int k, orx
     pd.out_dist = out_dist;
     pd.out_counts = out_counts;
     const bool out_on_dev = pd.out_on_dev;
+    // a lap search runs on the slot's own stream behind everything the index stream holds now; it joins the other
+    // slot's lap when that one is still running over the same rows (no write can have come between: a write settles
+    // every search in flight)
+    pd.lap = joinable && lap_search(ix, nq, k);
+    cudaStream_t index_stream = ix->stream;
+    if (pd.lap) {
+        int rc = ensure_lap(ix->cur);
+        if (rc != ORX_OK) return rc;
+        CK(cudaEventRecord(ix->cur->ev_entry, index_stream));
+        CK(cudaStreamWaitEvent(ix->cur->lap_stream, ix->cur->ev_entry, 0));
+        SearchSlot *other = &ix->slot[ix->cur == &ix->slot[0] ? 1 : 0];
+        const SearchSlot::Pending &op = other->pend;
+        pd.lap_rows = (uint32_t)ix->n_live;
+        if (op.active && op.lap && !op.complete && !op.settled && op.lap_rows == pd.lap_rows &&
+            cudaEventQuery(other->ev_lap) == cudaErrorNotReady)
+            pd.join_host = other;
+        ix->stream = ix->cur->lap_stream;
+    }
+    struct RestoreStream {
+        orx_index *ix;
+        cudaStream_t st;
+        ~RestoreStream() { ix->stream = st; }
+    } restore{ix, index_stream};
     cudaStream_t st = ix->stream;
     const size_t nk = (size_t)nq * k;
     ix->cur->scan_ev_used = 0;
@@ -1082,8 +1182,11 @@ int search_submit_locked(orx_index *ix, const float *queries, int nq, int k, orx
         return ORX_OK;
     }
     SearchCtx ctx = plain_ctx(pd.out);
+    ctx.lap = pd.lap;
+    ctx.join_host = pd.join_host;
     pd.token = next_token(ix);
     ctx.done = orx::DoneArgs{ix->cur->d_counters.p, (unsigned int)nq, ix->cur->h_done.p, pd.token};
+    if (pd.join_host) ix->cur->h_done.p[2] = 0;
     rc = scan_pass(ix, pd.q_src, nq, k, ctx, &pd.path);
     if (rc != ORX_OK) {
         cudaStreamSynchronize(st);          // part of the chain may be in flight: drain it, forget its count
@@ -1091,6 +1194,7 @@ int search_submit_locked(orx_index *ix, const float *queries, int nq, int k, orx
         cudaGetLastError();
         return rc;
     }
+    if (pd.lap) CK(cudaEventRecord(ix->cur->ev_done, st));
     pd.active = true;
     return ORX_OK;
 }
@@ -1492,6 +1596,13 @@ int search_wait_locked(orx_index *ix) {
         const char *peer = pd.sharded ? "sharded search: a peer rank" : nullptr;
         int rc = wait_done(ix, pd.token);       // the last kernel wrote the completion word; flags are on the host
         if (rc != ORX_OK) return rc;
+        if (pd.lap) {                           // the index stream (the caller's) is ordered after the search
+            CK(cudaStreamWaitEvent(ix->stream, ix->cur->ev_done, 0));
+            if (pd.join_host && ix->cur->h_done.p[2] != 0) {
+                ix->stats.shared_scans += 1;
+                ix->shared_rows += ix->cur->h_done.p[2];
+            }
+        }
         bool unproven = false;
         rc = search_verdict(ix->cur, nq, peer, &unproven);
         if (rc != ORX_OK) return rc;
@@ -1556,7 +1667,7 @@ int search_locked(orx_index *ix, Exchange *x, const float *queries, int nq, int 
     int rc = claim_slot(ix, nullptr);
     if (rc != ORX_OK) return rc;
     rc = x ? sharded_submit_locked(ix, x, queries, nq, k, out_ids, out_dist, out_counts)
-           : search_submit_locked(ix, queries, nq, k, out_ids, out_dist, out_counts);
+           : search_submit_locked(ix, queries, nq, k, out_ids, out_dist, out_counts, /*joinable=*/false);
     if (rc != ORX_OK) return rc;
     ix->tickets += 1;
     return search_wait_locked(ix);
@@ -1775,6 +1886,12 @@ int orx_get_stats(const orx_index *ix, orx_stats *out) {
     return ORX_OK;
 }
 
+uint64_t orx_shared_rows(const orx_index *ix) {
+    if (!ix || ix->group) return 0;
+    std::lock_guard<std::mutex> lk(ix->mu);
+    return ix->shared_rows;
+}
+
 int orx_contains(const orx_index *ix, orx_id id) {
     if (!ix) return 0;
     if (ix->group) return orx_contains(ix->group->shards[orx::shard_of_id(id, (uint32_t)ix->group->shards.size())], id);
@@ -1891,7 +2008,7 @@ int orx_search_submit(orx_index *ix, const float *queries, int nq, int dim, int 
     DeviceGuard g(ix->device);
     rc = claim_slot(ix, ticket);
     if (rc != ORX_OK) return rc;
-    rc = search_submit_locked(ix, queries, nq, k, out_ids, out_dist, out_counts);
+    rc = search_submit_locked(ix, queries, nq, k, out_ids, out_dist, out_counts, /*joinable=*/true);
     if (rc != ORX_OK) return rc;
     ix->cur->pend.ticket = ix->tickets;
     ix->tickets += 1;

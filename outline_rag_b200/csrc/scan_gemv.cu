@@ -21,26 +21,29 @@
 
 namespace orx {
 
-// per-CTA merge by counting, shared by the scan kernels: the 8 warp lists hold 8*K distinct keys (0 = empty), each sorted
-// descending; a key's rank is the number of larger keys (a binary search per list), ranks < K are the CTA's sorted
-// top-K -> partial[0..K)
-template <int S>
-__device__ __forceinline__ void cta_merge_store(const WarpTopK<S> &top, uint64_t (&s_keys)[SCAN_WARPS][32 * S],
+// per-CTA merge by counting, shared by the scan kernels: the NL lists of s_keys hold NL*K distinct keys (0 = empty), each
+// sorted descending -- the 8 warp lists, and for NL = SCAN_WARPS + 1 a list the caller put in s_keys[SCAN_WARPS] (the
+// CTA's list from an earlier launch of the same search); a key's rank is the number of larger keys (a binary search per
+// list), ranks < K are the CTA's sorted top-K -> partial[0..K)
+template <int S, int NL = SCAN_WARPS>
+__device__ __forceinline__ void cta_merge_store(const WarpTopK<S> &top, uint64_t (&s_keys)[NL][32 * S],
                                                 uint64_t *__restrict__ partial, int lane, int warp) {
     constexpr int K = 32 * S;
     top.store(s_keys[warp], lane);
     __syncthreads();
     const uint64_t *all = &s_keys[0][0];
-    constexpr int TOTAL = SCAN_WARPS * K;
+    constexpr int TOTAL = NL * K;
+    constexpr int ROUNDS = (TOTAL + SCAN_THREADS - 1) / SCAN_THREADS;
     int nonzero = 0;
 #pragma unroll
-    for (int h = 0; h < TOTAL / SCAN_THREADS; ++h) {
-        const uint64_t mine = all[threadIdx.x + h * SCAN_THREADS];
+    for (int h = 0; h < ROUNDS; ++h) {
+        const int i = threadIdx.x + h * SCAN_THREADS;
+        const uint64_t mine = i < TOTAL ? all[i] : 0ull;
         nonzero += (mine != 0ull);
         if (mine == 0ull) continue;
         int rank = 0;
 #pragma unroll
-        for (int w = 0; w < SCAN_WARPS; ++w) {
+        for (int w = 0; w < NL; ++w) {
             int lo = 0, hi = K;                         // keys of list w above `mine`: the first position not above it
             while (lo < hi) {
                 const int mid = (lo + hi) >> 1;
@@ -53,7 +56,7 @@ __device__ __forceinline__ void cta_merge_store(const WarpTopK<S> &top, uint64_t
     }
     int nnz = 0;
 #pragma unroll
-    for (int j = 1; j <= TOTAL / SCAN_THREADS; ++j) nnz += __syncthreads_count(nonzero >= j);
+    for (int j = 1; j <= ROUNDS; ++j) nnz += __syncthreads_count(nonzero >= j);
     if ((int)threadIdx.x < K && (int)threadIdx.x >= nnz) partial[threadIdx.x] = 0ull;
 }
 
@@ -404,6 +407,191 @@ void launch_scan_gemv8(const int8_t *image, const float *scale8, uint32_t n_rows
     else
         launch_pdl(scan_gemv8_kernel<false>, g, dim3(SCAN_THREADS), 0, st, image, scale8, n_rows, allow_bits, qhat8, prep,
                    partial);
+}
+
+// ------------------------------------------------------------------ the lap (internal.h LapState)
+// The single-query 8-bit scan with the schedule of scan_gemv8_kernel's rows (ROWS8 rows, one warp, the same
+// dot, reduction and keys), but rows come from the work queue: a warp claims LAP_CHUNK consecutive rows per atomicAdd,
+// and its claim seals the chunk's segment.  Both atomics run two chunks ahead of the scoring (claim, then seal one
+// chunk later, then scan), so their round trips hide behind the 64 KB a chunk streams.  A joined segment's rows are
+// scored a second time, against the joiner's slices (shared memory), into a second WarpTopK.  Scores and keys do not
+// depend on which lap or warp offered a row, so the lists of a query built by two laps hold the same top-K.
+__device__ __forceinline__ uint32_t ld_cg_u32(const uint32_t *p) { return __ldcg(p); }
+
+__global__ void __launch_bounds__(SCAN_THREADS, 2)
+scan_lap8_kernel(const int8_t *__restrict__ table, const float *__restrict__ scale8, uint32_t n_rows,
+                 uint32_t seg_rows, const int8_t *__restrict__ q8, const QueryPrep *__restrict__ prep,
+                 uint64_t *__restrict__ partial, LapState *lap, int catch_up) {
+    constexpr int K = 32 * SLOTS8;
+    __shared__ uint64_t s_keys[SCAN_WARPS + 1][K];
+    __shared__ uint4 s_q[4 * 32];                              // this lap's query: h | l slices (load_q8_slice layout)
+    __shared__ uint4 s_jq[SCAN_WARPS][4 * 32];                 // the joiner's, a copy per warp
+    __shared__ uint64_t *s_jpartial;
+    __shared__ uint32_t *s_jcovered;
+    __shared__ uint32_t s_cov[2];                              // rows this CTA offered: for this lap's query, the joiner's
+
+    const int lane = threadIdx.x & 31;
+    const int warp = threadIdx.x >> 5;
+    if (threadIdx.x < 2) s_cov[threadIdx.x] = 0u;
+    __syncthreads();
+
+    pdl_wait();
+    if (threadIdx.x < 4 * 32) s_q[threadIdx.x] = reinterpret_cast<const uint4 *>(q8)[threadIdx.x];
+    const float dq = prep->dq8;
+    __syncthreads();
+
+    WarpTopK<SLOTS8> top, topj;
+    top.init();
+    topj.init();
+    float dqj = 0.f;
+    bool have_j = false;
+
+    const uint4 *tab = reinterpret_cast<const uint4 *>(table);
+    const uint32_t cps = seg_rows / LAP_CHUNK;                 // chunks per segment
+    const uint32_t total = (catch_up ? ld_cg_u32(&lap->n_list) : (uint32_t)LAP_SEGS) * cps;
+    auto seg_of = [&](uint32_t c) { return catch_up ? lap->list[c / cps] : c / cps; };
+    const int my = lane >> 2;
+
+    // lane 0 holds the atomics in flight; c / w: the chunk being scanned and its segment's word, c1 claimed, unsealed
+    uint32_t a_c = 0, a_w = 0;
+    if (lane == 0) a_c = atomicAdd(&lap->next, 1u);
+    uint32_t c = __shfl_sync(FULL_MASK, a_c, 0);
+    if (lane == 0) {
+        a_c = c < total ? atomicAdd(&lap->next, 1u) : total;
+        a_w = c < total ? atomicOr(&lap->seg[seg_of(c)], SEG_SEALED) : 0u;
+    }
+    uint32_t w = __shfl_sync(FULL_MASK, a_w, 0);
+    uint32_t c1 = __shfl_sync(FULL_MASK, a_c, 0);
+    while (c < total) {
+        if (lane == 0) {
+            a_w = c1 < total ? atomicOr(&lap->seg[seg_of(c1)], SEG_SEALED) : 0u;
+            a_c = c1 < total ? atomicAdd(&lap->next, 1u) : total;
+        }
+        const bool joined = (w & SEG_JOINED) != 0u;
+        if (joined && !have_j) {                               // first joined chunk of this warp: fetch the joiner
+            // lane 0 observed SEG_JOINED (its atomicOr); its fence makes the join kernel's stores before the atomicCAS
+            // visible to it, and __syncwarp orders the other lanes' loads after lane 0's
+            const LapJoiner *J = &lap->joiner;
+            unsigned long long jq8 = 0, jprep = 0;
+            if (lane == 0) {
+                __threadfence();
+                jq8 = __ldcg(reinterpret_cast<const unsigned long long *>(&J->q8));
+                jprep = __ldcg(reinterpret_cast<const unsigned long long *>(&J->prep));
+                s_jpartial = reinterpret_cast<uint64_t *>(__ldcg(reinterpret_cast<const unsigned long long *>(&J->partial)));
+                s_jcovered = reinterpret_cast<uint32_t *>(__ldcg(reinterpret_cast<const unsigned long long *>(&J->covered)));
+            }
+            __syncwarp();
+            const uint4 *jp = reinterpret_cast<const uint4 *>(__shfl_sync(FULL_MASK, jq8, 0));
+            const QueryPrep *jpr = reinterpret_cast<const QueryPrep *>(__shfl_sync(FULL_MASK, jprep, 0));
+#pragma unroll
+            for (int j = 0; j < 4; ++j) s_jq[warp][lane + 32 * j] = __ldcg(jp + lane + 32 * j);
+            dqj = __ldcg(&jpr->dq8);
+            __syncwarp();
+            have_j = true;
+        }
+        const uint32_t seg = seg_of(c);
+        const uint32_t r0 = seg * seg_rows + (c % cps) * LAP_CHUNK;
+        const uint32_t r1 = min(r0 + LAP_CHUNK, n_rows);
+        for (uint32_t g = r0; g < r1; g += ROWS8) {
+            uint4 v[ROWS8][2];
+            const uint32_t my_row = g + my;
+            const bool my_ok = my_row < r1;
+            const float my_sc = __ldg(scale8 + min(my_row, n_rows - 1));
+#pragma unroll
+            for (int r = 0; r < ROWS8; ++r) {
+                const uint4 *p = tab + (size_t)min(g + r, n_rows - 1) * 64 + lane;   // tail rows re-read the last
+                v[r][0] = ldg_stream_u4(p);
+                v[r][1] = ldg_stream_u4(p + 32);
+            }
+            int p[ROWS8];
+            {
+                uint4 qh[2], ql[2];                            // 16 registers for the scan's 8 KB in flight otherwise
+#pragma unroll
+                for (int j = 0; j < 2; ++j) {
+                    qh[j] = s_q[lane + 32 * j];
+                    ql[j] = s_q[64 + lane + 32 * j];
+                }
+#pragma unroll
+                for (int r = 0; r < ROWS8; ++r) p[r] = lane_dot8(v[r], qh, ql);
+            }
+            const int D = warp_reduce8(p, lane);
+            const uint64_t key = my_ok ? make_key(score_ord(image8_dot(D, dq), my_sc), my_row) : 0ull;
+            top.offer_lanes((lane & 3) == 0 ? key : 0ull, lane);
+            if (joined) {
+                uint4 jh[2], jl[2];
+#pragma unroll
+                for (int j = 0; j < 2; ++j) {
+                    jh[j] = s_jq[warp][lane + 32 * j];
+                    jl[j] = s_jq[warp][64 + lane + 32 * j];
+                }
+#pragma unroll
+                for (int r = 0; r < ROWS8; ++r) p[r] = lane_dot8(v[r], jh, jl);
+                const int Dj = warp_reduce8(p, lane);
+                const uint64_t kj = my_ok ? make_key(score_ord(image8_dot(Dj, dqj), my_sc), my_row) : 0ull;
+                topj.offer_lanes((lane & 3) == 0 ? kj : 0ull, lane);
+            }
+        }
+        if (lane == 0 && r1 > r0) {
+            atomicAdd(&s_cov[0], r1 - r0);
+            if (joined) atomicAdd(&s_cov[1], r1 - r0);
+        }
+        c = c1;
+        w = __shfl_sync(FULL_MASK, a_w, 0);
+        c1 = __shfl_sync(FULL_MASK, a_c, 0);
+    }
+
+    uint64_t *mine = partial + (size_t)blockIdx.x * K;
+    if ((int)threadIdx.x < K) s_keys[SCAN_WARPS][threadIdx.x] = catch_up ? mine[threadIdx.x] : 0ull;
+    cta_merge_store<SLOTS8, SCAN_WARPS + 1>(top, s_keys, mine, lane, warp);     // (its barriers order the s_cov adds)
+    if (threadIdx.x == 0) atomicAdd(&lap->covered, s_cov[0]);
+    if (__syncthreads_or(have_j)) {                           // some warp scored rows for the joiner
+        if ((int)threadIdx.x < K) s_keys[SCAN_WARPS][threadIdx.x] = 0ull;
+        cta_merge_store<SLOTS8, SCAN_WARPS + 1>(topj, s_keys, s_jpartial + (size_t)blockIdx.x * K, lane, warp);
+        if (threadIdx.x == 0) atomicAdd(s_jcovered, s_cov[1]);
+    }
+    // only after the last store: the catch-up of a joiner waits for these lists through an event recorded behind this
+    // kernel (ev_lap).  With the trigger at the start, a second search submitted right after the first found that event
+    // complete while the lap still ran and never joined (pairs submitted back to back, ORX_OPT_SCAN_TIMING off)
+    __threadfence();
+    pdl_launch_dependents();
+}
+
+void launch_scan_lap8(const int8_t *image, const float *scale8, uint32_t n_rows, const int8_t *qhat8,
+                      const QueryPrep *prep, uint64_t *partial, LapState *lap, int catch_up, int grid, cudaStream_t st) {
+    launch_pdl(scan_lap8_kernel, dim3(grid), dim3(SCAN_THREADS), 0, st, image, scale8, n_rows, lap_seg_rows(n_rows),
+               qhat8, prep, partial, lap, catch_up);
+}
+
+__global__ void __launch_bounds__(LAP_SEGS)
+join_lap8_kernel(LapState *host, LapState *mine, LapJoiner me, uint32_t n_rows, uint32_t seg_rows,
+                 uint32_t *rows_joined) {
+    __shared__ uint32_t s_miss[LAP_SEGS / 32], s_rows;
+    const int t = threadIdx.x;
+    if (t == 0) {
+        host->joiner = me;
+        s_rows = 0u;
+    }
+    __threadfence();                                           // the joiner is published before any segment names it
+    __syncthreads();
+    const bool got = atomicCAS(&host->seg[t], 0u, SEG_JOINED) == 0u;
+    mine->seg[t] = got ? SEG_SEALED : 0u;                      // a joined segment is closed to whoever joins my catch-up
+    const uint32_t lo = (uint32_t)t * seg_rows;
+    if (got && lo < n_rows) atomicAdd(&s_rows, min(seg_rows, n_rows - lo));
+    const unsigned miss = __ballot_sync(FULL_MASK, !got);
+    if ((t & 31) == 0) s_miss[t >> 5] = miss;
+    __syncthreads();
+    int before = 0;                                            // the missed segments, in table order
+    for (int i = 0; i < (t >> 5); ++i) before += __popc(s_miss[i]);
+    before += __popc(miss & ((1u << (t & 31)) - 1u));
+    if (!got) mine->list[before] = (uint32_t)t;
+    if (t == LAP_SEGS - 1) mine->n_list = (uint32_t)before + (got ? 0u : 1u);
+    __syncthreads();
+    if (t == 0) *reinterpret_cast<volatile uint32_t *>(rows_joined) = s_rows;
+}
+
+void launch_join_lap8(LapState *host, LapState *mine, const LapJoiner &me, uint32_t n_rows, uint32_t *rows_joined,
+                      cudaStream_t st) {
+    join_lap8_kernel<<<1, LAP_SEGS, 0, st>>>(host, mine, me, n_rows, lap_seg_rows(n_rows), rows_joined);
 }
 
 // orx_debug_image8_scores: every row's 8-bit score (the value score_ord keys on) for nq queries, out[row * nq + query]

@@ -289,7 +289,9 @@ class Index:
     def stats(self) -> dict:
         st = OrxStats()
         check(lib.orx_get_stats(self._h, C.byref(st)))
-        return {name: getattr(st, name) for name, _ in OrxStats._fields_ if name != "reserved"}
+        out = {name: getattr(st, name) for name, _ in OrxStats._fields_}
+        out["shared_rows"] = int(lib.orx_shared_rows(self._h))
+        return out
 
     # -- writes
     def upsert(self, ids, vecs) -> None:
@@ -402,7 +404,9 @@ class Index:
     def search_submit(self, queries, k: int, out, sharded: bool = False) -> int:
         """Launch a search of a float32 CUDA tensor `queries` into the caller-owned CUDA tensors `out` =
         (ids int64 [nq,k,2], dist float64 [nq,k], counts int32 [nq]) and return a ticket at once; at most two
-        tickets may be outstanding.  `search_wait(ticket)` completes it (`out` is filled then).  `sharded=True`:
+        tickets may be outstanding.  `search_wait(ticket)` completes it (`out` is filled then).  The search's kernels
+        read `queries` after this returns, possibly on a stream of the index's own: keep the tensor alive and unchanged
+        until the wait.  `sharded=True`:
         the collective row-sharded search (every rank submits and waits in the same order)."""
         q = queries if queries.dim() == 2 else queries.unsqueeze(0)
         t = C.c_int(-1)
